@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- bases classified per second (Mbp/s) on the DeepGRP prediction hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mbp M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--mbp M] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (forward + vote + score + MSS + segment extraction)
 over one synthetic record.  Workload at N=1: BASELINE.json configs[1] -- defaults.toml architecture
@@ -20,6 +20,8 @@ Keys beyond the base contract:
              measured bf16 tensor peak of MEASURED_PEAKS.json;
   cpu_baseline  the oracle port (reference restated on CPU, TF absent) on a bounded prefix.
 `--impl reference` times the CPU restatement of the reference path only (rank 0).
+`--dump-outputs DIR` writes what the last timed `value` step computed on rank 0 (see dump_outputs); the inputs
+depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -250,6 +252,28 @@ def workload_config(args, bases):
             "sharding": "one record per rank, no collective"}
 
 
+DUMP_LABELS, DUMP_ROWS = 4_000_000, 1_000_000     # at most 16 MB of labels and 24 MB of rows
+
+
+def dump_outputs(out_dir, ctx, length, n_rows):
+    """What the last dgrp_predict_codes_dev left on the device, as float .npy files in `out_dir`: labels.npy, the
+    final labels (float32) at DUMP_LABELS positions; label_counts.npy, the count of each label over all positions
+    (float64); rows.npy, DUMP_ROWS of the rows as (start, end, label) (float64).  Positions and rows are fixed
+    samples (seeded, sorted) when there are more; all of them otherwise."""
+    from deepgrp_b200 import _lib
+    labels = np.empty(length, dtype=np.uint8)
+    rows = np.empty((n_rows, 3), dtype=np.int64)
+    _lib.check(_lib.lib().dgrp_predict_codes_dev_results(ctx.handle, _lib.ptr(labels), length, _lib.ptr(rows),
+                                                         n_rows))
+
+    def sample(n, k, seed):
+        return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "labels.npy"), labels[sample(length, DUMP_LABELS, 0)].astype(np.float32))
+    np.save(os.path.join(out_dir, "label_counts.npy"), np.bincount(labels, minlength=5).astype(np.float64))
+    np.save(os.path.join(out_dir, "rows.npy"), rows[sample(n_rows, DUMP_ROWS, 1)].astype(np.float64))
+
+
 def numa_bind(local_rank):
     """Run this rank (and what it allocates: first touch decides where pinned buffers live) on the CPUs local to
     its GPU, as `numactl --cpunodebind` would.  Returns a short description for the JSON line."""
@@ -304,10 +328,10 @@ def run_ours(args, rank, world, local_rank):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return [float(x) for x in t.cpu()]
 
-    def measure(weights, L, steps, warmup, sample_clocks):
+    def measure(weights, L, steps, warmup, sample_clocks, dump_dir=None):
         """One record of L bases per rank: `value` leg (codes resident in HBM, CUDA events on the library's
         stream) and `e2e` leg (FASTA text in pinned host memory -> TSV text on the host, through the public
-        streaming API, wall clock)."""
+        streaming API, wall clock).  With `dump_dir`, rank 0 writes the last `value` step's outputs there."""
         handle = weights.device_handle(ctx)
         codes = synth_codes(L, [1, rank])
         d_codes = torch.from_numpy(codes).cuda()
@@ -358,6 +382,8 @@ def run_ours(args, rank, world, local_rank):
         launches = ctx.launch_count() - launches0
         clocks = sampler.stop() if sampler else None
         used_kernel = ctx.get_int("forward_used_tc")
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, ctx, L, int(n_rows.value))
         for _ in range(max(1, min(warmup, 2))):
             st = e2e_step()
         barrier()
@@ -378,7 +404,7 @@ def run_ours(args, rank, world, local_rank):
 
     weights = make_weights(args)
     L = args.bases
-    main = measure(weights, L, args.steps, args.warmup, True)
+    main = measure(weights, L, args.steps, args.warmup, True, args.dump_outputs)
     tflops_peak, hbm_peak, peak_kind = peaks()
     n_windows = len(range(0, L - args.vecsize, STEP))
     kernel_ms = main["stages_ms"]["forward_ms"]
@@ -675,7 +701,14 @@ def main():
     ap.add_argument("--shard", default="contig", choices=["contig", "chunk"],
                     help="contig (default): one record per rank, weak scaling; chunk: ONE record split by "
                          "position ranges over the ranks (BASELINE.json configs[2], strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last `value` step's labels and rows (rank 0) as .npy "
+                         "files in DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.shard != "contig"):
+        ap.error("--dump-outputs writes the outputs of the default run (--impl ours --shard contig)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -101,6 +101,7 @@ SIGNATURES = {
     "dgrp_fasta_stream_waits": (_I, [_P, ctypes.POINTER(_D)]),
     "dgrp_fasta_stream_close": (_I, [_P]),
     "dgrp_predict_codes_dev": (_I, [_P, _P, _P, _L, _I, _I, _I, _I, _I, _I, _PL]),
+    "dgrp_predict_codes_dev_results": (_I, [_P, _P, _L, _P, _L]),
     "dgrp_predict_range_dev": (_I, [_P, _P, _P, _L, _L, _L, _L, _L, _I, _I, _I, _P, _P]),
     "dgrp_finish_record_dev": (_I, [_P, _P, _P, _L, _I, _I, _I, _I, _PL]),
     "dgrp_filter_segments": (_I, [_P, _P, _L, _L]),

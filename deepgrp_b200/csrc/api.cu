@@ -29,6 +29,7 @@ void set_error(const char *fmt, ...) {
 }
 
 int DevBuf::reserve(size_t bytes) {
+  ++reserves;
   if (bytes <= cap && p) return DGRP_OK;
   if (bytes < 256) bytes = 256;
   if (p) { cudaFree(p); p = nullptr; cap = 0; }
@@ -1043,6 +1044,7 @@ int dgrp_predict_codes_dev(dgrp_ctx *c, dgrp_model *m, const uint8_t *d_codes, i
   Use use(c->device);
   const int64_t launches0 = c->launches;
   *n_rows = 0;
+  c->codes_dev_length = -1;
   stamp(c, 0);
   stamp(c, 1);
   DGRP_CHECK(core_predict(c, m, d_codes, length, step, batch_size, compat, use_mss != 0));
@@ -1053,7 +1055,29 @@ int dgrp_predict_codes_dev(dgrp_ctx *c, dgrp_model *m, const uint8_t *d_codes, i
   if (length > 0) rc = core_rows(c, length, 0, 0, false, nullptr, 0, n_rows);
   stamp(c, 5);
   finish_timings(c, launches0);
+  if (rc == DGRP_OK) {
+    c->codes_dev_length = length;
+    c->codes_dev_rows = *n_rows;
+    c->codes_dev_reserves[0] = c->labels2.reserves;
+    c->codes_dev_reserves[1] = c->segs.reserves;
+  }
   return rc;
+}
+
+int dgrp_predict_codes_dev_results(dgrp_ctx *c, uint8_t *labels, int64_t length, int64_t *rows, int64_t n_rows) {
+  Use use(c->device);
+  DGRP_REQUIRE(c->codes_dev_length >= 0 && c->codes_dev_reserves[0] == c->labels2.reserves &&
+                   c->codes_dev_reserves[1] == c->segs.reserves,
+               "no dgrp_predict_codes_dev result to fetch: none ran, or another call has used its buffers since");
+  DGRP_REQUIRE(length == c->codes_dev_length && n_rows == c->codes_dev_rows,
+               "the last dgrp_predict_codes_dev has length %lld and %lld rows", (long long)c->codes_dev_length,
+               (long long)c->codes_dev_rows);
+  if (labels && length > 0)
+    DGRP_CUDA(cudaMemcpyAsync(labels, c->labels2.p, (size_t)length, cudaMemcpyDeviceToHost, c->stream));
+  if (rows && n_rows > 0)
+    DGRP_CUDA(cudaMemcpyAsync(rows, c->segs.p, (size_t)n_rows * 24, cudaMemcpyDeviceToHost, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  return DGRP_OK;
 }
 
 }  // extern "C"

@@ -40,6 +40,9 @@ void set_error(const char *fmt, ...);
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  // reserve() calls so far.  Every call that writes a buffer reserves it first, so an unchanged count means
+  // unchanged contents (dgrp_predict_codes_dev_results relies on it).
+  uint64_t reserves = 0;
   int reserve(size_t bytes);
   void release();
   template <typename T>
@@ -125,6 +128,11 @@ struct dgrp_ctx {
   // results of the last dgrp_predict_fasta (fetched with dgrp_fasta_rows / dgrp_fasta_records)
   std::vector<dgrp_row_t> fa_rows;
   std::vector<int64_t> fa_hdr_off, fa_hdr_len, fa_startpos, fa_length, fa_tsv_off, fa_tsv_len, fa_owner;
+  // the last dgrp_predict_codes_dev: record length, row count, and the reserve counts of labels2 and segs when it
+  // returned (its labels in labels2 and rows in segs are fetched with dgrp_predict_codes_dev_results while neither
+  // buffer has been reserved since)
+  int64_t codes_dev_length = -1, codes_dev_rows = 0;
+  uint64_t codes_dev_reserves[2] = {};
   int shard_rank = 0, shard_world = 1;   // contig sharding of dgrp_predict_fasta* (dgrp_ctx_set_int)
   dgrp::PinBuf tsv_host;     // finished TSV text of the last dgrp_predict_fasta_tsv
   int64_t tsv_len = 0;

@@ -293,6 +293,11 @@ int dgrp_fasta_stream_close(dgrp_fasta_stream *stream);
 int dgrp_predict_codes_dev(dgrp_ctx *ctx, dgrp_model *model, const uint8_t *d_codes,
                            int64_t length, int step, int batch_size, int use_mss,
                            int min_mss_len, int xdrop_len, int compat, int64_t *n_rows);
+/* Copies what the last dgrp_predict_codes_dev left on the device to the host: the final label of each of its
+ * `length` positions (labels, may be NULL) and its n_rows rows as (start, end, label) int64 triples (rows, may be
+ * NULL).  `length` and `n_rows` must be those of that call, and no call that overwrites them (one computing labels
+ * or rows) may have run on the context since, even one that failed (DGRP_E_ARG otherwise). */
+int dgrp_predict_codes_dev_results(dgrp_ctx *ctx, uint8_t *labels, int64_t length, int64_t *rows, int64_t n_rows);
 
 #ifdef __cplusplus
 }

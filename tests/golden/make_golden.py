@@ -1,4 +1,4 @@
-"""Generate tests/golden/native_vectors.npz from the REFERENCE's own compiled natives
+"""Generate tests/golden/native_vectors.npz and reference_trials.npz from the REFERENCE's own compiled natives
 (oracle/_ref, built by oracle/build_ref.py from /root/reference).  Run in the build container:
 
     python oracle/build_ref.py && python tests/golden/make_golden.py
@@ -13,6 +13,38 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import build_ref  # noqa: E402
+
+TRIAL_MSS_PARAMS = ((0, -1), (3, 2), (50, 50))
+
+
+def reference_trials():
+    """The seeded inputs of tests/test_oracle.py::test_oracle_against_compiled_reference: 40 trials of
+    (scores, labels, text)."""
+    rng = np.random.default_rng(9)
+    for _ in range(40):
+        n = int(rng.integers(1, 3000))
+        s = rng.normal(size=n) * 3 - rng.random()
+        lab = rng.integers(0, 5, size=n)
+        text = "".join(np.array(list("ACGTNacgtnX"))[rng.integers(0, 11, size=n)])
+        yield s, lab, text
+
+
+def trial_vectors(seq, mss):
+    """find_mss_labels (as its argmax: the rows are one-hot), one_hot_encode_dna_sequence and yield_segments of
+    `seq` / `mss` (the reference modules, or the oracle) on reference_trials()."""
+    out = {}
+    for i, (s, lab, text) in enumerate(reference_trials()):
+        for k, (ml, xd) in enumerate(TRIAL_MSS_PARAMS):
+            res = np.asarray(mss.find_mss_labels(s, lab, 5, ml, xd))
+            assert ((res == 0) | (res == 1)).all() and (res.sum(axis=1) == 1).all()
+            out["mss_%d_%d" % (i, k)] = res.argmax(axis=1).astype(np.uint8)
+        if set(text) != {"N"}:
+            st, fwd = seq.one_hot_encode_dna_sequence(text)
+            out["enc_start_%d" % i] = np.int64(st)
+            out["enc_fwd_%d" % i] = np.asarray(fwd)
+        out["seg_%d" % i] = np.array(list(seq.yield_segments(lab, 5)), dtype=np.int64).reshape(-1, 3)
+    out["n"] = np.int64(i + 1)
+    return out
 
 
 def main():
@@ -77,6 +109,9 @@ def main():
     out["mss_n"] = np.int64(k)
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "native_vectors.npz")
     np.savez_compressed(path, **out)
+    print("wrote", path, os.path.getsize(path), "bytes")
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_trials.npz")
+    np.savez_compressed(path, **trial_vectors(ref_seq, ref_mss))
     print("wrote", path, os.path.getsize(path), "bytes")
 
 

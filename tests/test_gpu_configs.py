@@ -305,6 +305,10 @@ def test_chunk_sharding_device_entry_points(dg):
     n_whole = ctypes.c_int64(0)
     _lib.check(lib.dgrp_predict_codes_dev(ctx.handle, h, ctypes.c_void_p(d_codes.data_ptr()), L, 50, 256, 1, 50, 50,
                                           _lib.COMPAT_REFERENCE, ctypes.byref(n_whole)))
+    whole_lab = np.empty(L, dtype=np.uint8)
+    whole_rows = np.empty((n_whole.value, 3), dtype=np.int64)
+    _lib.check(lib.dgrp_predict_codes_dev_results(ctx.handle, _lib.ptr(whole_lab), L, _lib.ptr(whole_rows),
+                                                  n_whole.value))
     full_lab = torch.empty(L, dtype=torch.uint8, device="cuda")
     full_sc = torch.empty(L, dtype=torch.float32, device="cuda")
     for (a, b) in sharding.split_positions(L, 3):
@@ -324,8 +328,13 @@ def test_chunk_sharding_device_entry_points(dg):
     _lib.check(lib.dgrp_finish_record_dev(ctx.handle, ctypes.c_void_p(full_lab.data_ptr()),
                                           ctypes.c_void_p(full_sc.data_ptr()), L, 5, 1, 50, 50, ctypes.byref(n_rows)))
     assert n_rows.value == n_whole.value and n_rows.value > 0
+    with pytest.raises(_lib.DeepgrpError):      # dgrp_finish_record_dev has overwritten those results
+        _lib.check(lib.dgrp_predict_codes_dev_results(ctx.handle, _lib.ptr(whole_lab), L, None, 0))
     out, rows = sharding.finish_record(full_lab.cpu().numpy(), full_sc.cpu().numpy(), 5, True, 50, 50, 0)
     assert rows.size == n_rows.value
+    # what dgrp_predict_codes_dev left on the device (bench.py --dump-outputs) is the whole-record result
+    assert np.array_equal(whole_lab, out)
+    assert np.array_equal(whole_rows, np.stack([rows["start"], rows["end"], rows["label"]], axis=1))
 
 
 def test_predict_complete_from_files_on_disk(dg, oracle, tmp_path):

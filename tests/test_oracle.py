@@ -141,25 +141,33 @@ def test_oracle_fasta_reader(oracle, tmp_path):
 
 
 def test_oracle_against_compiled_reference(oracle):
+    """The oracle against the reference's natives on 40 seeded trials: live against oracle/_ref when it is built,
+    otherwise against their outputs stored by tests/golden/make_golden.py (reference_trials.npz)."""
+    import importlib.util
     from oracle import build_ref
+    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
+    make_golden = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(make_golden)
     mods = build_ref.load()
-    if mods is None:
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
-    ref_seq, ref_mss = mods
-    rng = np.random.default_rng(9)
-    for trial in range(40):
-        n = int(rng.integers(1, 3000))
-        s = rng.normal(size=n) * 3 - rng.random()
-        lab = rng.integers(0, 5, size=n)
-        for ml, xd in ((0, -1), (3, 2), (50, 50)):
-            assert np.array_equal(ref_mss.find_mss_labels(s, lab, 5, ml, xd),
-                                  oracle.find_mss_labels(s, lab, 5, ml, xd))
-        text = "".join(np.array(list("ACGTNacgtnX"))[rng.integers(0, 11, size=n)])
-        a, b = ref_seq.one_hot_encode_dna_sequence(text) if set(text) != {"N"} else (None, None), None
-        if a[0] is not None:
+    stored = os.path.join(HERE, "golden", "reference_trials.npz")
+    if mods is not None:
+        ref = make_golden.trial_vectors(*mods)
+    elif os.path.exists(stored):
+        ref = np.load(stored)
+    else:
+        pytest.skip("neither oracle/_ref nor tests/golden/reference_trials.npz (both come from the reference's "
+                    "sources: python oracle/build_ref.py && python tests/golden/make_golden.py)")
+    assert int(ref["n"]) == 40
+    for i, (s, lab, text) in enumerate(make_golden.reference_trials()):
+        for k, (ml, xd) in enumerate(make_golden.TRIAL_MSS_PARAMS):
+            full = oracle.find_mss_labels(s, lab, 5, ml, xd)
+            assert ((full == 0) | (full == 1)).all() and (full.sum(axis=1) == 1).all()
+            assert np.array_equal(full.argmax(axis=1), ref["mss_%d_%d" % (i, k)]), (i, k)
+        if set(text) != {"N"}:
             st, fwd = oracle.one_hot_encode_dna_sequence(text)
-            assert st == a[0] and np.array_equal(fwd, a[1])
-        assert list(ref_seq.yield_segments(lab, 5)) == list(oracle.yield_segments(lab, 5))
+            assert st == int(ref["enc_start_%d" % i]) and np.array_equal(fwd, ref["enc_fwd_%d" % i]), i
+        segs = np.array(list(oracle.yield_segments(lab, 5)), dtype=np.int64).reshape(-1, 3)
+        assert np.array_equal(segs, ref["seg_%d" % i]), i
 
 
 def test_oracle_lstm_engines_agree(oracle):
