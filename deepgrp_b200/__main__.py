@@ -3,7 +3,7 @@
 (reference ``deepgrp/__main__.py``).  Same options (``-b -s -x -l -t --xla -v``, ``predict
 --output --no_use_mss``); ``-t`` and ``--xla`` are accepted and ignored (there is no TensorFlow).
 The README form ``deepgrp <modelfile> <fastafile>...`` (reference ``README.rst:92-98``) is accepted
-as well as the ``predict`` sub-command.  ``train`` is out of scope.
+as well as the ``predict`` sub-command.  ``train`` trains a GRU model on the GPU (``deepgrp_b200.training``).
 """
 from __future__ import annotations
 
@@ -126,7 +126,7 @@ class CommandLineParser:
         sub = {name: commands.add_parser(name=name, description=text,
                                          formatter_class=argparse.ArgumentDefaultsHelpFormatter)
                for name, text in (("predict", "predict using a deepgrp model"),
-                                  ("train", "Train a deepgrp model (not part of deepgrp_b200: parsed, then refused)"))}
+                                  ("train", "Train a deepgrp model"))}
         sub["predict"].add_argument("model", type=str, help="Keras model in HDF5 format (or .npz weights)")
         sub["predict"].add_argument("FASTA", nargs="+", type=str, help="Fasta input files")
         sub["predict"].add_argument("--output", type=str, default="-", help="Output filename")
@@ -135,10 +135,13 @@ class CommandLineParser:
         sub["predict"].add_argument("--stepwise", action="store_true",
                                     help="Run the reference's five Python-level calls per record instead of the "
                                          "fused whole-record GPU call")
-        for name in ("parameter", "trainfile", "validfile", "bedfile"):
-            sub["train"].add_argument(name, type=str)
-        sub["train"].add_argument("--logdir", type=str, default=".")
-        sub["train"].add_argument("--modelfile", type=str, default="model.hdf5")
+        for name, text in (("parameter", "TOML file of hyper-parameters (Options)"),
+                           ("trainfile", "one-hot .npz of the training chromosome (preprocess_sequence)"),
+                           ("validfile", "one-hot .npz of the validation chromosome"),
+                           ("bedfile", "repeat annotations: chromosome, begin, end, repeat number")):
+            sub["train"].add_argument(name, type=str, help=text)
+        sub["train"].add_argument("--logdir", type=str, default=".", help="Directory for best.hdf5 and history.tsv")
+        sub["train"].add_argument("--modelfile", type=str, default="model.hdf5", help="Keras HDF5 file to write")
 
     def parse_args(self, argv=None) -> "CommandLineParser":
         """Parse command line arguments."""
@@ -223,9 +226,43 @@ class CommandLineParser:
             outstream.close()
 
     @staticmethod
-    def train(args, options):  # pragma: no cover
-        raise SystemExit("deepgrp_b200 implements the prediction path only; use the reference "
-                         "package to train")
+    def train(args: argparse.Namespace, options: dgmodel.Options):
+        """Train a model (reference ``deepgrp/__main__.py:299-351``): TOML hyper-parameters, the two one-hot
+        ``.npz`` files, their labels from the annotation table, ``training``, then the Keras HDF5 model file."""
+        names = ("parameter", "trainfile", "validfile", "bedfile", "logdir", "modelfile")
+        if any(getattr(args, name, None) is None for name in names):
+            raise SystemExit("usage: deepgrp train parameter trainfile validfile bedfile [--logdir LOGDIR] "
+                             "[--modelfile MODELFILE]")
+        from . import hdf5
+        from . import preprocessing as dgprep
+        from . import training as dgtrain
+        options = _train_options(args.parameter, options)
+        data = []
+        for path in (args.trainfile, args.validfile):
+            fwd, _ = dgprep.load_onehot_npz(path)
+            dgtrain.onehot_to_codes(fwd)                      # columns must be one-hot (ValueError)
+            truelbl = dgprep.preprocess_y(args.bedfile, chromosome_name(path), fwd.shape[1],
+                                          options.repeats_to_search)
+            data.append(dgprep.Data(*dgprep.drop_start_end_n(fwd, truelbl)))
+        model = dgmodel.create_model(options)
+        _LOG.info("Training on %s (%d bases), validating on %s (%d bases)", args.trainfile, data[0].fwd.shape[1],
+                  args.validfile, data[1].fwd.shape[1])
+        dgtrain.training(tuple(data), options, model, args.logdir)
+        hdf5.save_keras_model(args.modelfile, model)
+        _LOG.info("Model written to %s", args.modelfile)
+
+
+def chromosome_name(path: str) -> str:
+    """The chromosome a one-hot file holds: its base name up to the first ``.`` (``chr1.fa.gz.npz`` -> ``chr1``)."""
+    return os.path.basename(path).split(".", 1)[0]
+
+
+def _train_options(parameter: str, cli_options: dgmodel.Options) -> dgmodel.Options:
+    """Options of ``deepgrp train``: the TOML file's keys, and the command line's values for what it lacks."""
+    import tomllib
+    with open(parameter, "rb") as fh:
+        parsed = tomllib.load(fh)
+    return dgmodel.Options(**{**cli_options.todict(), **parsed})
 
 
 def main():

@@ -53,6 +53,7 @@ _P = ctypes.c_void_p
 _I = ctypes.c_int
 _L = ctypes.c_int64
 _D = ctypes.c_double
+_F = ctypes.c_float
 _PL = ctypes.POINTER(ctypes.c_int64)
 _PI = ctypes.POINTER(ctypes.c_int)
 
@@ -106,7 +107,17 @@ SIGNATURES = {
     "dgrp_finish_record_dev": (_I, [_P, _P, _P, _L, _I, _I, _I, _I, _PL]),
     "dgrp_filter_segments": (_I, [_P, _P, _L, _L]),
     "dgrp_confusion_matrix": (_I, [_P, _P, _P, _L, _P]),
+    "dgrp_train_create": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _I, _F, _F, _F, _F, _F,
+                               ctypes.POINTER(_P)]),
+    "dgrp_train_set_data": (_I, [_P, _I, _P, _P, _L]),
+    "dgrp_train_step": (_I, [_P, _P, _P, _L, ctypes.POINTER(_F)]),
+    "dgrp_train_eval": (_I, [_P, _I, _P, _L, ctypes.POINTER(_F), _P]),
+    "dgrp_train_get_weights": (_I, [_P, _P, _P, _P, _P, _P, _P]),
+    "dgrp_train_get_grads": (_I, [_P, _P, _P, _P, _P, _P, _P]),
+    "dgrp_train_timings": (_I, [_P, _P]),
+    "dgrp_train_destroy": (_I, [_P]),
 }
+OPT_RMSPROP, OPT_ADAM = 0, 1
 
 _lib: Optional[ctypes.CDLL] = None
 _lock = threading.Lock()

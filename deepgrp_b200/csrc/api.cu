@@ -1080,6 +1080,208 @@ int dgrp_predict_codes_dev_results(dgrp_ctx *c, uint8_t *labels, int64_t length,
   return DGRP_OK;
 }
 
+/* -------------------------------------- training --------------------------------------- */
+
+// the Keras arrays <-> the trainer's flat parameter vector (TrainLayout)
+static void train_pack(const dgrp_trainer *tr, std::vector<float> &flat, const float *kernel, const float *recurrent,
+                       const float *bias, const float *att_scale, const float *ff_kernel, const float *ff_bias) {
+  const TrainLayout &L = tr->L;
+  const int U = tr->U, C = tr->C;
+  flat.assign(L.n, 0.f);
+  std::copy(kernel, kernel + 15 * U, flat.begin() + L.oK);
+  std::copy(recurrent, recurrent + 3 * U * U, flat.begin() + L.oR);
+  std::copy(bias, bias + 6 * U, flat.begin() + L.oB);
+  if (tr->attention) std::copy(att_scale, att_scale + U, flat.begin() + L.oS);
+  std::copy(ff_kernel, ff_kernel + L.F * C, flat.begin() + L.oF);
+  std::copy(ff_bias, ff_bias + C, flat.begin() + L.oFB);
+}
+
+static int train_unpack(dgrp_trainer *tr, const DevBuf &src, float *kernel, float *recurrent, float *bias,
+                        float *att_scale, float *ff_kernel, float *ff_bias) {
+  dgrp_ctx *c = tr->ctx;
+  const TrainLayout &L = tr->L;
+  const int U = tr->U, C = tr->C;
+  std::vector<float> flat(L.n);
+  DGRP_CUDA(cudaMemcpyAsync(flat.data(), src.p, (size_t)L.n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  auto put = [&](float *dst, int off, int count) { if (dst) std::copy(flat.begin() + off, flat.begin() + off + count, dst); };
+  put(kernel, L.oK, 15 * U);
+  put(recurrent, L.oR, 3 * U * U);
+  put(bias, L.oB, 6 * U);
+  if (tr->attention) put(att_scale, L.oS, U);
+  put(ff_kernel, L.oF, L.F * C);
+  put(ff_bias, L.oFB, C);
+  return DGRP_OK;
+}
+
+int dgrp_train_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classes, int attention,
+                      const float *kernel, const float *recurrent, const float *bias, const float *att_scale,
+                      const float *ff_kernel, const float *ff_bias, int optimizer, float learning_rate, float rho,
+                      float momentum, float epsilon, float dropout, dgrp_trainer **out) {
+  Use use(c->device);
+  *out = nullptr;
+  if (rnn != 0) {
+    set_error("training supports rnn=\"GRU\" only (LSTM is not implemented)");
+    return DGRP_E_UNSUPPORTED;
+  }
+  DGRP_CHECK(train_check_shape(vecsize, units, n_classes, attention != 0));
+  DGRP_REQUIRE(optimizer == DGRP_OPT_RMSPROP || optimizer == DGRP_OPT_ADAM,
+               "optimizer must be DGRP_OPT_RMSPROP or DGRP_OPT_ADAM, got %d", optimizer);
+  DGRP_REQUIRE(dropout >= 0.f && dropout < 1.f, "dropout must be in [0, 1), got %g", (double)dropout);
+  DGRP_REQUIRE(learning_rate >= 0.f && epsilon >= 0.f && rho >= 0.f && momentum >= 0.f,
+               "learning_rate, rho, momentum and epsilon must not be negative");
+  DGRP_REQUIRE(kernel && recurrent && bias && ff_kernel && ff_bias && (!attention || att_scale),
+               "a weight array is NULL");
+  dgrp_trainer *tr = new dgrp_trainer();
+  tr->ctx = c;
+  tr->T = vecsize; tr->U = units; tr->C = n_classes; tr->attention = attention != 0;
+  tr->optimizer = optimizer; tr->lr = learning_rate; tr->rho = rho; tr->momentum = momentum;
+  tr->epsilon = epsilon; tr->dropout = dropout;
+  tr->L = make_train_layout(units, n_classes, tr->attention);
+  std::vector<float> flat;
+  train_pack(tr, flat, kernel, recurrent, bias, att_scale, ff_kernel, ff_bias);
+  const size_t bytes = (size_t)tr->L.n * sizeof(float);
+  int rc = DGRP_OK;
+  for (auto &e : tr->ev)
+    if (rc == DGRP_OK && cudaEventCreate(&e) != cudaSuccess) { set_error("cudaEventCreate failed"); rc = DGRP_E_CUDA; }
+  if (rc == DGRP_OK) rc = tr->w.reserve(bytes);
+  if (rc == DGRP_OK) rc = tr->g.reserve(bytes);
+  if (rc == DGRP_OK) rc = tr->s1.reserve(bytes);
+  if (rc == DGRP_OK) rc = tr->s2.reserve(bytes);
+  if (rc == DGRP_OK && cudaMemcpyAsync(tr->w.p, flat.data(), bytes, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
+    set_error("uploading the weights failed");
+    rc = DGRP_E_CUDA;
+  }
+  if (rc == DGRP_OK && (cudaMemsetAsync(tr->g.p, 0, bytes, c->stream) != cudaSuccess ||
+                        cudaMemsetAsync(tr->s1.p, 0, bytes, c->stream) != cudaSuccess ||
+                        cudaMemsetAsync(tr->s2.p, 0, bytes, c->stream) != cudaSuccess)) {
+    set_error("clearing the optimiser state failed");
+    rc = DGRP_E_CUDA;
+  }
+  if (rc == DGRP_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) {
+    set_error("creating the trainer failed");
+    rc = DGRP_E_CUDA;
+  }
+  if (rc != DGRP_OK) {
+    dgrp_train_destroy(tr);
+    return rc;
+  }
+  *out = tr;
+  return DGRP_OK;
+}
+
+int dgrp_train_set_data(dgrp_trainer *tr, int which, const uint8_t *codes, const uint8_t *ymask, int64_t length) {
+  dgrp_ctx *c = tr->ctx;
+  Use use(c->device);
+  DGRP_REQUIRE(which == 0 || which == 1, "which must be 0 (training) or 1 (validation), got %d", which);
+  DGRP_REQUIRE(length >= tr->T, "record length %lld is shorter than vecsize %d", (long long)length, tr->T);
+  DGRP_REQUIRE(codes && ymask, "codes and ymask must not be NULL");
+  for (int64_t i = 0; i < length; ++i) {
+    DGRP_REQUIRE(codes[i] <= 4, "code %d at position %lld is not a base code 0..4", codes[i], (long long)i);
+    DGRP_REQUIRE((ymask[i] >> tr->C) == 0, "label mask 0x%x at position %lld names a class >= %d", ymask[i],
+                 (long long)i, tr->C);
+  }
+  tr->length[which] = -1;
+  DGRP_CHECK(tr->codes[which].reserve((size_t)length));
+  DGRP_CHECK(tr->ymask[which].reserve((size_t)length));
+  DGRP_CUDA(cudaMemcpyAsync(tr->codes[which].p, codes, (size_t)length, cudaMemcpyHostToDevice, c->stream));
+  DGRP_CUDA(cudaMemcpyAsync(tr->ymask[which].p, ymask, (size_t)length, cudaMemcpyHostToDevice, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  tr->length[which] = length;
+  return DGRP_OK;
+}
+
+static int train_upload_starts(dgrp_trainer *tr, int which, const int64_t *starts, int64_t n) {
+  dgrp_ctx *c = tr->ctx;
+  DGRP_REQUIRE(which == 0 || which == 1, "which must be 0 (training) or 1 (validation), got %d", which);
+  DGRP_REQUIRE(tr->length[which] >= 0, "no %s data set: call dgrp_train_set_data first",
+               which ? "validation" : "training");
+  DGRP_REQUIRE(n >= 1, "n must be at least 1, got %lld", (long long)n);
+  DGRP_REQUIRE(starts, "starts must not be NULL");
+  const int64_t last = tr->length[which] - tr->T;
+  for (int64_t b = 0; b < n; ++b)
+    DGRP_REQUIRE(starts[b] >= 0 && starts[b] <= last, "window start %lld (window %lld) is outside [0, %lld]",
+                 (long long)starts[b], (long long)b, (long long)last);
+  DGRP_CHECK(tr->starts.reserve((size_t)n * sizeof(int64_t)));
+  DGRP_CUDA(cudaMemcpyAsync(tr->starts.p, starts, (size_t)n * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+  return DGRP_OK;
+}
+
+static float train_mean_loss(const std::vector<float> &lpart, int64_t n, int T) {
+  double s = 0.0;
+  for (int64_t b = 0; b < n; ++b) s += lpart[b];
+  return (float)(s / ((double)n * T));
+}
+
+int dgrp_train_step(dgrp_trainer *tr, const int64_t *starts, const uint8_t *keep, int64_t n, float *loss) {
+  dgrp_ctx *c = tr->ctx;
+  Use use(c->device);
+  DGRP_CHECK(train_upload_starts(tr, 0, starts, n));
+  DGRP_REQUIRE(keep, "keep must not be NULL");
+  DGRP_CHECK(tr->keep.reserve((size_t)n * 10));
+  DGRP_CUDA(cudaMemcpyAsync(tr->keep.p, keep, (size_t)n * 10, cudaMemcpyHostToDevice, c->stream));
+  DGRP_CHECK(train_run_step(c, tr, n, tr->starts.as<int64_t>(), tr->keep.as<uint8_t>()));
+  tr->h_lpart.resize((size_t)n);
+  DGRP_CUDA(cudaMemcpyAsync(tr->h_lpart.data(), tr->lpart.p, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost,
+                            c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  if (loss) *loss = train_mean_loss(tr->h_lpart, n, tr->T);
+  return DGRP_OK;
+}
+
+int dgrp_train_eval(dgrp_trainer *tr, int which, const int64_t *starts, int64_t n, float *loss, float *probs) {
+  dgrp_ctx *c = tr->ctx;
+  Use use(c->device);
+  DGRP_CHECK(train_upload_starts(tr, which, starts, n));
+  float *d_probs = nullptr;
+  if (probs) {
+    DGRP_CHECK(tr->probs.reserve((size_t)n * tr->T * tr->C * sizeof(float)));
+    d_probs = tr->probs.as<float>();
+  }
+  tr->h_lpart.resize((size_t)n);
+  DGRP_CHECK(train_run_eval(c, tr, which, n, tr->starts.as<int64_t>(), d_probs, tr->h_lpart.data()));
+  if (probs)
+    DGRP_CUDA(cudaMemcpyAsync(probs, d_probs, (size_t)n * tr->T * tr->C * sizeof(float), cudaMemcpyDeviceToHost,
+                              c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  if (loss) *loss = train_mean_loss(tr->h_lpart, n, tr->T);
+  return DGRP_OK;
+}
+
+int dgrp_train_get_weights(dgrp_trainer *tr, float *kernel, float *recurrent, float *bias, float *att_scale,
+                           float *ff_kernel, float *ff_bias) {
+  Use use(tr->ctx->device);
+  return train_unpack(tr, tr->w, kernel, recurrent, bias, att_scale, ff_kernel, ff_bias);
+}
+
+int dgrp_train_get_grads(dgrp_trainer *tr, float *kernel, float *recurrent, float *bias, float *att_scale,
+                         float *ff_kernel, float *ff_bias) {
+  Use use(tr->ctx->device);
+  return train_unpack(tr, tr->g, kernel, recurrent, bias, att_scale, ff_kernel, ff_bias);
+}
+
+int dgrp_train_timings(dgrp_trainer *tr, float *out5) {
+  Use use(tr->ctx->device);
+  DGRP_REQUIRE(tr->timed, "no training step has run");
+  DGRP_CUDA(cudaEventSynchronize(tr->ev[5]));
+  for (int i = 0; i < 5; ++i) DGRP_CUDA(cudaEventElapsedTime(&out5[i], tr->ev[i], tr->ev[i + 1]));
+  return DGRP_OK;
+}
+
+int dgrp_train_destroy(dgrp_trainer *tr) {
+  if (!tr) return DGRP_OK;
+  Use use(tr->ctx->device);
+  cudaStreamSynchronize(tr->ctx->stream);
+  DevBuf *bufs[] = {&tr->w, &tr->g, &tr->s1, &tr->s2, &tr->codes[0], &tr->codes[1], &tr->ymask[0], &tr->ymask[1],
+                    &tr->starts, &tr->keep, &tr->Hs, &tr->GS, &tr->D, &tr->avg, &tr->dhin, &tr->hpart,
+                    &tr->rpart, &tr->lpart, &tr->probs};
+  for (auto b : bufs) b->release();
+  for (auto &e : tr->ev)
+    if (e) cudaEventDestroy(e);
+  delete tr;
+  return DGRP_OK;
+}
+
 }  // extern "C"
 
 // positions [pos0, pos1) of a record from device codes: label + score into device buffers

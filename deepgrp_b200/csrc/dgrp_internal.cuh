@@ -146,6 +146,34 @@ struct dgrp_ctx {
 };
 
 namespace dgrp {
+// offsets into a trainer's flat parameter vector: the Keras arrays of a GRU model concatenated
+struct TrainLayout {
+  int F;                        // FF kernel rows (2U with attention, else U)
+  int oK, oR, oB, oS, oF, oFB;  // kernel [5,3U], recurrent [U,3U], bias [2,3U], scale [U], FF kernel [F,C], FF bias [C]
+  int n;                        // parameter count
+  int HP;                       // per-window head gradient floats: F*C + C + U
+};
+}  // namespace dgrp
+
+struct dgrp_trainer {
+  dgrp_ctx *ctx = nullptr;
+  int T = 0, U = 0, C = 0;
+  bool attention = false;
+  int optimizer = 0;
+  float lr = 0.f, rho = 0.f, momentum = 0.f, epsilon = 0.f, dropout = 0.f;
+  int64_t steps = 0;
+  int64_t length[2] = {-1, -1};   // record length of the training / validation data (-1: not set)
+  dgrp::TrainLayout L = {};
+  // parameters, gradients of the last step, optimiser state (RMSprop ms / mom, Adam m / v)
+  dgrp::DevBuf w, g, s1, s2;
+  dgrp::DevBuf codes[2], ymask[2], starts, keep;
+  dgrp::DevBuf Hs, GS, D, avg, dhin, hpart, rpart, lpart, probs;
+  std::vector<float> h_lpart;
+  cudaEvent_t ev[6] = {};   // forward | head | BPTT | reduction | update of the last step
+  bool timed = false;
+};
+
+namespace dgrp {
 
 struct Use {  // RAII: make the context's device current
   int prev = -1;
@@ -238,5 +266,15 @@ int run_segments(dgrp_ctx *c, const uint8_t *d_label, const int64_t *d_label64, 
                  int64_t *open_tail = nullptr);
 int launch_get_segments(dgrp_ctx *c, const int64_t *d_classes, int64_t size, int64_t startpos,
                         int64_t *d_out3);
+// train.cu
+constexpr int TR_CMAX = 8;   // classes a trainer supports
+TrainLayout make_train_layout(int U, int C, bool att);
+int train_check_shape(int T, int U, int C, bool att);
+// one training step on n windows of the training record (starts, keep on the device); leaves the gradients in
+// tr->g, the per-window losses in tr->lpart, and updates tr->w
+int train_run_step(dgrp_ctx *c, dgrp_trainer *tr, int64_t n, const int64_t *d_starts, const uint8_t *d_keep);
+// forward only, no dropout: per-window losses into h_lpart[n] (host), probabilities [n][T][C] into d_probs if set
+int train_run_eval(dgrp_ctx *c, dgrp_trainer *tr, int which, int64_t n, const int64_t *d_starts, float *d_probs,
+                   float *h_lpart);
 
 }  // namespace dgrp

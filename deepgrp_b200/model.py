@@ -11,7 +11,9 @@ Mirrors the parts of the reference's ``deepgrp/model.py`` that the prediction pa
 * ``ModelWeights`` stands where ``keras.Model`` stood: it has ``input_shape``/``output_shape``
   (used by the CLI, reference ``deepgrp/__main__.py:270`` and ``:75``) and ``predict_on_batch``.
 
-Training-only members (``_get_optimizer``, ``create_logdir``) are out of scope (SURVEY.md §8).
+The optimiser that ``_get_optimizer`` builds in the reference is chosen by ``deepgrp_b200.training`` from
+``Options.optimizer`` (``"RMSprop"`` or ``"Adam"``) and runs on the GPU; ``create_logdir`` has no counterpart (training
+writes into the ``logdir`` it is given).
 """
 from __future__ import annotations
 
@@ -25,7 +27,7 @@ _DEFAULTS: Dict[str, Any] = dict(
     # general (reference deepgrp/model.py:84-99)
     project_root_dir=".", repeats_to_search=[1, 2, 3, 4], vecsize=150, n_epochs=200,
     n_batches=250, early_stopping_th=10, batch_size=256, repeat_probability=0.3,
-    # optimiser (:103-112) -- carried for TOML compatibility, unused on the prediction path
+    # optimiser (:103-112) -- used by deepgrp_b200.training
     optimizer="RMSprop", learning_rate=0.001, momentum=0.9, rho=0.9, epsilon=1e-10,
     # network (:116-123)
     rnn="GRU", units=32, dropout=0.25, attention=False,

@@ -299,6 +299,43 @@ int dgrp_predict_codes_dev(dgrp_ctx *ctx, dgrp_model *model, const uint8_t *d_co
  * or rows) may have run on the context since, even one that failed (DGRP_E_ARG otherwise). */
 int dgrp_predict_codes_dev_results(dgrp_ctx *ctx, uint8_t *labels, int64_t length, int64_t *rows, int64_t n_rows);
 
+/* ---- training (deepgrp/training.py, deepgrp/model.py:202-215) ----------------------------------------------- */
+
+/* A trainer holds one GRU model's weights, its optimiser state and its training / validation records on the
+ * context's GPU.  Supported: rnn = 0 (GRU, reset_after=True) with 1 <= units <= 64, n_classes 2..8, with or without
+ * attention; LSTM and units > 64 give DGRP_E_UNSUPPORTED.  Every step is fp32 on CUDA cores and bit-reproducible on
+ * one GPU (no float atomics).  Weights and gradients use the Keras layouts of dgrp_model_create: kernel[5,3U],
+ * recurrent[U,3U], bias[2,3U], att_scale[U] (NULL without attention), ff_kernel[F,C], ff_bias[C].
+ * optimizer: DGRP_OPT_RMSPROP (momentum > 0: TF ApplyRMSProp, ms = rho ms + (1-rho) g^2, mom = momentum mom +
+ * lr g / sqrt(ms + eps), w -= mom; momentum = 0: w -= lr g / (sqrt(ms) + eps)) or DGRP_OPT_ADAM (Keras: beta1 0.9,
+ * beta2 0.999, w -= lr sqrt(1-beta2^t) / (1-beta1^t) m / (sqrt(v) + eps)).  dropout in [0, 1) is the GRU's input
+ * dropout (recurrent dropout 0). */
+#define DGRP_OPT_RMSPROP 0
+#define DGRP_OPT_ADAM 1
+typedef struct dgrp_trainer dgrp_trainer;
+int dgrp_train_create(dgrp_ctx *ctx, int rnn, int vecsize, int units, int n_classes, int attention,
+                      const float *kernel, const float *recurrent, const float *bias, const float *att_scale,
+                      const float *ff_kernel, const float *ff_bias, int optimizer, float learning_rate, float rho,
+                      float momentum, float epsilon, float dropout, dgrp_trainer **out);
+/* Uploads one record: which = 0 training, 1 validation; codes[L] base codes 0..4 (A, C, G, T, N: the row of the
+ * one-hot matrix), ymask[L] bit c set where class c is annotated (several bits where annotations overlap).
+ * DGRP_E_ARG when L < vecsize or a code / bit is out of range. */
+int dgrp_train_set_data(dgrp_trainer *tr, int which, const uint8_t *codes, const uint8_t *ymask, int64_t length);
+/* One step on n windows of the training record: window b covers [starts[b], starts[b] + vecsize); keep[b][dir][c]
+ * (0/1) is the input dropout mask of direction dir (0 forward, 1 reverse complement) for the channel c the GRU
+ * sees.  *loss receives the batch's mean loss before the update. */
+int dgrp_train_step(dgrp_trainer *tr, const int64_t *starts, const uint8_t *keep, int64_t n, float *loss);
+/* Forward only (no dropout, no update) on n windows of record `which`: *loss = mean loss, probs [n][T][C] or NULL. */
+int dgrp_train_eval(dgrp_trainer *tr, int which, const int64_t *starts, int64_t n, float *loss, float *probs);
+/* Current weights / gradients of the last step (before its update), host arrays in the Keras layouts above. */
+int dgrp_train_get_weights(dgrp_trainer *tr, float *kernel, float *recurrent, float *bias, float *att_scale,
+                           float *ff_kernel, float *ff_bias);
+int dgrp_train_get_grads(dgrp_trainer *tr, float *kernel, float *recurrent, float *bias, float *att_scale,
+                         float *ff_kernel, float *ff_bias);
+/* Device milliseconds of the last step's phases: forward, head, BPTT, weight-gradient reduction, update. */
+int dgrp_train_timings(dgrp_trainer *tr, float *out5);
+int dgrp_train_destroy(dgrp_trainer *tr);
+
 #ifdef __cplusplus
 }
 #endif
