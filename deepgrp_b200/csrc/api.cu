@@ -542,7 +542,8 @@ int dgrp_model_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classe
   }
   if (rnn == 1) att_scale = nullptr;   // attention is ignored for LSTM (deepgrp/model.py:308)
   DGRP_REQUIRE(vecsize > 0 && units > 0, "vecsize and units must be positive");
-  DGRP_REQUIRE(n_classes >= 2 && n_classes <= 5, "n_classes must be in [2, 5], got %d", n_classes);
+  DGRP_REQUIRE(n_classes >= MODEL_CMIN && n_classes <= MODEL_CMAX, "n_classes must be in [%d, %d], got %d",
+               MODEL_CMIN, MODEL_CMAX, n_classes);
   if (units > 128) {
     set_error("units=%d not supported by the CUDA forward (max 128)", units);
     return DGRP_E_UNSUPPORTED;

@@ -11,6 +11,10 @@
 
 namespace dgrp {
 
+// class counts a model may have: the prediction kernels' output layout holds at most 5 classes, and the trainer
+// accepts only models that prediction can run
+constexpr int MODEL_CMIN = 2, MODEL_CMAX = 5;
+
 void set_error(const char *fmt, ...);
 
 #define DGRP_CUDA(call)                                                                      \
@@ -267,7 +271,7 @@ int run_segments(dgrp_ctx *c, const uint8_t *d_label, const int64_t *d_label64, 
 int launch_get_segments(dgrp_ctx *c, const int64_t *d_classes, int64_t size, int64_t startpos,
                         int64_t *d_out3);
 // train.cu
-constexpr int TR_CMAX = 8;   // classes a trainer supports
+constexpr int TR_CMAX = 8;   // classes the head kernel's per-thread arrays hold (>= MODEL_CMAX)
 TrainLayout make_train_layout(int U, int C, bool att);
 int train_check_shape(int T, int U, int C, bool att);
 // one training step on n windows of the training record (starts, keep on the device); leaves the gradients in

@@ -1,5 +1,5 @@
-// Training of GRU models (rnn="GRU", reset_after=True, units <= 64, n_classes <= 8): forward with saved state,
-// loss + head backward, BPTT, deterministic weight-gradient reduction and the optimiser update, all fp32 on CUDA
+// Training of GRU models (rnn="GRU", reset_after=True, units <= 64, n_classes <= MODEL_CMAX): forward with saved
+// state, loss + head backward, BPTT, deterministic weight-gradient reduction and the optimiser update, all fp32 on CUDA
 // cores.  The model is the one forward.cu computes (SURVEY.md section 3.2); the loss is Keras'
 // categorical_crossentropy on the softmax probabilities, averaged over every position of the batch.
 //
@@ -31,6 +31,7 @@ constexpr int TR_UMAX = 64;
 constexpr int TR_KAMAX = TR_UMAX + 6;   // reduction rows: h_prev[U], 1 (bias), one-hot x dropout scale [5]
 constexpr int TR_TILE = 32;         // reduction items staged per pass
 constexpr int TR_EVAL_CHUNK = 1024; // windows per forward pass of an evaluation
+static_assert(TR_CMAX >= MODEL_CMAX, "the head kernel holds every class of a model in registers");
 
 struct TrainArgs {
   int T, U, C, att, n;
@@ -472,7 +473,11 @@ int train_check_shape(int T, int U, int C, bool att) {
     return DGRP_E_UNSUPPORTED;
   }
   DGRP_REQUIRE(U >= 1 && T >= 1, "vecsize and units must be positive");
-  DGRP_REQUIRE(C >= 2 && C <= TR_CMAX, "n_classes must be in [2, %d], got %d", TR_CMAX, C);
+  DGRP_REQUIRE(C >= MODEL_CMIN, "n_classes must be at least %d, got %d", MODEL_CMIN, C);
+  if (C > MODEL_CMAX) {
+    set_error("training supports n_classes <= %d, the most prediction can run, got %d", MODEL_CMAX, C);
+    return DGRP_E_UNSUPPORTED;
+  }
   if (head_smem(T, U, C, att) > 200 * 1024) {
     set_error("vecsize %d needs too much shared memory in the training head kernel", T);
     return DGRP_E_UNSUPPORTED;

@@ -4,7 +4,8 @@ The reference builds two ``tf.data`` datasets from ``fetch_batch`` and calls ``k
 loop runs through the CUDA trainer of ``csrc/train.cu`` (``dgrp_train_*``): the windows of a batch are never
 materialised -- the sampler hands the GPU window starts and input-dropout masks, the record's base codes and label
 masks are uploaded once -- and the forward, backward and optimiser update are CUDA kernels (fp32, bit-reproducible
-on one GPU).  Supported: ``rnn="GRU"`` with ``units <= 64`` and at most 8 classes; anything else is refused.
+on one GPU).  Supported: ``rnn="GRU"`` with ``units <= 64`` and 2 to 5 classes, the models prediction runs; anything
+else is refused when the ``Trainer`` is created, before the first step.
 
 Rules of this port where the reference's exact behaviour is not available (README.md lists them):
 

@@ -302,9 +302,9 @@ int dgrp_predict_codes_dev_results(dgrp_ctx *ctx, uint8_t *labels, int64_t lengt
 /* ---- training (deepgrp/training.py, deepgrp/model.py:202-215) ----------------------------------------------- */
 
 /* A trainer holds one GRU model's weights, its optimiser state and its training / validation records on the
- * context's GPU.  Supported: rnn = 0 (GRU, reset_after=True) with 1 <= units <= 64, n_classes 2..8, with or without
- * attention; LSTM and units > 64 give DGRP_E_UNSUPPORTED.  Every step is fp32 on CUDA cores and bit-reproducible on
- * one GPU (no float atomics).  Weights and gradients use the Keras layouts of dgrp_model_create: kernel[5,3U],
+ * context's GPU.  Supported: rnn = 0 (GRU, reset_after=True) with 1 <= units <= 64, n_classes 2..5 (the classes
+ * dgrp_model_create accepts), with or without attention; LSTM, units > 64 and n_classes > 5 give
+ * DGRP_E_UNSUPPORTED.  Every step is fp32 on CUDA cores and bit-reproducible on one GPU (no float atomics).  Weights and gradients use the Keras layouts of dgrp_model_create: kernel[5,3U],
  * recurrent[U,3U], bias[2,3U], att_scale[U] (NULL without attention), ff_kernel[F,C], ff_bias[C].
  * optimizer: DGRP_OPT_RMSPROP (momentum > 0: TF ApplyRMSProp, ms = rho ms + (1-rho) g^2, mom = momentum mom +
  * lr g / sqrt(ms + eps), w -= mom; momentum = 0: w -= lr g / (sqrt(ms) + eps)) or DGRP_OPT_ADAM (Keras: beta1 0.9,

@@ -22,15 +22,19 @@ TRAIN_PARAMS = ("kernel", "recurrent_kernel", "bias", "att_scale", "ff_kernel", 
 
 
 def train_forward(w: Dict[str, np.ndarray], codes: np.ndarray, ymask: np.ndarray, starts: np.ndarray,
-                  keep: np.ndarray, dropout: float, vecsize: int):
-    """The training forward of a GRU model on the windows [s, s + vecsize) of a record, as torch float64 tensors
+                  keep: np.ndarray, dropout: float, vecsize: int, dtype=None):
+    """The training forward of a GRU model on the windows [s, s + vecsize) of a record, as torch tensors
     that autograd can differentiate: (loss, probs [B,T,C], {name: leaf tensor}).
 
     Input dropout: keep[b][dir][c] (0/1) scaled by 1/(1-dropout) multiplies channel c of the input the GRU sees
     (dir 0: x, dir 1: the reverse complement).  Loss: Keras categorical_crossentropy on probabilities -- p / sum p,
-    clipped to [1e-7, 1-1e-7], -sum_c y_c log p_c -- averaged over every position; y_c = bit c of ymask."""
+    clipped to [1e-7, 1-1e-7], -sum_c y_c log p_c -- averaged over every position; y_c = bit c of ymask.
+
+    ``dtype`` (default torch.float64) is the torch type of every tensor.  With torch.float32 the same math runs in
+    float32 on the CPU: its distance from the float64 result measures the float32 rounding noise of a shape, the
+    yardstick for the tolerance of a comparison with the fp32 GPU kernels."""
     import torch
-    dt = torch.float64
+    dt = torch.float64 if dtype is None else dtype
     prm = {k: torch.tensor(np.asarray(w[k], dtype=np.float64), dtype=dt, requires_grad=True)
            for k in TRAIN_PARAMS if w.get(k) is not None}
     T = int(vecsize)
@@ -38,7 +42,7 @@ def train_forward(w: Dict[str, np.ndarray], codes: np.ndarray, ymask: np.ndarray
     idx = starts[:, None] + np.arange(T)[None, :]
     x = torch.nn.functional.one_hot(torch.from_numpy(np.asarray(codes, np.int64)[idx]), 5).to(dt)
     x_rc = x.flip(1)[:, :, COMPLEMENT]
-    keep = torch.from_numpy(np.asarray(keep, dtype=np.float64)) / (1.0 - dropout)
+    keep = (torch.from_numpy(np.asarray(keep, dtype=np.float64)) / (1.0 - dropout)).to(dt)
     units = prm["recurrent_kernel"].shape[0]
 
     def gru(inp):
@@ -68,7 +72,7 @@ def train_forward(w: Dict[str, np.ndarray], codes: np.ndarray, ymask: np.ndarray
     probs = torch.softmax(feat @ prm["ff_kernel"] + prm["ff_bias"], dim=2)
     n_classes = probs.shape[2]
     ybits = np.asarray(ymask, np.int64)[idx][:, :, None] >> np.arange(n_classes)[None, None, :]
-    y = torch.from_numpy((ybits & 1).astype(np.float64))
+    y = torch.from_numpy((ybits & 1).astype(np.float64)).to(dt)
     p = probs / probs.sum(-1, keepdim=True)
     p = torch.clamp(p, 1e-7, 1 - 1e-7)
     loss = -(y * torch.log(p)).sum(-1).mean()
@@ -76,9 +80,10 @@ def train_forward(w: Dict[str, np.ndarray], codes: np.ndarray, ymask: np.ndarray
 
 
 def train_loss_and_grads(w: Dict[str, np.ndarray], codes: np.ndarray, ymask: np.ndarray, starts: np.ndarray,
-                         keep: np.ndarray, dropout: float, vecsize: int):
-    """(loss, {name: float64 gradient}, probs float64[B,T,C]) of one training batch (see `train_forward`)."""
-    loss, probs, prm = train_forward(w, codes, ymask, starts, keep, dropout, vecsize)
+                         keep: np.ndarray, dropout: float, vecsize: int, dtype=None):
+    """(loss, {name: gradient}, probs [B,T,C]) of one training batch (see `train_forward`), as numpy arrays of
+    ``dtype`` (default float64)."""
+    loss, probs, prm = train_forward(w, codes, ymask, starts, keep, dropout, vecsize, dtype)
     loss.backward()
     return float(loss.item()), {k: v.grad.numpy().copy() for k, v in prm.items()}, probs.detach().numpy()
 

@@ -70,6 +70,32 @@ def test_oracle_gradients_match_finite_differences(attention):
     assert set(grads) == {k for k, v in w.items() if v is not None}
 
 
+@pytest.mark.parametrize("attention", [True, False])
+def test_oracle_float32_is_float64_to_rounding_noise(attention):
+    """The float32 run of the oracle (the GPU tests' measure of a shape's rounding noise) is the same math: it agrees
+    with float64 to float32 noise, and asking for float64 explicitly changes no bit of the default result."""
+    import torch
+    T, U = 12, 6
+    codes, ymask, _ = _record(120, 12)
+    w = _weights(T, U, attention, 13, scale=2.0)
+    starts = np.array([0, 31, 108])
+    keep = (np.random.default_rng(14).random((3, 2, 5)) < 0.75).astype(np.uint8)
+    loss, grads, probs = train_oracle.train_loss_and_grads(w, codes, ymask, starts, keep, 0.25, T)
+    loss64, grads64, probs64 = train_oracle.train_loss_and_grads(w, codes, ymask, starts, keep, 0.25, T,
+                                                                  dtype=torch.float64)
+    assert loss == loss64 and np.array_equal(probs, probs64) and probs.dtype == np.float64
+    assert all(np.array_equal(grads[k], grads64[k]) and grads[k].dtype == np.float64 for k in grads)
+    loss32, grads32, probs32 = train_oracle.train_loss_and_grads(w, codes, ymask, starts, keep, 0.25, T,
+                                                                  dtype=torch.float32)
+    assert probs32.dtype == np.float32 and set(grads32) == set(grads)
+    assert abs(loss32 - loss) <= 1e-6 * loss
+    assert np.abs(probs32 - probs).max() <= 1e-6
+    for k, g in grads.items():
+        assert grads32[k].dtype == np.float32
+        err = np.linalg.norm(grads32[k] - g) / np.linalg.norm(g)
+        assert 0 < err <= 1e-4, (k, err)      # 0 would mean the float32 path did not run in float32
+
+
 def test_optimizer_step_rules():
     w, g = np.array([1.0, -2.0]), np.array([0.5, -0.25])
     new, st = train_oracle.optimizer_step("RMSprop", w, g, {}, 1, 0.1, 0.9, 0.5, 1e-10)
