@@ -164,7 +164,7 @@ class Context:
         check(lib().dgrp_ctx_create(device, ctypes.byref(handle)))
         self.handle = handle
         self.device = device
-        # tuning knobs from the environment: DEEPGRP_KNOBS="forward_sum16=1,mss_chunk=4096"
+        # tuning knobs from the environment: DEEPGRP_KNOBS="forward_tc=0,mss_chunk=4096"
         for item in filter(None, os.environ.get("DEEPGRP_KNOBS", "").split(",")):
             key, _, value = item.partition("=")
             self.set_int(key.strip(), int(value))

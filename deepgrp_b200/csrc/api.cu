@@ -299,14 +299,10 @@ int dgrp_ctx_set_int(dgrp_ctx *c, const char *key, int64_t value) {
   if (!strcmp(key, "mss_chunk")) c->mss_chunk = (int)value;
   else if (!strcmp(key, "mss_max_rounds")) c->mss_max_rounds = (int)value;
   else if (!strcmp(key, "forward_tc")) c->forward_tc = (int)value;
-  else if (!strcmp(key, "forward_sum16")) c->forward_sum16 = (int)value;
-  else if (!strcmp(key, "forward_fp16x2")) c->forward_fp16x2 = (int)value;
   else if (!strcmp(key, "forward_gather")) c->forward_gather = (int)value;
   else if (!strcmp(key, "forward_fuse_score")) c->forward_fuse_score = (int)value;
   else if (!strcmp(key, "forward_smem_vote")) c->forward_smem_vote = (int)value;
   else if (!strcmp(key, "forward_wide")) c->forward_wide = (int)value;
-  else if (!strcmp(key, "forward_overlap")) c->forward_overlap = (int)value;
-  else if (!strcmp(key, "forward_ub")) c->forward_ub = (int)value;
   else if (!strcmp(key, "stream_slot_mb")) c->stream_slot_mb = (int)value;
   else if (!strcmp(key, "stream_early_rows")) c->stream_early_rows = (int)value;
   else if (!strcmp(key, "stream_early_slabs")) c->stream_early_slabs = (int)value;
@@ -323,15 +319,11 @@ int dgrp_ctx_get_int(dgrp_ctx *c, const char *key, int64_t *value) {
   else if (!strcmp(key, "mss_max_rounds")) *value = c->mss_max_rounds;
   else if (!strcmp(key, "mss_rounds")) *value = c->mss_rounds;
   else if (!strcmp(key, "forward_tc")) *value = c->forward_tc;
-  else if (!strcmp(key, "forward_sum16")) *value = c->forward_sum16;
-  else if (!strcmp(key, "forward_fp16x2")) *value = c->forward_fp16x2;
   else if (!strcmp(key, "forward_gather")) *value = c->forward_gather;
   else if (!strcmp(key, "forward_fuse_score")) *value = c->forward_fuse_score;
   else if (!strcmp(key, "forward_smem_vote")) *value = c->forward_smem_vote;
   else if (!strcmp(key, "fused_last")) *value = c->fused_last;
   else if (!strcmp(key, "forward_wide")) *value = c->forward_wide;
-  else if (!strcmp(key, "forward_overlap")) *value = c->forward_overlap;
-  else if (!strcmp(key, "forward_ub")) *value = c->forward_ub;
   else if (!strcmp(key, "stream_slot_mb")) *value = c->stream_slot_mb;
   else if (!strcmp(key, "stream_early_rows")) *value = c->stream_early_rows;
   else if (!strcmp(key, "stream_early_slabs")) *value = c->stream_early_slabs;
@@ -569,26 +561,12 @@ int dgrp_model_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classe
     for (int g = 0; g < G; ++g)
       for (int u = 0; u < U; ++u)
         Rp[((size_t)k * G + g) * UP + u] = recurrent[(size_t)k * G * U + g * U + u];
-  // bf16 hi|mid|lo pieces of recurrent^T in the tcgen05 operand layout (forward_tc.cu)
-  std::vector<uint16_t> Bs, Bh;
-  int b16_shift = 0;
+  // the two-tile tcgen05 kernel's weight operand (forward_tc.cu)
+  std::vector<uint16_t> Bh;
+  int b_shift = 0;
   if (UP <= 64 && rnn == 0) {
-    const int N = 3 * UP + 16, SBO = (UP / 8) * 128;   // 16 extra rows: FF kernel halves (forward_tc.cu)
+    const int N = 3 * UP + 16;   // 16 extra rows: FF kernel halves (forward_tc.cu)
     const bool att = att_scale != nullptr;
-    Bs.assign((size_t)3 * N * UP, 0);
-    auto f2bf = [](float f) -> uint16_t {
-      uint32_t u;
-      memcpy(&u, &f, 4);
-      if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40);
-      const uint32_t r = 0x7fffu + ((u >> 16) & 1u);
-      return (uint16_t)((u + r) >> 16);
-    };
-    auto bf2f = [](uint16_t b) -> float {
-      const uint32_t u = (uint32_t)b << 16;
-      float f;
-      memcpy(&f, &u, 4);
-      return f;
-    };
     // x(n, k): column n of [R | K/2] (pre-scaled gate columns, halved projection columns), row k
     auto entry = [&](int n, int k) -> float {
       if (n < 3 * UP) {
@@ -604,27 +582,12 @@ int dgrp_model_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classe
         return 0.5f * ff_kernel[(size_t)((att ? U : 0) + k) * n_classes + (j - 8)];
       return 0.f;
     };
-    float bmax = 0.f;
-    for (int n = 0; n < N; ++n)
-      for (int k = 0; k < UP; ++k) {
-        const float x = entry(n, k);
-        bmax = std::fmax(bmax, std::fabs(x));
-        const uint16_t hi = f2bf(x);
-        const float r1 = x - bf2f(hi);
-        const uint16_t mid = f2bf(r1);
-        const float r2 = r1 - bf2f(mid);
-        const uint16_t lo = f2bf(r2);
-        const size_t off = ((size_t)(n / 8) * SBO + (size_t)(k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2) / 2;
-        Bs[off] = hi;
-        Bs[(size_t)N * UP + off] = mid;
-        Bs[(size_t)2 * N * UP + off] = lo;
-      }
-    // fp16 hi|lo of the same matrix times 2^shift (largest entry just below 2^14, so that the low
+    // fp16 hi|lo of this matrix times 2^shift (largest entry just below 2^14, so that the low
     // pieces of all but negligible entries are normal half-precision numbers), with 16 more K rows:
     // rows UP + c (c = 0..4) hold the z / r entries of the input table for base c -- the kernel puts
     // one_hot(x_t) * 2^8 into the matching K columns of A, so the MMA adds the input projection of the
     // z and r gates (the h gate's stays outside r * (.), reset_after=True) and the h gate's recurrent bias.
-    const int KP = UP + 16, SBO16 = (KP / 8) * 128;
+    const int KP = UP + 16, SBO = (KP / 8) * 128;
     auto entry16 = [&](int n, int k) -> float {
       if (k < UP) return entry(n, k);
       const int cc = k - UP;
@@ -632,35 +595,35 @@ int dgrp_model_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classe
       if (n >= 2 * UP) return b1[n] * 2.8853900817779268f;   // h gate: its recurrent bias (inside r * (.))
       return (P[(size_t)cc * G * UP + n] + b1[n]) * -1.4426950408889634f;   // n = g * UP + u, g < 2
     };
-    bmax = 0.f;
+    float bmax = 0.f;
     for (int n = 0; n < N; ++n)
       for (int k = 0; k < KP; ++k) bmax = std::fmax(bmax, std::fabs(entry16(n, k)));
     if (bmax > 0.f && std::isfinite(bmax)) {
       int e = 0;
       std::frexp(bmax, &e);             // bmax = f * 2^e, f in [0.5, 1)
-      b16_shift = 14 - e;
-      if (b16_shift > 24) b16_shift = 24;
-      if (b16_shift < -24) b16_shift = -24;
+      b_shift = 14 - e;
+      if (b_shift > 24) b_shift = 24;
+      if (b_shift < -24) b_shift = -24;
     }
     Bh.assign((size_t)2 * N * KP, 0);
     for (int n = 0; n < N; ++n)
       for (int k = 0; k < KP; ++k) {
-        const float x = std::ldexp(entry16(n, k), b16_shift);
+        const float x = std::ldexp(entry16(n, k), b_shift);
         const __half hi = __float2half_rn(x);
         const __half lo = __float2half_rn(x - __half2float(hi));
-        const size_t off = ((size_t)(n / 8) * SBO16 + (size_t)(k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2) / 2;
+        const size_t off = ((size_t)(n / 8) * SBO + (size_t)(k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2) / 2;
         memcpy(&Bh[off], &hi, 2);
         memcpy(&Bh[(size_t)N * KP + off], &lo, 2);
       }
   }
-  std::vector<uint16_t> Bw[2][2];
+  std::vector<uint16_t> Bw[2];
   int bw_shift = 0;
   build_tcw_operands(rnn, U, UP, n_classes, att_scale != nullptr, Rp.data(), P.data(), b1.data(), ff_kernel, Bw,
                      &bw_shift);
   dgrp_model *m = new dgrp_model();
   m->device = c->device; m->rnn = rnn; m->T = vecsize; m->U = U; m->C = n_classes; m->UP = UP;
   m->attention = att_scale != nullptr;
-  m->b16_shift = b16_shift;
+  m->b_shift = b_shift;
   m->bw_shift = bw_shift;
   const int F = m->attention ? 2 * U : U;
   auto up = [&](float **dst, const float *src, size_t count) -> int {
@@ -675,20 +638,15 @@ int dgrp_model_create(dgrp_ctx *c, int rnn, int vecsize, int units, int n_classe
       (rc = up(&m->d_ffk, ff_kernel, (size_t)F * n_classes)) ||
       (rc = up(&m->d_ffb, ff_bias, (size_t)n_classes)) ||
       (m->attention && (rc = up(&m->d_scale, att_scale, (size_t)U))) ||
-      (!Bs.empty() && (rc = up(reinterpret_cast<float **>(&m->d_Bsplit),
-                               reinterpret_cast<const float *>(Bs.data()), Bs.size() / 2))) ||
-      (!Bh.empty() && (rc = up(reinterpret_cast<float **>(&m->d_Bsplit16),
-                               reinterpret_cast<const float *>(Bh.data()), Bh.size() / 2))) ||
-      (!Bh.empty() && false)) {
+      (!Bh.empty() && (rc = up(reinterpret_cast<float **>(&m->d_Bsplit),
+                               reinterpret_cast<const float *>(Bh.data()), Bh.size() / 2)))) {
     cudaStreamSynchronize(c->stream);
     dgrp_model_destroy(m);
     return rc;
   }
   for (int a = 0; a < 2 && rc == DGRP_OK; ++a)
-    for (int b = 0; b < 2 && rc == DGRP_OK; ++b)
-      if (!Bw[a][b].empty())
-        rc = up(reinterpret_cast<float **>(&m->d_Bw[a][b]), reinterpret_cast<const float *>(Bw[a][b].data()),
-                Bw[a][b].size() / 2);
+    if (!Bw[a].empty())
+      rc = up(reinterpret_cast<float **>(&m->d_Bw[a]), reinterpret_cast<const float *>(Bw[a].data()), Bw[a].size() / 2);
   if (rc != DGRP_OK) {
     cudaStreamSynchronize(c->stream);
     dgrp_model_destroy(m);
@@ -707,10 +665,8 @@ int dgrp_model_destroy(dgrp_model *m) {
   for (float *p : ptrs)
     if (p) cudaFree(p);
   if (m->d_Bsplit) cudaFree(m->d_Bsplit);
-  if (m->d_Bsplit16) cudaFree(m->d_Bsplit16);
-  for (auto &a : m->d_Bw)
-    for (uint16_t *q : a)
-      if (q) cudaFree(q);
+  for (uint16_t *q : m->d_Bw)
+    if (q) cudaFree(q);
   delete m;
   return DGRP_OK;
 }

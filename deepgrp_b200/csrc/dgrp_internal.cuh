@@ -79,12 +79,13 @@ struct dgrp_model {
   float *d_b0 = nullptr;         // [3, UP]     bias[0, g*U+u], zero padded
   float *d_Rp = nullptr;         // [UP, 3, UP] recurrent[k, g*U+u], zero padded
   float *d_b1 = nullptr;         // [3, UP]     bias[1, g*U+u], zero padded
-  uint16_t *d_Bsplit = nullptr;  // [3][3UP x UP] bf16 hi|mid|lo of recurrent^T, UMMA K-major core matrices
-  uint16_t *d_Bsplit16 = nullptr;  // [2][..] fp16 hi|lo of (recurrent^T * 2^b16_shift), same layout
-  int b16_shift = 0;
+  // two-tile tcgen05 form (forward_tc.cu): [2][(3UP + 16) x (UP + 16)] fp16 hi|lo of ([R | K/2]^T * 2^b_shift)
+  // (+ 16 one-hot K rows), UMMA K-major core matrices; null where the shape has no such form
+  uint16_t *d_Bsplit = nullptr;
+  int b_shift = 0;
   // wide tcgen05 form (forward_tcw.cu): fp16 hi|lo pieces of the blocked [R | K/2]^T (+ 16 one-hot K rows), for one
   // CTA per tile and for a CTA pair ([rank][piece][rows of the rank]); null where the shape has no such form
-  uint16_t *d_Bw[2][2] = {};   // [0 one CTA | 1 CTA pair][0 default column blocks | 1 the GRU's 32-unit blocks]
+  uint16_t *d_Bw[2] = {};   // [0 one CTA | 1 CTA pair]
   int bw_shift = 0;
   float *d_scale = nullptr;      // [U] or null
   float *d_ffk = nullptr;        // [F, C]
@@ -107,8 +108,6 @@ struct dgrp_ctx {
   int mss_max_rounds = 0;  // Jacobi rounds before the sequential completion (0 = default)
   int mss_rounds = 0;      // rounds used by the last MSS call (negative: completed sequentially)
   int forward_tc = 1;      // 1: tcgen05 recurrence where available, 0: fp32 FFMA kernel
-  int forward_sum16 = 1;   // tcgen05 forward: keep h_fwd + h_rc (attention scores only) in half precision
-  int forward_fp16x2 = 1;  // tcgen05 forward: operands as 2 fp16 pieces / 3 products instead of 3 bf16 pieces / 6 products
   int forward_gather = 1;  // tcgen05 forward: write window probabilities and max-merge them in a gather pass
                            // (1) instead of 5 atomicMax per window-step (0); falls back to 0 above 40 GB
   int forward_wide = 0;    // 0: the wide tcgen05 kernel (forward_tcw.cu) only where the two-tile kernel has no form
@@ -121,8 +120,6 @@ struct dgrp_ctx {
   int stream_early_unit = 0;   // windows per unit of a slab (0 = one wave of the forward kernel: 128 x SM count)
   int stream_early_ratio = 0;  // size of a slab relative to the one before it, per cent (0 = default: 80)
   int stream_early_parts = 0;  // diagnostic: parts of the last record's text that left before its last slab
-  int forward_ub = 0;      // wide kernel, GRU: units per column block (64 or 32; 0 = default: 64)
-  int forward_overlap = 1; // wide kernel with two column blocks: issue the MMAs block by block so that they overlap the gates
   int64_t forward_slab_bytes = (int64_t)8 << 30;   // bound of the window-probability buffer: the windows of a
                            // record run in slabs of at most this many bytes of [windows][T][C] probabilities
   int forward_smem_vote = 1;    // tcgen05 forward: max-merge a tile's windows in shared memory (no window probabilities in HBM)
@@ -235,7 +232,7 @@ int run_forward_dense(dgrp_ctx *c, dgrp_model *m, const float *d_batch, int64_t 
                       float *d_probs);
 // forward_tcw.cu: host-side packing of the wide tcgen05 kernel's weight operand (empty where the shape has no form)
 void build_tcw_operands(int rnn, int U, int UP, int C, bool att, const float *Rp, const float *P, const float *b1,
-                        const float *ffk, std::vector<uint16_t> (&out)[2][2], int *shift);
+                        const float *ffk, std::vector<uint16_t> (&out)[2], int *shift);
 // mss.cu
 // L0: the running sum the scan starts from (0 at the start of a record).  resume != nullptr: the scores are a
 // PREFIX of a record ("open end"): only the segments that are final whatever follows are returned -- those the

@@ -19,10 +19,10 @@ struct FwdParams {
   int T, U, C, step, attention;
   int64_t full_windows, tail_base;
   const float *P, *Wk, *b0, *Rp, *b1, *scale, *ffk, *ffb;
-  const uint16_t *Bsplit; // tcgen05 form: operand pieces of [R | K/2]^T, UMMA layout (bf16 x3 or fp16 x2)
+  const uint16_t *Bsplit; // tcgen05 form: fp16 hi|lo pieces of [R | K/2]^T, UMMA layout
   int code_span;          // tcgen05 form: bytes per tile of the staged base codes (multiple of 16)
   int wpp;                // tcgen05 form: windows per pass of the second phase (8..64)
-  float b_unscale;        // fp16 x2 form: 1 / (state scale * weight scale), applied to the accumulator
+  float b_unscale;        // tcgen05 form: 1 / (state scale * weight scale), applied to the accumulator
   float *scratch, *ff2, *qbuf;
   float *pred;
   int64_t pred_row0, pred_rows;

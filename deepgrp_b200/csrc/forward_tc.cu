@@ -5,14 +5,12 @@
 // Precision.  The parity bar (>= 99.99 % identical labels against a float32 CPU run, on random-init
 // weights whose class margins are ~1e-4) needs fp32-faithful pre-activations through a 150..512 step
 // recurrence (SURVEY.md section 7 H1); plain bf16 misses it by orders of magnitude.  Both operands are
-// therefore split into pieces and the product is formed from the piece products that matter, each a
-// kind::f16 tcgen05.mma accumulating in fp32 into the same TMEM tile, smallest terms first:
-//   NP = 2 (default)  two fp16 pieces of the scaled value (state x 2^8, weights x 2^shift so that the
-//                     low pieces stay normal): hi.hi + hi.lo + lo.hi, relative error ~2^-21 per product;
-//   NP = 3            three bf16 pieces (8+8+8 bits = the fp32 significand), the six products of weight
-//                     >= 2^-16: hi.hi + hi.mid + mid.hi + mid.mid + hi.lo + lo.hi.
-// Both measure the same distance from the float64 oracle as the fp32 kernel (tools/accuracy_study.py).
-// The gates, sigmoid/tanh and the state update stay in fp32 registers.
+// therefore split into two fp16 pieces of the scaled value (state x 2^8, weights x 2^shift so that the
+// low pieces stay normal) and the product is formed from three piece products, each a kind::f16
+// tcgen05.mma accumulating in fp32 into the same TMEM tile, smallest terms first: lo.hi + hi.lo + hi.hi,
+// relative error ~2^-21 per product.  This measures the same distance from the float64 oracle as the fp32
+// kernel (tools/accuracy_study.py); three bf16 pieces (six products) measured no closer at twice the
+// tensor work.  The gates, sigmoid/tanh and the state update stay in fp32 registers.
 //
 // One CTA = 20 warps, persistent, one per SM; a unit of work = two tiles of 64 windows x 2 directions
 // (M = 128 rows; row r = window r/2, direction r%2) in flight:
@@ -21,7 +19,7 @@
 //                (tcgen05.ld), add the input projection (a table row: x_t is one-hot), apply the gates,
 //                write the new state as operand pieces into A (shared memory), fence, arrive on the
 //                tile's "ready" mbarrier, and only then store the step's scratch;
-//   warp 16      MMA issuer: waits for "ready" (with back-off), issues the step's NP(NP+1)/2 x UP/16
+//   warp 16      MMA issuer: waits for "ready" (with back-off), issues the step's 3 x UP/16 + 2
 //                tcgen05.mma (M128, N = 3*UP + 16, K16) and commits them to "done".
 //                (Letting the last-arriving gate warp issue instead was measured 14 % slower.)
 //   warps 17..19 exit after setmaxnreg: the CTA launches with 96 registers per thread, the issuer's
@@ -34,8 +32,8 @@
 //   TMEM   2 x [128 lanes x (3*UP + 16) columns] fp32 accumulators: z | r | h gate blocks, then 16
 //          projection columns h.(K/2) (the FF layer's two halves): avg[t].K = h_fwd[t].K/2 + h_rc[t].K/2
 //          comes out of the same MMA and the second phase needs no FFMA over the units
-//   smem   B = [R | K/2]^T pieces, [NP][(3*UP+16) x UP], K-major core matrices, resident
-//          A = state pieces, [2 tiles][NP][128 x UP], rewritten every step by the gate warps
+//   smem   B = [R | K/2]^T pieces, [2][(3*UP+16) x (UP+16)], K-major core matrices, resident
+//          A = state pieces, [2 tiles][2][128 x (UP+16)], rewritten every step by the gate warps
 //          input table [10 rows][3*UP + 4] (A,C,G,T of either direction 4 banks apart, then 'N')
 //          staged bases of the unit's tiles as table rows, [2 tiles][forward | reversed+complemented]
 //          scores of one pass of the second phase, [wpp windows][T]
@@ -45,10 +43,10 @@
 //
 // Scratch in HBM (per CTA, rewritten by every unit; the attention query avg[T-1] is only known after
 // the last step, so the scores need a second pass over all avg[t]):
-//   sum    ST[2][64/wpp][T][UP/8][wpp][8]  h_fwd[t] + h_rc[t] (= 2 avg[t], one lane shuffle) -- feeds ONLY the
-//                                 additive-attention scores; ST = half by default (|sum| < 2; a
+//   sum    f16[2][64/wpp][T][UP/8][wpp][8]  h_fwd[t] + h_rc[t] (= 2 avg[t], one lane shuffle) -- feeds ONLY the
+//                                 additive-attention scores, so half precision suffices (|sum| < 2; a
 //                                 probability moves by ~1e-7 on random-init weights, <= 3e-5 on sharp
-//                                 ones), float with forward_sum16 = 0
+//                                 ones); float32 measured 8 % slower
 //   q      f32[2][64][UP]         avg[T-1] in full precision (the query)
 //   proj   f32[2][64][T][16]      avg[t].K, both FF halves (the logits come from these, full precision)
 // = 192 B per (window, t), written once and read once.  All CTAs run the same amount of work, so without
@@ -61,17 +59,16 @@
 
 namespace dgrp {
 
-template <int UP, int NP>
+template <int UP>
 struct TCfg {
   static constexpr int NG = 3 * UP;            // gate columns (z | r | h)
   static constexpr int N = 3 * UP + 16;        // + 16 projection columns: h.[FF ctx half(5) pad(3) | FF avg half(5) pad(3)]
   static constexpr int ROWS = 128, WT = 64;
   static constexpr int UPT = UP / 4;           // units per gate thread
-  // NP = 2 folds the z / r input projection into the MMA: 16 more K columns hold one_hot(x_t) * 2^8 in A
+  // The z / r input projection is folded into the MMA: 16 more K columns hold one_hot(x_t) * 2^8 in A
   // (5 used) and, in B, the z / r rows of the input table plus the h gate's recurrent bias, so the gate
   // warps read only the h-gate row of the table (a quarter of their former shared-memory loads).
-  static constexpr bool FOLD = NP == 2;
-  static constexpr int KP = UP + (FOLD ? 16 : 0);   // K of the operands
+  static constexpr int KP = UP + 16;           // K of the operands
   static constexpr int KC = KP / 8;            // core matrices along K
   static constexpr int SBO = KC * 128;         // bytes between 8-row groups
   static constexpr int A_BYTES = ROWS * KP * 2;  // one piece of one tile
@@ -81,20 +78,19 @@ struct TCfg {
 };
 
 
-// NP = 3: bf16 hi|mid|lo pieces, 6 products (fp32-faithful).  NP = 2: fp16 hi|lo pieces of the scaled
-// operands, 3 products (hi.hi + hi.lo + lo.hi, relative error ~2^-21 per product): half the tensor
-// work, half the operand traffic out of shared memory.
-template <int UP, typename ST, int NP>
+template <int UP>
 __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(const FwdParams p) {
-  using K = TCfg<UP, NP>;
+  using K = TCfg<UP>;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  unsigned char *s_B = smem_raw;                               // [3][B_BYTES]
-  unsigned char *s_A = s_B + NP * K::B_BYTES;                  // [2][NP][A_BYTES]
-  float *s_P = reinterpret_cast<float *>(s_A + 2 * NP * K::A_BYTES);  // [10][PSTRIDE]: rows 0..3 A,C,G,T of the forward
+  unsigned char *s_B = smem_raw;                               // [2][B_BYTES]
+  unsigned char *s_A = s_B + 2 * K::B_BYTES;                   // [2][2][A_BYTES]
+  float *s_P = reinterpret_cast<float *>(s_A + 2 * 2 * K::A_BYTES);  // [10][PSTRIDE]: rows 0..3 A,C,G,T of the forward
                                                                // pass, 4..7 of the rc pass (complemented), 8, 9
                                                                // 'N' of either: the eight common rows start 4
                                                                // banks apart, so a warp's mixed reads do not conflict
-  float *s_bh = s_P + 10 * K::PSTRIDE;                         // [UP] recurrent bias of the h gate
+                                                               // (only the h-gate columns are read)
+  float *s_bh = s_P + 10 * K::PSTRIDE;                         // [UP] recurrent bias of the h gate (unread: B's
+                                                               // one-hot K rows carry it)
   float *s_scale = s_bh + UP;                                  // [UP] attention scale
   float *s_score = s_scale + UP;                               // [wpp][T]
   uint8_t *s_codes = reinterpret_cast<uint8_t *>(s_score + (size_t)p.wpp * p.T);   // [2 tiles][fwd | rc][code_span] staged bases
@@ -108,7 +104,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
   {
     const uint4 *src = reinterpret_cast<const uint4 *>(p.Bsplit);
     uint4 *dst = reinterpret_cast<uint4 *>(s_B);
-    for (int i = tid; i < NP * K::B_BYTES / 16; i += TC_THREADS) dst[i] = src[i];
+    for (int i = tid; i < 2 * K::B_BYTES / 16; i += TC_THREADS) dst[i] = src[i];
     for (int i = tid; i < 10 * K::PSTRIDE; i += TC_THREADS) {
       const int row = i / K::PSTRIDE, j = i % K::PSTRIDE;
       // reverse complement: [3,2,1,0,4] (model.py:277)
@@ -162,10 +158,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
   const int64_t tile_lo = n_tiles * blockIdx.x / gridDim.x, tile_hi = n_tiles * (blockIdx.x + 1) / gridDim.x;
   const int64_t my_tiles = tile_hi - tile_lo;   // a single-tile unit costs ~3/4 of a period for half the work
   const int lead = my_tiles >= 32 ? (int)(blockIdx.x & 3) : (my_tiles >= 16 ? (int)(blockIdx.x & 1) : 0);
-  // instruction descriptor: D fp32, A/B bf16, both K-major, N = 3*UP + 16, M = 128
-  const uint32_t ab_fmt = NP == 3 ? 1u : 0u;   // operand format: 1 = bf16, 0 = fp16
-  const uint32_t idesc = (1u << 4) | (ab_fmt << 7) | (ab_fmt << 10) | ((uint32_t)(K::N >> 3) << 17) |
-                         ((uint32_t)(128 >> 4) << 24);
+  // instruction descriptor: D fp32, A/B fp16, both K-major, N = 3*UP + 16, M = 128
+  const uint32_t idesc = (1u << 4) | ((uint32_t)(K::N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
 
   if (!is_gate) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(TC_AUX_REGS));
@@ -185,23 +179,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
           tc_fence_after();
           TC_TRACE(5);
           if (lane == 0) {
-            const uint32_t a0 = smem_u32(s_A + (size_t)s * NP * K::A_BYTES), b0 = smem_u32(s_B);
+            const uint32_t a0 = smem_u32(s_A + (size_t)s * 2 * K::A_BYTES), b0 = smem_u32(s_B);
             const uint32_t d = tmem_base + (uint32_t)(s * K::TCOLS);
-            // (A piece, B piece), smallest products first: lo.hi, hi.lo, mid.mid, mid.hi, hi.mid, hi.hi
-            // (fp16 x2: lo.hi, hi.lo, hi.hi)
-            const int pa[6] = {NP == 3 ? 2 : 1, 0, NP == 3 ? 1 : 0, 1, 0, 0};
-            const int pb[6] = {0, NP == 3 ? 2 : 1, NP == 3 ? 1 : 0, 0, 1, 0};
+            // (A piece, B piece), smallest products first: lo.hi, hi.lo, hi.hi
+            const int pa[3] = {1, 0, 0};
+            const int pb[3] = {0, 1, 0};
             uint32_t acc = 0;
 #pragma unroll
-            for (int q = 0; q < (NP == 3 ? 6 : 3); ++q) {
+            for (int q = 0; q < 3; ++q) {
               // the one-hot K chunk only exists in the hi piece of A (its lo piece is zero)
-              const int nkc = UP / 16 + ((K::FOLD && pa[q] == 0) ? 1 : 0);
+              const int nkc = UP / 16 + (pa[q] == 0 ? 1 : 0);
 #pragma unroll
               for (int kc = 0; kc < UP / 16 + 1; ++kc) {
                 if (kc >= nkc) break;
                 const uint64_t ad = umma_desc(a0 + pa[q] * K::A_BYTES + kc * 256, 128, K::SBO);
                 const uint64_t bd = umma_desc(b0 + pb[q] * K::B_BYTES + kc * 256, 128, K::SBO);
-                umma_bf16(d, ad, bd, idesc, acc);
+                umma_f16(d, ad, bd, idesc, acc);
                 acc = 1;
               }
             }
@@ -220,7 +213,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
   }
 
   asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(TC_GATE_REGS));
-  ST *sum0 = reinterpret_cast<ST *>(p.scratch) + (size_t)blockIdx.x * 2 * K::WT * T * UP;         // [2][WT][T][UP]
+  __half *sum0 = reinterpret_cast<__half *>(p.scratch) + (size_t)blockIdx.x * 2 * K::WT * T * UP; // [2][WT][T][UP]
   float *proj0 = p.ff2 + (size_t)blockIdx.x * 2 * K::WT * T * 16;                                 // [2][WT][T][16]
   float *q0 = p.qbuf + (size_t)blockIdx.x * 2 * K::WT * UP;                                       // [2][WT][UP]
   const float2 us = make_float2(p.b_unscale, p.b_unscale);
@@ -234,11 +227,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
     const int row = quad * 32 + lane;        // row of the tile = TMEM lane
     const int wl = row >> 1, dir = row & 1;  // window in tile, direction
     const float *tblp = s_P + uq * K::UPT;
-    const float *bhp = s_bh + uq * K::UPT;
     const uint32_t a_off = (uint32_t)((row >> 3) * K::SBO + (row & 7) * 16 + ((uq * K::UPT) >> 3) * 128);
     // this thread's constant part of the `sum` index: pass of its window, window within the pass, half
     const size_t sum_thr = ((size_t)(wl / p.wpp) * T * (UP / 8) * p.wpp + (size_t)(wl % p.wpp)) * 8 + (dir ? 4 : 0);
-    const uint32_t oh_off = (uint32_t)((row >> 3) * K::SBO + (row & 7) * 16 + (UP / 8) * 128);   // FOLD: one-hot K chunk
+    const uint32_t oh_off = (uint32_t)((row >> 3) * K::SBO + (row & 7) * 16 + (UP / 8) * 128);   // the one-hot K chunk
     const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16);
     // The bases of a tile are one contiguous span of 63 * step + T codes: staged in shared memory once
     // per unit, so that the step loop has no global load (an L2 miss there stalls the whole tile).  Two
@@ -275,14 +267,14 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
       for (int j = 0; j < K::UPT; ++j) hprev[s][j] = 0.f;
       if (s == 1 && !live1) continue;
       // h[-1] = 0: zero this thread's slots of the A operand and let the issuer prime the accumulator
-      unsigned char *a_tile = s_A + (size_t)s * NP * K::A_BYTES + a_off;
+      unsigned char *a_tile = s_A + (size_t)s * 2 * K::A_BYTES + a_off;
 #pragma unroll
       for (int c8 = 0; c8 < K::UPT / 8; ++c8)
 #pragma unroll
-        for (int pc = 0; pc < NP; ++pc)
+        for (int pc = 0; pc < 2; ++pc)
           *reinterpret_cast<uint4 *>(a_tile + pc * K::A_BYTES + c8 * 128) = make_uint4(0u, 0u, 0u, 0u);
-      if (K::FOLD && uq == 0) {   // one_hot(x_0) in the hi piece's extra K chunk (its second half stays zero)
-        unsigned char *oh = s_A + (size_t)s * NP * K::A_BYTES + oh_off;
+      if (uq == 0) {   // one_hot(x_0) in the hi piece's extra K chunk (its second half stays zero)
+        unsigned char *oh = s_A + (size_t)s * 2 * K::A_BYTES + oh_off;
         *reinterpret_cast<uint4 *>(oh) = onehot_row(s_codes[cbase + s * 2 * p.code_span]);
         *reinterpret_cast<uint4 *>(oh + 128) = make_uint4(0u, 0u, 0u, 0u);
       }
@@ -307,7 +299,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
         TC_TRACE(0);
         const float *prow = tblp + trow * K::PSTRIDE;
         const uint32_t t_tile = t_lane + (uint32_t)(s * K::TCOLS);
-        unsigned char *a_tile = s_A + (size_t)s * NP * K::A_BYTES + a_off;
+        unsigned char *a_tile = s_A + (size_t)s * 2 * K::A_BYTES + a_off;
         const size_t rt = (size_t)(s * K::WT + wl) * T + t;   // (window, t) row of the scratch arrays
         float pj[4];   // projection of h[t-1] (4 of the 16 extra columns per unit quarter)
         tmem_ld4(t_tile + (uint32_t)(K::NG + 4 * uq), pj);
@@ -325,31 +317,19 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
           }
 #pragma unroll
           for (int j4 = 0; j4 < 2; ++j4) {
-            const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
-            const float4 xz = K::FOLD ? zero4 : *reinterpret_cast<const float4 *>(prow + c8 * 8 + 4 * j4);
-            const float4 xr = K::FOLD ? zero4 : *reinterpret_cast<const float4 *>(prow + UP + c8 * 8 + 4 * j4);
             const float4 xh = *reinterpret_cast<const float4 *>(prow + 2 * UP + c8 * 8 + 4 * j4);
-            const float4 bh = K::FOLD ? zero4 : *reinterpret_cast<const float4 *>(bhp + c8 * 8 + 4 * j4);
-            gru_cell4<NP == 2, K::FOLD>(xz, xr, xh, bh, az + 4 * j4, ar + 4 * j4, ah + 4 * j4,
-                               &hprev[s][c8 * 8 + 4 * j4], us, hn2[c8][2 * j4], hn2[c8][2 * j4 + 1]);
+            gru_cell4(xh, az + 4 * j4, ar + 4 * j4, ah + 4 * j4, &hprev[s][c8 * 8 + 4 * j4], us, hn2[c8][2 * j4],
+                      hn2[c8][2 * j4 + 1]);
           }
           // new state -> operand pieces in A (one 16-byte core-matrix row per piece)
-          uint32_t hi[4], mid[4], lo[4];
-          if (NP == 3) {
+          uint32_t hi[4], lo[4];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) split3(hn2[c8][j], hi[j], mid[j], lo[j]);
-            *reinterpret_cast<uint4 *>(a_tile + c8 * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-            *reinterpret_cast<uint4 *>(a_tile + K::A_BYTES + c8 * 128) = make_uint4(mid[0], mid[1], mid[2], mid[3]);
-            *reinterpret_cast<uint4 *>(a_tile + 2 * K::A_BYTES + c8 * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-          } else {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) split2h(hn2[c8][j], hi[j], lo[j]);
-            *reinterpret_cast<uint4 *>(a_tile + c8 * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-            *reinterpret_cast<uint4 *>(a_tile + K::A_BYTES + c8 * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-          }
+          for (int j = 0; j < 4; ++j) split2h(hn2[c8][j], hi[j], lo[j]);
+          *reinterpret_cast<uint4 *>(a_tile + c8 * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+          *reinterpret_cast<uint4 *>(a_tile + K::A_BYTES + c8 * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
         }
-        if (K::FOLD && uq == 0 && t + 1 < T)   // the next step's base for the MMA's one-hot K columns
-          *reinterpret_cast<uint4 *>(s_A + (size_t)s * NP * K::A_BYTES + oh_off) =
+        if (uq == 0 && t + 1 < T)   // the next step's base for the MMA's one-hot K columns
+          *reinterpret_cast<uint4 *>(s_A + (size_t)s * 2 * K::A_BYTES + oh_off) =
               onehot_row(s_codes[cbase + s * 2 * p.code_span + t + 1]);
         TC_TRACE(2);
         // Hand the new A operand to the tensor core (the last step's MMA only feeds the projection).
@@ -366,7 +346,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
           o.y = pj[1] + __shfl_xor_sync(0xffffffffu, pj[1], 1);
           o.z = pj[2] + __shfl_xor_sync(0xffffffffu, pj[2], 1);
           o.w = pj[3] + __shfl_xor_sync(0xffffffffu, pj[3], 1);
-          if (NP == 2) { o.x *= us.x; o.y *= us.x; o.z *= us.x; o.w *= us.x; }
+          o.x *= us.x; o.y *= us.x; o.z *= us.x; o.w *= us.x;
           if (dir == 0 && t > 0) *reinterpret_cast<float4 *>(proj0 + (rt - 1) * 16 + 4 * uq) = o;
         }
         TC_TRACE(5);
@@ -386,14 +366,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
             }
             const int u = uq * K::UPT + c8 * 8 + (dir ? 4 : 0);
             // [slot][pass][t][chunk][wpp windows][8 units]: the warp's 32 rows write 32 consecutive 4-unit groups
-            ST *dst = sum0 + (size_t)s * K::WT * T * UP + sum_thr + ((size_t)t * (UP / 8) + (uq * (K::UPT / 8) + c8)) * p.wpp * 8;
-            if (sizeof(ST) == 2) {
-              const __half2 h0 = __floats2half2_rn(sm2[0].x, sm2[0].y), h1 = __floats2half2_rn(sm2[1].x, sm2[1].y);
-              *reinterpret_cast<uint2 *>(dst) =
-                  make_uint2(*reinterpret_cast<const uint32_t *>(&h0), *reinterpret_cast<const uint32_t *>(&h1));
-            } else {
-              *reinterpret_cast<float4 *>(dst) = make_float4(sm2[0].x, sm2[0].y, sm2[1].x, sm2[1].y);
-            }
+            __half *dst = sum0 + (size_t)s * K::WT * T * UP + sum_thr + ((size_t)t * (UP / 8) + (uq * (K::UPT / 8) + c8)) * p.wpp * 8;
+            const __half2 h0 = __floats2half2_rn(sm2[0].x, sm2[0].y), h1 = __floats2half2_rn(sm2[1].x, sm2[1].y);
+            *reinterpret_cast<uint2 *>(dst) =
+                make_uint2(*reinterpret_cast<const uint32_t *>(&h0), *reinterpret_cast<const uint32_t *>(&h1));
             if (t == T - 1)   // the query avg[T-1] in full precision
               *reinterpret_cast<float4 *>(q0 + (size_t)(s * K::WT + wl) * UP + u) =
                   make_float4(0.5f * sm2[0].x, 0.5f * sm2[0].y, 0.5f * sm2[1].x, 0.5f * sm2[1].y);
@@ -416,7 +392,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
       o.y = pj[1] + __shfl_xor_sync(0xffffffffu, pj[1], 1);
       o.z = pj[2] + __shfl_xor_sync(0xffffffffu, pj[2], 1);
       o.w = pj[3] + __shfl_xor_sync(0xffffffffu, pj[3], 1);
-      if (NP == 2) { o.x *= us.x; o.y *= us.x; o.z *= us.x; o.w *= us.x; }
+      o.x *= us.x; o.y *= us.x; o.z *= us.x; o.w *= us.x;
       if (dir == 0)
         *reinterpret_cast<float4 *>(proj0 + ((size_t)(s * K::WT + wl) * T + (T - 1)) * 16 + 4 * uq) = o;
     }
@@ -427,7 +403,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
     gate_bar_sync();
 #pragma unroll 1
     for (int s = 0; s < nt; ++s)
-      attention_vote_sum_tile<UP, K::WT, TC_GATE_WARPS, ST>(
+      attention_vote_sum_tile<UP, K::WT, TC_GATE_WARPS>(
           p, sum0 + (size_t)s * K::WT * T * UP, q0 + (size_t)s * K::WT * UP,
           proj0 + (size_t)s * K::WT * T * 16, tile_range(p, tile + s, K::WT), p.wpp, s_scale, s_score,
           p.smem_vote == 1 ? reinterpret_cast<float *>(s_A)            // A is idle: every MMA of the unit has completed
@@ -449,16 +425,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1) gru_tc_attention_vote_kernel(co
   }
 }
 
-template <int UP, int NP>
+template <int UP>
 static size_t tc_smem_bytes(int T, int wpp, int code_span) {
-  using K = TCfg<UP, NP>;
-  return (size_t)NP * K::B_BYTES + 2 * NP * K::A_BYTES +
+  using K = TCfg<UP>;
+  return (size_t)2 * K::B_BYTES + 2 * 2 * K::A_BYTES +
          sizeof(float) * ((size_t)10 * K::PSTRIDE + 2 * UP + (size_t)wpp * T) + 4 * (size_t)code_span + 128;
 }
 
-template <int UP, typename ST, int NP>
+template <int UP>
 static int launch_tc_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
-  using K = TCfg<UP, NP>;
+  using K = TCfg<UP>;
   const int64_t n_windows = p.w_end - p.w_begin;
   if (n_windows <= 0 && p.w2_end <= p.w2_begin) return DGRP_OK;
   // windows per pass of the second phase: as many score rows as shared memory holds
@@ -467,8 +443,8 @@ static int launch_tc_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
   if (span > 16384) return DGRP_E_UNSUPPORTED;
   p.code_span = (int)((span + 15) & ~(int64_t)15);
   int wpp = K::WT;
-  while (wpp > 8 && tc_smem_bytes<UP, NP>(p.T, wpp, p.code_span) > 227 * 1024) wpp >>= 1;
-  const size_t smem = tc_smem_bytes<UP, NP>(p.T, wpp, p.code_span);
+  while (wpp > 8 && tc_smem_bytes<UP>(p.T, wpp, p.code_span) > 227 * 1024) wpp >>= 1;
+  const size_t smem = tc_smem_bytes<UP>(p.T, wpp, p.code_span);
   if (smem > 227 * 1024) return DGRP_E_UNSUPPORTED;   // caller falls back to the fp32 kernel
   p.wpp = wpp;
   // the tile's span of rows, max-merged in the A operand's shared memory during the second phase
@@ -478,22 +454,22 @@ static int launch_tc_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
   size_t smem_total = smem;
   p.smem_vote = 0;
   if (c->forward_smem_vote) {
-    if (vote_bytes <= (size_t)2 * NP * K::A_BYTES) p.smem_vote = 1;
+    if (vote_bytes <= (size_t)2 * 2 * K::A_BYTES) p.smem_vote = 1;
     else if (smem + vote_bytes <= 227 * 1024) { p.smem_vote = 2; smem_total = smem + vote_bytes; }
   }
   if (p.query) return DGRP_OK;
   if (p.smem_vote) p.win_probs = nullptr;
-  auto kern = gru_tc_attention_vote_kernel<UP, ST, NP>;
+  auto kern = gru_tc_attention_vote_kernel<UP>;
   DGRP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_total));
   const int64_t n_tiles = (n_windows > 0 ? (n_windows + K::WT - 1) / K::WT : 0) +
                           (p.w2_end > p.w2_begin ? (p.w2_end - p.w2_begin + K::WT - 1) / K::WT : 0);
   const int64_t n_pairs = (n_tiles + 1) / 2;
   const int grid = (int)(n_pairs < c->sm_count ? n_pairs : c->sm_count);
   const size_t rows = (size_t)grid * 2 * K::WT;   // window slots in flight
-  DGRP_CHECK(c->avg.reserve(rows * p.T * UP * sizeof(ST) + rows * UP * sizeof(float)));
+  DGRP_CHECK(c->avg.reserve(rows * p.T * UP * sizeof(__half) + rows * UP * sizeof(float)));
   DGRP_CHECK(c->io_c.reserve(rows * p.T * 16 * sizeof(float)));
   p.scratch = c->avg.as<float>();
-  p.qbuf = reinterpret_cast<float *>(c->avg.as<unsigned char>() + rows * p.T * UP * sizeof(ST));
+  p.qbuf = reinterpret_cast<float *>(c->avg.as<unsigned char>() + rows * p.T * UP * sizeof(__half));
   p.ff2 = c->io_c.as<float>();
   // p.win_probs (window probabilities, max-merged by the caller's gather pass) or the atomic vote: forward.cu
   kern<<<grid, TC_THREADS, smem_total, c->stream>>>(p);
@@ -502,8 +478,6 @@ static int launch_tc_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
   return DGRP_OK;
 }
 
-// Returns DGRP_E_UNSUPPORTED when this model/shape has no tcgen05 form (the caller then uses the
-// fp32 kernel): units > 64, or a window too long for the score buffer in shared memory.
 #ifdef DGRP_TC_TRACE
 extern "C" int dgrp_debug_tc_trace(unsigned long long *out, int reset) {
   if (reset) {
@@ -521,20 +495,15 @@ extern "C" int dgrp_debug_tc_trace2(unsigned long long *out, int reset) {
 }
 #endif
 
-template <int UP>
-static int launch_tc_up(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
-  if (c->forward_fp16x2)
-    return c->forward_sum16 ? launch_tc_t<UP, __half, 2>(c, m, p) : launch_tc_t<UP, float, 2>(c, m, p);
-  return c->forward_sum16 ? launch_tc_t<UP, __half, 3>(c, m, p) : launch_tc_t<UP, float, 3>(c, m, p);
-}
-
+// Returns DGRP_E_UNSUPPORTED when this model/shape has no tcgen05 form (the caller then uses the
+// fp32 kernel): units > 64, or a window too long for the score buffer in shared memory.
 int launch_forward_tc(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
-  if (!m->d_Bsplit || !m->d_Bsplit16) return DGRP_E_UNSUPPORTED;
-  p.Bsplit = c->forward_fp16x2 ? m->d_Bsplit16 : m->d_Bsplit;
-  p.b_unscale = c->forward_fp16x2 ? ldexpf(1.0f, -(8 + m->b16_shift)) : 1.0f;
+  if (!m->d_Bsplit) return DGRP_E_UNSUPPORTED;
+  p.Bsplit = m->d_Bsplit;
+  p.b_unscale = ldexpf(1.0f, -(8 + m->b_shift));
   switch (m->UP) {
-    case 32: return launch_tc_up<32>(c, m, p);
-    case 64: return launch_tc_up<64>(c, m, p);
+    case 32: return launch_tc_t<32>(c, m, p);
+    case 64: return launch_tc_t<64>(c, m, p);
     default: return DGRP_E_UNSUPPORTED;
   }
 }

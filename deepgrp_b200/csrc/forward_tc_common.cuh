@@ -3,7 +3,6 @@
 // descriptor and TMEM wrappers, the operand split, the packed gate arithmetic and the second phase
 // (attention scores, softmax over t, FF logits, class softmax, vote).
 #pragma once
-#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include "forward_common.cuh"
@@ -83,8 +82,8 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint
   d |= 1ull << 46;  // descriptor version (sm_100)
   return d;         // layout_type = 0: no swizzle
 }
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t idesc,
-                                          uint32_t accumulate) {
+__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a, uint64_t b, uint32_t idesc,
+                                         uint32_t accumulate) {
   asm volatile(
       "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n"
       " tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}"
@@ -134,22 +133,10 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 
-// (a, b) = hi + mid + lo in bf16 pieces; each output word packs a's piece (low half) and b's (high half).
-// The residuals are formed with one packed FFMA2 (x - hi exactly, as the scalar subtraction would).
-__device__ __forceinline__ void split3(float2 ab, uint32_t &hi, uint32_t &mid, uint32_t &lo) {
-  const float2 neg1 = make_float2(-1.0f, -1.0f);
-  __nv_bfloat162 h2 = __floats2bfloat162_rn(ab.x, ab.y);
-  hi = *reinterpret_cast<uint32_t *>(&h2);
-  const float2 r = __ffma2_rn(make_float2(__uint_as_float(hi << 16), __uint_as_float(hi & 0xffff0000u)), neg1, ab);
-  __nv_bfloat162 m2 = __floats2bfloat162_rn(r.x, r.y);
-  mid = *reinterpret_cast<uint32_t *>(&m2);
-  const float2 q = __ffma2_rn(make_float2(__uint_as_float(mid << 16), __uint_as_float(mid & 0xffff0000u)), neg1, r);
-  __nv_bfloat162 l2 = __floats2bfloat162_rn(q.x, q.y);
-  lo = *reinterpret_cast<uint32_t *>(&l2);
-}
-
-// fp16 x2 form: (a, b) * 2^8 = hi + lo in half-precision pieces (11 + 11 significant bits; the scale keeps
-// the low piece a normal number for every |h| > 5e-4 and exact-to-2^-33 below)
+// (a, b) * 2^8 = hi + lo in half-precision pieces (11 + 11 significant bits; the scale keeps the low piece a
+// normal number for every |h| > 5e-4 and exact-to-2^-33 below); each output word packs a's piece (low half)
+// and b's (high half).  The residual is formed with one packed FFMA2 (x - hi exactly, as the scalar
+// subtraction would).
 constexpr float kStateScale = 256.0f;
 __device__ __forceinline__ void split2h(float2 ab, uint32_t &hi, uint32_t &lo) {
   const float2 x = __fmul2_rn(ab, make_float2(kStateScale, kStateScale));
@@ -161,7 +148,7 @@ __device__ __forceinline__ void split2h(float2 ab, uint32_t &hi, uint32_t &lo) {
   lo = *reinterpret_cast<const uint32_t *>(&l2);
 }
 
-// FOLD: the 16-byte core-matrix row that holds one_hot(x) * 2^8 (half precision, 0x5C00 = 256) for the
+// The 16-byte core-matrix row that holds one_hot(x) * 2^8 (half precision, 0x5C00 = 256) for the
 // input-table row `trow` (0..3 forward A,C,G,T; 4..7 the rc pass, already complemented; 8, 9 'N'):
 // K position p = the base the table row stands for.
 __device__ __forceinline__ uint4 onehot_row(int trow) {
@@ -191,33 +178,17 @@ __device__ __forceinline__ void sigmoid_pair(float2 sz, float2 sr, float2 &z, fl
   z = __fmul2_rn(iab, b);
   r = __fmul2_rn(iab, a);
 }
-// SCALED: the accumulator holds (state scale * weight scale) h.R and is multiplied by `us` on the way in
-// (an FFMA2 in place of the FADD2, so the scaling is free).
-template <bool SCALED>
-__device__ __forceinline__ float2 acc_add(float2 acc, float2 x, float2 us) {
-  return SCALED ? __ffma2_rn(acc, us, x) : __fadd2_rn(x, acc);
-}
-// FOLD: the z / r pre-activations already contain the input projection (one-hot K columns of the MMA).
-template <bool SCALED, bool FOLD>
-__device__ __forceinline__ void gru_cell4(const float4 xz, const float4 xr, const float4 xh, const float4 bh,
-                                          const float *az, const float *ar, const float *ah, float *hp,
+// The accumulators hold (state scale * weight scale) times the pre-activation and are multiplied by `us` on the
+// way in.  The one-hot K columns of the MMA have already added the z / r input projection and the h gate's
+// recurrent bias; only the h gate's input row `xh` stays outside r * (.) (reset_after=True).
+__device__ __forceinline__ void gru_cell4(const float4 xh, const float *az, const float *ar, const float *ah, float *hp,
                                           float2 us, float2 &h01, float2 &h23) {
   const float2 one = make_float2(1.0f, 1.0f);
   float2 z0, r0, z1, r1;
-  if (FOLD) {
-    sigmoid_pair(__fmul2_rn(make_float2(az[0], az[1]), us), __fmul2_rn(make_float2(ar[0], ar[1]), us), z0, r0);
-    sigmoid_pair(__fmul2_rn(make_float2(az[2], az[3]), us), __fmul2_rn(make_float2(ar[2], ar[3]), us), z1, r1);
-  } else {
-    sigmoid_pair(acc_add<SCALED>(make_float2(az[0], az[1]), make_float2(xz.x, xz.y), us),
-                 acc_add<SCALED>(make_float2(ar[0], ar[1]), make_float2(xr.x, xr.y), us), z0, r0);
-    sigmoid_pair(acc_add<SCALED>(make_float2(az[2], az[3]), make_float2(xz.z, xz.w), us),
-                 acc_add<SCALED>(make_float2(ar[2], ar[3]), make_float2(xr.z, xr.w), us), z1, r1);
-  }
-  // FOLD: the h-gate accumulator already contains its recurrent bias (the one-hot K rows of B)
-  const float2 g0 = FOLD ? __fmul2_rn(make_float2(ah[0], ah[1]), us)
-                         : acc_add<SCALED>(make_float2(ah[0], ah[1]), make_float2(bh.x, bh.y), us);
-  const float2 g1 = FOLD ? __fmul2_rn(make_float2(ah[2], ah[3]), us)
-                         : acc_add<SCALED>(make_float2(ah[2], ah[3]), make_float2(bh.z, bh.w), us);
+  sigmoid_pair(__fmul2_rn(make_float2(az[0], az[1]), us), __fmul2_rn(make_float2(ar[0], ar[1]), us), z0, r0);
+  sigmoid_pair(__fmul2_rn(make_float2(az[2], az[3]), us), __fmul2_rn(make_float2(ar[2], ar[3]), us), z1, r1);
+  const float2 g0 = __fmul2_rn(make_float2(ah[0], ah[1]), us);
+  const float2 g1 = __fmul2_rn(make_float2(ah[2], ah[3]), us);
   const float2 t0 = __ffma2_rn(r0, g0, make_float2(xh.x, xh.y));
   const float2 t1 = __ffma2_rn(r1, g1, make_float2(xh.z, xh.w));
   const float2 d0 = __fadd2_rn(make_float2(ex2_approx(fminf(t0.x, 30.0f)), ex2_approx(fminf(t0.y, 30.0f))), one);
@@ -282,18 +253,8 @@ __device__ __forceinline__ float tanh_mufu(float x) {   // MUFU.TANH: relative e
 __device__ __forceinline__ float exp_fast(float x) {   // e^x through ex2.approx (2 ulp), e^{-inf} = 0
   return ex2_approx(x * 1.4426950408889634f);
 }
-__device__ __forceinline__ float inv4_dot(const float *d, const float *sc) {
-  // sum_k sc[k] / d[k], k < 4, with one reciprocal (d[k] <= 2^30 + 1, so the product is finite)
-  const float2 d01 = make_float2(d[0], d[1]), d23 = make_float2(d[2], d[3]);
-  const float2 m = __fmul2_rn(d01, d23);
-  const float inv = rcp_approx(m.x * m.y);
-  const float2 j = make_float2(inv * m.y, inv * m.x);
-  const float2 i01 = __fmul2_rn(j, d23), i23 = __fmul2_rn(j, d01);
-  return fmaf(sc[0], i01.x, fmaf(sc[1], i01.y, fmaf(sc[2], i23.x, sc[3] * i23.y)));
-}
-
-template <int UP, int WT, int NWARPS, typename ST>
-__device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, const ST *sum, const float *qbuf,
+template <int UP, int WT, int NWARPS>
+__device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, const __half *sum, const float *qbuf,
                                                         const float *proj, const TileRange tr, int wpp,
                                                         const float *s_scale, float *s_score, float *s_vote = nullptr) {
   const int64_t w_tile0 = tr.w0;
@@ -312,9 +273,7 @@ __device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, cons
   constexpr int NCH = UP / 8;          // 8-unit chunks per avg row
   constexpr int CPL = NCH / 4;         // chunks per lane: cj, cj + 4, ...
   constexpr int CH = CPL > 2 ? 2 : CPL;   // chunks per lane and sweep
-  constexpr bool H16 = sizeof(ST) == 2;
-  constexpr int NV = H16 ? 1 : 2;      // 16-byte loads per chunk
-  constexpr int UNR = H16 ? 4 : 2;     // t's in flight per lane (scores)
+  constexpr int UNR = 4;               // t's in flight per lane (scores)
   constexpr int PU = 11;               // rows in flight per lane (softmax / vote passes): all of T <= 352 at once
   TC_TRACE_DECL;
   for (int w0 = 0; w0 < WT; w0 += wpp) {
@@ -328,24 +287,23 @@ __device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, cons
       // four chunks would not fit the register budget); the second sweep adds to the first one's scores
 #pragma unroll 1
       for (int i0 = 0; i0 < CPL; i0 += CH) {
-      float q2[CH][8], sc2[CH][8];   // 2 log2(e) q[u], -2 scale[u]
+      float q2[CH][8], sc2[CH][8];   // q[u], scale[u]: score = sum_u scale[u] tanh.approx(q[u] + sum/2)
 #pragma unroll
       for (int i = 0; i < CH; ++i) {
         const int u0 = (cj + 4 * (i0 + i)) * 8;
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-          // H16 (the default, "forward_sum16"): score = sum_u scale[u] tanh.approx(q[u] + sum/2); else the exact form
-          q2[i][j] = H16 ? qbuf[(size_t)wl * UP + u0 + j] : qbuf[(size_t)wl * UP + u0 + j] * kTwoLog2e;
-          sc2[i][j] = H16 ? s_scale[u0 + j] : -2.0f * s_scale[u0 + j];
+          q2[i][j] = qbuf[(size_t)wl * UP + u0 + j];
+          sc2[i][j] = s_scale[u0 + j];
         }
       }
       // the pass's windows are contiguous per (t, chunk): [pass][t][chunk][wpp windows][8 units]
-      const ST *sum_pass = sum + (size_t)(w0 / wpp) * T * NCH * wpp * 8;
-      const ST *base = sum_pass + ((size_t)(cj + 4 * i0) * wpp + (grp * 8 + wi)) * 8;
+      const __half *sum_pass = sum + (size_t)(w0 / wpp) * T * NCH * wpp * 8;
+      const __half *base = sum_pass + ((size_t)(cj + 4 * i0) * wpp + (grp * 8 + wi)) * 8;
       // one warp per t-slice keeps the L2 PF_AHEAD rows ahead of the demand loads, PF_BLOCK rows at a time
       // (a t-row of the tile is NCH * WT * 8 contiguous elements)
       constexpr int PF_BLOCK = 4, PF_AHEAD = 12;
-      const uint32_t ROW_BYTES = (uint32_t)(NCH * wpp * 8 * sizeof(ST));
+      const uint32_t ROW_BYTES = (uint32_t)(NCH * wpp * 8 * sizeof(__half));
       if (grp == 0 && lane == 0 && i0 == 0) {
         const int n0 = min(PF_AHEAD, t_end - t_begin);
         l2_prefetch(sum_pass + (size_t)t_begin * NCH * wpp * 8, (uint32_t)n0 * ROW_BYTES);
@@ -355,15 +313,13 @@ __device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, cons
           const int ta = t0 + PF_AHEAD;
           if (ta < t_end) l2_prefetch(sum_pass + (size_t)ta * NCH * wpp * 8, (uint32_t)min(PF_BLOCK, t_end - ta) * ROW_BYTES);
         }
-        uint4 v[UNR][CH][NV];
+        uint4 v[UNR][CH];
 #pragma unroll
         for (int k = 0; k < UNR; ++k) {
           const int t = min(t0 + k, t_end - 1);
 #pragma unroll
           for (int i = 0; i < CH; ++i)
-#pragma unroll
-            for (int n = 0; n < NV; ++n)
-              v[k][i][n] = __ldcs(reinterpret_cast<const uint4 *>(base + ((size_t)t * NCH + 4 * i) * wpp * 8) + n);
+            v[k][i] = __ldcs(reinterpret_cast<const uint4 *>(base + ((size_t)t * NCH + 4 * i) * wpp * 8));
         }
 #pragma unroll
         for (int k = 0; k < UNR; ++k) {
@@ -371,33 +327,19 @@ __device__ __forceinline__ void attention_vote_sum_tile(const FwdParams &p, cons
 #pragma unroll
           for (int i = 0; i < CH; ++i) {
             float x[8];   // h_fwd[t] + h_rc[t] of 8 units
-            if (H16) {
-              const uint32_t wv[4] = {v[k][i][0].x, v[k][i][0].y, v[k][i][0].z, v[k][i][0].w};
+            const uint32_t wv[4] = {v[k][i].x, v[k][i].y, v[k][i].z, v[k][i].w};
 #pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&wv[j]));
-                x[2 * j] = f.x; x[2 * j + 1] = f.y;
-              }
-            } else {
-              const uint32_t wv[8] = {v[k][i][0].x, v[k][i][0].y, v[k][i][0].z, v[k][i][0].w,
-                                      v[k][i][NV - 1].x, v[k][i][NV - 1].y, v[k][i][NV - 1].z, v[k][i][NV - 1].w};
-#pragma unroll
-              for (int j = 0; j < 8; ++j) x[j] = __uint_as_float(wv[j]);
+            for (int j = 0; j < 4; ++j) {
+              const float2 f = __half22float2(*reinterpret_cast<const __half2 *>(&wv[j]));
+              x[2 * j] = f.x; x[2 * j + 1] = f.y;
             }
-            if (H16) {
-              // The half-precision `sum` already limits a score to ~2^-11 per term; MUFU.TANH (tanh.approx.f32, relative
-              // error 2^-11) is the matching arithmetic: 3.5 instead of ~8.5 instructions and 1 instead of 1.25 MUFU
-              // operations per (t, unit).  Measured against the exact form: max |dp| 3.5e-8 on random-init weights,
-              // 3.5e-5 on the x4 set (1.4e-5 from the half-precision sum alone); forward_sum16 = 0 is the exact path.
+            // The half-precision `sum` already limits a score to ~2^-11 per term; MUFU.TANH (tanh.approx.f32, relative
+            // error 2^-11) is the matching arithmetic: 3.5 instead of ~8.5 instructions and 1 instead of 1.25 MUFU
+            // operations per (t, unit) of the exact form -2 sum_u scale[u] / (e^{2(q + sum/2)} + 1).  Measured against
+            // the exact form: max |dp| 3.5e-8 on random-init weights, 3.5e-5 on the x4 set (1.4e-5 from the
+            // half-precision sum alone).
 #pragma unroll
-              for (int j = 0; j < 8; ++j) sacc = fmaf(sc2[i][j], tanh_mufu(fmaf(x[j], 0.5f, q2[i][j])), sacc);
-            } else {
-              float d[8];
-#pragma unroll
-              for (int j = 0; j < 8; ++j)   // e^{2 (q + sum/2)} + 1 = 2^{2 log2e q + log2e sum} + 1
-                d[j] = ex2_approx(fminf(fmaf(x[j], 1.4426950408889634f, q2[i][j]), 30.0f)) + 1.0f;
-              sacc += inv4_dot(d, sc2[i]) + inv4_dot(d + 4, sc2[i] + 4);
-            }
+            for (int j = 0; j < 8; ++j) sacc = fmaf(sc2[i][j], tanh_mufu(fmaf(x[j], 0.5f, q2[i][j])), sacc);
           }
           sacc += __shfl_xor_sync(0xffffffffu, sacc, 8);
           sacc += __shfl_xor_sync(0xffffffffu, sacc, 16);

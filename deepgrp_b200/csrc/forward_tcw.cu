@@ -26,14 +26,18 @@
 
 namespace dgrp {
 
-// UB_ = units per column block: G * UB + 16 <= 256 (GRU: 64 or 32, LSTM: 32)
-template <int UP_, int RNN_, bool PAIR_, int UB_ = (RNN_ ? 32 : 64)>
+template <int UP_, int RNN_, bool PAIR_>
 struct WCfg {
   static constexpr int UP = UP_, RNN = RNN_;
   static constexpr bool PAIR = PAIR_;
   static constexpr int G = RNN ? 4 : 3;             // gates: GRU z, r, h; LSTM i, f, c, o
-  static constexpr int UB = UP < UB_ ? UP : UB_;
+  // units per column block, G * UB + 16 <= 256: GRU 64, LSTM 32.  (32-unit GRU blocks measured the same: 144 against
+  // 147 Mbp/s at 128 units.)
+  static constexpr int UB = UP < (RNN ? 32 : 64) ? UP : (RNN ? 32 : 64);
   static constexpr int NBLK = UP / UB;
+  // several column blocks: the MMAs of one block overlap the gate work on another (see rnn_tcw_kernel; one round of
+  // MMAs between two steps measured 117-125 against 134 Mbp/s at 128 units, 356 against 428 Mbp/s for LSTM, 60 units)
+  static constexpr bool OVL = NBLK >= 2;
   static_assert(G * UB + 16 <= 256, "a column block is one MMA: at most 256 columns");
   static constexpr int NW0 = G * UB + 16, NW = G * UB;   // columns of block 0 (with the projection) / of the others
   static constexpr int N = G * UP + 16;
@@ -131,7 +135,7 @@ __device__ __forceinline__ void lstm_cell4(const float *ai, const float *af, con
   h23 = make_float2(h[2], h[3]);
 }
 
-// OVL (two or four column blocks): the MMAs of a round are issued block by block, as soon as the state columns they
+// OVL (several column blocks): the MMAs of a round are issued block by block, as soon as the state columns they
 // read have been written, so that the tensor core works while the gate warps do.  With blocks 0..n-1 (the gate warps
 // go through them in this order, all 16 warps on one block at a time) and P(i, j) = "columns of block i from the
 // state units of block j":
@@ -142,13 +146,13 @@ __device__ __forceinline__ void lstm_cell4(const float *ai, const float *af, con
 //                       MMAs that read block j's old columns of A are done) -> write them, arrive ready[j]
 // Only P(0, n-1) -- 1/n^2 of the products -- is exposed between two steps; a D block is overwritten (first product,
 // no accumulate) only after the gate warps have read it (ready[j] is arrived on after the TMEM loads of block j).
-template <int UP, int RNN, bool PAIR, int UB, bool OVL>
+template <int UP, int RNN, bool PAIR>
 __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams p) {
-  using K = WCfg<UP, RNN, PAIR, UB>;
-  using ST = __half;
+  using K = WCfg<UP, RNN, PAIR>;
   constexpr int G = K::G;
   constexpr int NB = K::NBLK;
-  static_assert(!OVL || (NB >= 2 && NB <= 4), "the overlapped protocol needs 2..4 column blocks");
+  constexpr bool OVL = K::OVL;
+  static_assert(NB <= 4, "one ready / done / free barrier per column block: at most 4");
   constexpr int NBAR = OVL ? NB : 1;     // ready / done barriers: one per column block when overlapped
   extern __shared__ __align__(128) unsigned char smem_raw[];
   unsigned char *s_B = smem_raw;                                        // [2 pieces][B_BYTES]  this CTA's weight rows
@@ -242,7 +246,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
             const uint64_t ad = umma_desc(a0 + pa[q] * K::A_BYTES + kc * 256, 128, K::SBO);
             const uint64_t bd = umma_desc(brow + pb[q] * K::B_BYTES + kc * 256, 128, K::SBO);
             if (PAIR) umma_f16_pair(d, ad, bd, idesc, acc);
-            else umma_bf16(d, ad, bd, idesc, acc);
+            else umma_f16(d, ad, bd, idesc, acc);
             acc = 1;
           }
         }
@@ -299,7 +303,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
   }
 
   asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(TC_GATE_REGS));
-  ST *sum0 = reinterpret_cast<ST *>(p.scratch) + (size_t)blockIdx.x * K::WT * T * UP;   // [passes][T][UP/8][wpp][8]
+  __half *sum0 = reinterpret_cast<__half *>(p.scratch) + (size_t)blockIdx.x * K::WT * T * UP;   // [passes][T][UP/8][wpp][8]
   float *proj0 = p.ff2 + (size_t)blockIdx.x * K::WT * T * 16;                           // [WT][T][16]
   float *q0 = p.qbuf + (size_t)blockIdx.x * K::WT * UP;                                 // [WT][UP]
   const float2 us = make_float2(p.b_unscale, p.b_unscale);
@@ -395,10 +399,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
               lstm_cell4(a0 + 4 * j4, a1 + 4 * j4, a2 + 4 * j4, a3 + 4 * j4, &st[ci * 8 + 4 * j4], us.x,
                          hn2[2 * j4], hn2[2 * j4 + 1]);
             } else {
-              const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
               const float4 xh = *reinterpret_cast<const float4 *>(s_P + trow * K::PSTRIDE + b * K::UB + ub + 4 * j4);
-              gru_cell4<true, true>(zero4, zero4, xh, zero4, a0 + 4 * j4, a1 + 4 * j4, a2 + 4 * j4,
-                                    &st[ci * 8 + 4 * j4], us, hn2[2 * j4], hn2[2 * j4 + 1]);
+              gru_cell4(xh, a0 + 4 * j4, a1 + 4 * j4, a2 + 4 * j4, &st[ci * 8 + 4 * j4], us, hn2[2 * j4],
+                        hn2[2 * j4 + 1]);
             }
           }
 #pragma unroll
@@ -446,7 +449,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
             sm2[j] = __fadd2_rn(mine, recv);
           }
           const int u0 = (ci / K::CB) * K::UB + uq * K::UBT + (ci % K::CB) * 8;   // first unit of the chunk
-          ST *dst = sum0 + sum_thr + ((size_t)t * (UP / 8) + (u0 >> 3)) * p.wpp * 8;
+          __half *dst = sum0 + sum_thr + ((size_t)t * (UP / 8) + (u0 >> 3)) * p.wpp * 8;
           const __half2 h0 = __floats2half2_rn(sm2[0].x, sm2[0].y), h1 = __floats2half2_rn(sm2[1].x, sm2[1].y);
           *reinterpret_cast<uint2 *>(dst) =
               make_uint2(*reinterpret_cast<const uint32_t *>(&h0), *reinterpret_cast<const uint32_t *>(&h1));
@@ -483,10 +486,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
     __threadfence_block();
     gate_bar_sync();
     if (live)
-      attention_vote_sum_tile<UP, K::WT, TC_GATE_WARPS, ST>(p, sum0, q0, proj0, tile_range(p, tile, K::WT), p.wpp,
-                                                            s_scale, s_score,
-                                                            p.smem_vote == 1 ? reinterpret_cast<float *>(s_A)
-                                                            : (p.smem_vote == 2 ? reinterpret_cast<float *>(s_codes + 2 * (size_t)p.code_span) : nullptr));
+      attention_vote_sum_tile<UP, K::WT, TC_GATE_WARPS>(p, sum0, q0, proj0, tile_range(p, tile, K::WT), p.wpp,
+                                                        s_scale, s_score,
+                                                        p.smem_vote == 1 ? reinterpret_cast<float *>(s_A)
+                                                        : (p.smem_vote == 2 ? reinterpret_cast<float *>(s_codes + 2 * (size_t)p.code_span) : nullptr));
   }
 
   // ---- teardown: every MMA of the pair has completed (each CTA saw its last "done"); the pair's CTAs
@@ -501,24 +504,24 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rnn_tcw_kernel(const FwdParams 
   }
 }
 
-template <int UP, int RNN, bool PAIR, int UB>
+template <int UP, int RNN, bool PAIR>
 static size_t tcw_smem_bytes(int T, int wpp, int code_span) {
-  using K = WCfg<UP, RNN, PAIR, UB>;
+  using K = WCfg<UP, RNN, PAIR>;
   return (size_t)2 * K::B_BYTES + 2 * K::A_BYTES +
          sizeof(float) * ((size_t)(RNN ? 0 : 10 * K::PSTRIDE) + UP + (size_t)wpp * T) + 2 * (size_t)code_span + 128;
 }
 
-template <int UP, int RNN, bool PAIR, int UB, bool OVL>
-static int launch_tcw_o(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
-  using K = WCfg<UP, RNN, PAIR, UB>;
+template <int UP, int RNN, bool PAIR>
+static int launch_tcw_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
+  using K = WCfg<UP, RNN, PAIR>;
   const int64_t n_windows = p.w_end - p.w_begin;
   if (n_windows <= 0 && p.w2_end <= p.w2_begin) return DGRP_OK;
   const int64_t span = (int64_t)(K::WT - 1) * p.step + p.T;
   if (span > 16384) return DGRP_E_UNSUPPORTED;
   p.code_span = (int)((span + 15) & ~(int64_t)15);
   int wpp = K::WT;
-  while (wpp > 8 && tcw_smem_bytes<UP, RNN, PAIR, UB>(p.T, wpp, p.code_span) > 227 * 1024) wpp >>= 1;
-  const size_t smem = tcw_smem_bytes<UP, RNN, PAIR, UB>(p.T, wpp, p.code_span);
+  while (wpp > 8 && tcw_smem_bytes<UP, RNN, PAIR>(p.T, wpp, p.code_span) > 227 * 1024) wpp >>= 1;
+  const size_t smem = tcw_smem_bytes<UP, RNN, PAIR>(p.T, wpp, p.code_span);
   if (smem > 227 * 1024) return DGRP_E_UNSUPPORTED;   // caller falls back to the fp32 kernel
   p.wpp = wpp;
   const size_t vote_bytes = (size_t)span * p.C * sizeof(float);
@@ -530,7 +533,7 @@ static int launch_tcw_o(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
   }
   if (p.query) return DGRP_OK;
   if (p.smem_vote) p.win_probs = nullptr;
-  auto kern = rnn_tcw_kernel<UP, RNN, PAIR, UB, OVL>;
+  auto kern = rnn_tcw_kernel<UP, RNN, PAIR>;
   DGRP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_total));
   const int64_t n_tiles = (n_windows > 0 ? (n_windows + K::WT - 1) / K::WT : 0) +
                           (p.w2_end > p.w2_begin ? (p.w2_end - p.w2_begin + K::WT - 1) / K::WT : 0);
@@ -560,32 +563,19 @@ static int launch_tcw_o(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
   return DGRP_OK;
 }
 
-template <int UP, int RNN, bool PAIR, int UB>
-static int launch_tcw_t(dgrp_ctx *c, dgrp_model *m, FwdParams &p) {
-  // several column blocks: the MMAs of one block overlap the gate work on another ("forward_overlap", default on)
-  constexpr bool CAN = WCfg<UP, RNN, PAIR, UB>::NBLK >= 2;
-  if (CAN && c->forward_overlap) return launch_tcw_o<UP, RNN, PAIR, UB, CAN>(c, m, p);
-  return launch_tcw_o<UP, RNN, PAIR, UB, false>(c, m, p);
-}
-
 // which = 1: single CTA, 2: CTA pair.  Returns DGRP_E_UNSUPPORTED when the shape has no wide form.
-// "forward_ub" (GRU): units per column block, 64 (two blocks at 128 units; the default) or 32 (four blocks).
 int launch_forward_tcw(dgrp_ctx *c, dgrp_model *m, FwdParams &p, int which) {
   const bool pair = which == 2;
-  const bool fine = m->rnn == 0 && c->forward_ub == 32;   // measured at 128 units: 64-unit blocks 147 Mbp/s, 32-unit 144
-  p.Bsplit = m->d_Bw[pair ? 1 : 0][fine ? 1 : 0];
+  p.Bsplit = m->d_Bw[pair ? 1 : 0];
   if (!p.Bsplit) return DGRP_E_UNSUPPORTED;
   p.b_unscale = ldexpf(1.0f, -(8 + m->bw_shift));
   if (m->rnn == 0) {
-    if (m->UP == 32) return pair ? DGRP_E_UNSUPPORTED : launch_tcw_t<32, 0, false, 32>(c, m, p);
-    if (m->UP == 64) {
-      if (fine) return pair ? launch_tcw_t<64, 0, true, 32>(c, m, p) : launch_tcw_t<64, 0, false, 32>(c, m, p);
-      return pair ? launch_tcw_t<64, 0, true, 64>(c, m, p) : launch_tcw_t<64, 0, false, 64>(c, m, p);
-    }
-    if (m->UP == 128 && pair) return fine ? launch_tcw_t<128, 0, true, 32>(c, m, p) : launch_tcw_t<128, 0, true, 64>(c, m, p);
+    if (m->UP == 32) return pair ? DGRP_E_UNSUPPORTED : launch_tcw_t<32, 0, false>(c, m, p);
+    if (m->UP == 64) return pair ? launch_tcw_t<64, 0, true>(c, m, p) : launch_tcw_t<64, 0, false>(c, m, p);
+    if (m->UP == 128 && pair) return launch_tcw_t<128, 0, true>(c, m, p);
   } else {
-    if (m->UP == 32) return pair ? DGRP_E_UNSUPPORTED : launch_tcw_t<32, 1, false, 32>(c, m, p);
-    if (m->UP == 64) return pair ? launch_tcw_t<64, 1, true, 32>(c, m, p) : launch_tcw_t<64, 1, false, 32>(c, m, p);
+    if (m->UP == 32) return pair ? DGRP_E_UNSUPPORTED : launch_tcw_t<32, 1, false>(c, m, p);
+    if (m->UP == 64) return pair ? launch_tcw_t<64, 1, true>(c, m, p) : launch_tcw_t<64, 1, false>(c, m, p);
   }
   return DGRP_E_UNSUPPORTED;
 }
@@ -595,10 +585,10 @@ int launch_forward_tcw(dgrp_ctx *c, dgrp_model *m, FwdParams &p, int which) {
 // end of block 0) against K row k (units, then 16 rows for the one-hot input columns).  Gate columns are
 // pre-scaled (sigmoid gates by -log2 e, tanh gates by 2 log2 e), projection columns are the halved FF kernel.
 // Rp [UP][G][UP], P [5][G][UP] (kernel + input bias), b1 [G][UP] (GRU recurrent bias; zero for LSTM).
-template <int UP, int RNN, int UB>
+template <int UP, int RNN>
 static void tcw_fill(int U, int C, bool att, const float *Rp, const float *P, const float *b1, const float *ffk,
                      std::vector<float> &dense) {
-  using K = WCfg<UP, RNN, false, UB>;
+  using K = WCfg<UP, RNN, false>;
   constexpr int G = K::G;
   dense.assign((size_t)K::N * K::KP, 0.f);
   for (int b = 0; b < K::NBLK; ++b)
@@ -627,9 +617,9 @@ static void tcw_fill(int U, int C, bool att, const float *Rp, const float *P, co
     }
 }
 
-template <int UP, int RNN, bool PAIR, int UB>
+template <int UP, int RNN, bool PAIR>
 static void tcw_pack(const std::vector<float> &dense, int shift, std::vector<uint16_t> &out) {
-  using K = WCfg<UP, RNN, PAIR, UB>;
+  using K = WCfg<UP, RNN, PAIR>;
   // [rank][piece][B_ROWS x KP] in the UMMA K-major core-matrix layout; CTA `rank` holds, for every column
   // block, rows [rank * cw/NCTA, (rank + 1) * cw/NCTA) of the block at local rows coff/NCTA ...
   out.assign((size_t)K::NCTA * 2 * K::B_ROWS * K::KP, 0);
@@ -651,12 +641,12 @@ static void tcw_pack(const std::vector<float> &dense, int shift, std::vector<uin
     }
 }
 
-template <int UP, int RNN, int UB>
+template <int UP, int RNN>
 static void tcw_build_t(int U, int C, bool att, const float *Rp, const float *P, const float *b1, const float *ffk,
                         bool want_single, bool want_pair, std::vector<uint16_t> &single, std::vector<uint16_t> &pair,
                         int *shift) {
   std::vector<float> dense;
-  tcw_fill<UP, RNN, UB>(U, C, att, Rp, P, b1, ffk, dense);
+  tcw_fill<UP, RNN>(U, C, att, Rp, P, b1, ffk, dense);
   float bmax = 0.f;
   for (float v : dense) bmax = std::fmax(bmax, std::fabs(v));
   int s = 0;
@@ -665,30 +655,24 @@ static void tcw_build_t(int U, int C, bool att, const float *Rp, const float *P,
     std::frexp(bmax, &e);   // the largest entry lands just below 2^14: the low pieces stay normal numbers
     s = std::min(24, std::max(-24, 14 - e));
   }
-  *shift = s;   // the same for every block layout of a model (the entries are the same numbers)
-  if (want_single) tcw_pack<UP, RNN, false, UB>(dense, s, single);
-  if (want_pair) tcw_pack<UP, RNN, true, UB>(dense, s, pair);
+  *shift = s;
+  if (want_single) tcw_pack<UP, RNN, false>(dense, s, single);
+  if (want_pair) tcw_pack<UP, RNN, true>(dense, s, pair);
 }
 
-// Builds the operands for the shapes launch_forward_tcw serves (empty vectors otherwise): out[pair][fine], fine =
-// the GRU's 32-unit column blocks.
+// Builds the operands for the shapes launch_forward_tcw serves (empty vectors otherwise): out[0] single CTA,
+// out[1] CTA pair.
 void build_tcw_operands(int rnn, int U, int UP, int C, bool att, const float *Rp, const float *P, const float *b1,
-                        const float *ffk, std::vector<uint16_t> (&out)[2][2], int *shift) {
-  for (auto &a : out)
-    for (auto &v : a) v.clear();
+                        const float *ffk, std::vector<uint16_t> (&out)[2], int *shift) {
+  for (auto &v : out) v.clear();
   *shift = 0;
   if (rnn == 0) {
-    if (UP == 32) tcw_build_t<32, 0, 32>(U, C, att, Rp, P, b1, ffk, true, false, out[0][0], out[1][0], shift);
-    else if (UP == 64) {
-      tcw_build_t<64, 0, 64>(U, C, att, Rp, P, b1, ffk, true, true, out[0][0], out[1][0], shift);
-      tcw_build_t<64, 0, 32>(U, C, att, Rp, P, b1, ffk, true, true, out[0][1], out[1][1], shift);
-    } else if (UP == 128) {
-      tcw_build_t<128, 0, 64>(U, C, att, Rp, P, b1, ffk, false, true, out[0][0], out[1][0], shift);
-      tcw_build_t<128, 0, 32>(U, C, att, Rp, P, b1, ffk, false, true, out[0][1], out[1][1], shift);
-    }
+    if (UP == 32) tcw_build_t<32, 0>(U, C, att, Rp, P, b1, ffk, true, false, out[0], out[1], shift);
+    else if (UP == 64) tcw_build_t<64, 0>(U, C, att, Rp, P, b1, ffk, true, true, out[0], out[1], shift);
+    else if (UP == 128) tcw_build_t<128, 0>(U, C, att, Rp, P, b1, ffk, false, true, out[0], out[1], shift);
   } else {
-    if (UP == 32) tcw_build_t<32, 1, 32>(U, C, att, Rp, P, b1, ffk, true, false, out[0][0], out[1][0], shift);
-    else if (UP == 64) tcw_build_t<64, 1, 32>(U, C, att, Rp, P, b1, ffk, true, true, out[0][0], out[1][0], shift);
+    if (UP == 32) tcw_build_t<32, 1>(U, C, att, Rp, P, b1, ffk, true, false, out[0], out[1], shift);
+    else if (UP == 64) tcw_build_t<64, 1>(U, C, att, Rp, P, b1, ffk, true, true, out[0], out[1], shift);
   }
 }
 

@@ -77,18 +77,12 @@ int dgrp_ctx_timings(dgrp_ctx *ctx, dgrp_timings_t *out);
 int64_t dgrp_ctx_launch_count(dgrp_ctx *ctx);
 /* tuning knobs and diagnostics: "mss_chunk" (elements per MSS scan chunk, 0 = automatic),
  * "mss_max_rounds" (parallel rounds before the sequential completion), "forward_tc" (1 = tcgen05
- * recurrence where available, 0 = fp32 kernel), "forward_sum16" (tcgen05 forward: 1 = the
- * h_fwd + h_rc scratch that feeds the attention scores is kept in half precision [default; a
- * probability moves by <= 3e-5 on sharp-attention weights and ~1e-7 on random-init ones], 0 = in
- * float32 [+5 % forward time]), "forward_fp16x2" (tcgen05 forward: operands of the recurrent
- * product as 1 = two scaled fp16 pieces, three products [default], 0 = three bf16 pieces, six
- * products [+15 % forward time, same measured accuracy]), "shard_rank" / "shard_world" (contig sharding of
+ * recurrence where available, 0 = fp32 kernel), "shard_rank" / "shard_world" (contig sharding of
  * dgrp_predict_fasta*: records are assigned largest-first to the least loaded rank; a rank
  * computes only its own records), and read-only "mss_rounds" (rounds the last MSS call used;
  * negative = completed sequentially), "forward_used_tc" (what the last forward used: 0 fp32 kernel, 1 two-tile tcgen05, 2 wide tcgen05 with one CTA per
  * tile, 3 wide tcgen05 CTA pair), "fused_last", "sm_count".  Round 2: "forward_wide" (0 auto, 1 / 2 force the wide
- * kernel's one-CTA / CTA-pair variant where it exists), "forward_ub" (GRU column blocks of 64 or 32 units),
- * "forward_overlap" (issue the wide kernel's MMAs block by block under the gate work), "forward_slab_mb" (bound of the
+ * kernel's one-CTA / CTA-pair variant where it exists), "forward_slab_mb" (bound of the
  * window-probability buffer), "forward_fuse_score" (fuse vote + score transform for whole-record calls),
  * "stream_slot_mb" (host piece size of dgrp_fasta_stream), "stream_early_rows" / "stream_early_slabs" /
  * "stream_early_ratio" / "stream_early_unit" (position slabs of a long record in dgrp_fasta_stream; get-only
