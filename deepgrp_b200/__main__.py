@@ -135,6 +135,11 @@ class CommandLineParser:
         sub["predict"].add_argument("--stepwise", action="store_true",
                                     help="Run the reference's five Python-level calls per record instead of the "
                                          "fused whole-record GPU call")
+        sub["predict"].add_argument("--mask", type=str, default=None, metavar="FILE",
+                                    help="Also write the input FASTA with the predicted repeats masked to FILE "
+                                         "('-' = stdout, when --output is a file); every input file in order")
+        sub["predict"].add_argument("--mask_mode", choices=("soft", "hard"), default="soft",
+                                    help="soft: lower-case the masked bases; hard: replace them by N")
         for name, text in (("parameter", "TOML file of hyper-parameters (Options)"),
                            ("trainfile", "one-hot .npz of the training chromosome (preprocess_sequence)"),
                            ("validfile", "one-hot .npz of the validation chromosome"),
@@ -160,6 +165,11 @@ class CommandLineParser:
                     break
             argv.insert(i, "predict")
         args = self.parser.parse_args(argv)
+        if getattr(args, "mask", None) is not None:
+            if args.stepwise:
+                self.parser.error("--mask is not available with --stepwise")
+            if args.mask == "-" and args.output == "-":
+                self.parser.error("--mask - needs --output to name a file")
         self.threads = args.threads
         self.verbose = args.verbose
         self.xla = args.xla
@@ -193,6 +203,20 @@ class CommandLineParser:
         _LOG.info("Model loading finished successfully!")
         outstream = sys.stdout if args.output == "-" else open(args.output, "w")
         use_mss = not args.no_use_mss
+        mask = getattr(args, "mask", None)
+        maskstream = None
+        if mask is not None:
+            maskstream = _ByteSink(sys.stdout) if mask == "-" else open(mask, "wb")
+        try:
+            CommandLineParser._predict_files(args, options, model, outstream, use_mss, maskstream)
+        finally:
+            if maskstream is not None and mask != "-":
+                maskstream.close()
+        if args.output != "-":
+            outstream.close()
+
+    @staticmethod
+    def _predict_files(args, options, model, outstream, use_mss, maskstream):
         for filename in args.FASTA:
             _LOG.info("Processing %s", filename)
             if getattr(args, "stepwise", False):
@@ -214,6 +238,13 @@ class CommandLineParser:
                 finally:
                     if filename != "-":
                         filestream.close()
+            elif maskstream is not None:
+                # slice by slice: each slice's rows, then its masked text
+                stats = dgpred.predict_fasta_tsv_masked(
+                    model, _read_raw(filename), filename, _ByteSink(outstream), maskstream, args.step_size,
+                    options.batch_size, use_mss, options.min_mss_len, options.xdrop_len, args.mask_mode)
+                _LOG.info("%s: %d records, %d bases, %d rows, masked", filename, stats["records"], stats["bases"],
+                          stats["rows"])
             else:
                 # records stream through the GPU pipeline; a record's rows are written as soon as it is done,
                 # so an error in a later record leaves the earlier rows in the output, as in the reference
@@ -222,8 +253,6 @@ class CommandLineParser:
                     options.batch_size, use_mss, options.min_mss_len, options.xdrop_len)
                 _LOG.info("%s: %d records, %d bases, %d rows", filename, stats["records"], stats["bases"],
                           stats["rows"])
-        if args.output != "-":
-            outstream.close()
 
     @staticmethod
     def train(args: argparse.Namespace, options: dgmodel.Options):

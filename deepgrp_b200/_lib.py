@@ -19,6 +19,7 @@ LIB_PATH = os.environ.get("DEEPGRP_B200_LIB") or os.path.join(_HERE, "libdeepgrp
 
 OK, E_CUDA, E_ARG, E_NOGPU, E_ALLN, E_CAPACITY, E_UNSUPPORTED, E_FASTA = 0, -1, -2, -3, -4, -5, -6, -7
 COMPAT_REFERENCE, COMPAT_FIXED = 0, 1
+MASK_SOFT, MASK_HARD = 0, 1
 
 
 class DeepgrpError(RuntimeError):
@@ -91,6 +92,8 @@ SIGNATURES = {
     "dgrp_predict_fasta": (_I, [_P, _P, _P, _L, _I, _I, _I, _I, _I, _I, _PL, _PL]),
     "dgrp_predict_fasta_tsv": (_I, [_P, _P, _P, _L, ctypes.c_char_p, _I, _I, _I, _I, _I, _I,
                                     ctypes.POINTER(_P), _PL, _PL, _PL]),
+    "dgrp_mask_fasta": (_I, [_P, _P, _L, _P, _L, _I, _P]),
+    "dgrp_mask_fasta_last": (_I, [_P, _P, _L, _I, _P]),
     "dgrp_fasta_rows": (_I, [_P, _P, _L]),
     "dgrp_fasta_records": (_I, [_P, _P, _P, _P, _P, _L]),
     "dgrp_fasta_record_tsv": (_I, [_P, _P, _P, _P, _L]),

@@ -278,6 +278,7 @@ int dgrp_ctx_destroy(dgrp_ctx *c) {
   for (auto b : bufs) b->release();
   c->pin_small.release(); c->pin_a.release(); c->pin_b.release(); c->tsv_host.release();
   c->tsv_dev.release(); c->tsv_prefix.release();
+  c->fa_tri.release(); c->mask_rec.release(); c->mask_bits.release(); c->mask_out.release();
   for (int i = 0; i < 2; ++i) { c->st_raw[i].release(); c->st_text[i].release(); c->st_stage[i].release(); }
   for (int i = 0; i < 4; ++i) c->st_slot[i].release();
   for (auto &e : c->ev) cudaEventDestroy(e);
@@ -783,6 +784,22 @@ int dgrp_predict_sequence(dgrp_ctx *c, dgrp_model *m, const uint8_t *seq, int64_
   return rc;
 }
 
+// buf[used, used + bytes) = d_src[0, bytes) (device to device), growing buf and keeping buf[0, used)
+static int append_dev(dgrp_ctx *c, DevBuf &buf, size_t used, const void *d_src, size_t bytes) {
+  if (used + bytes > buf.cap) {
+    DevBuf bigger;
+    DGRP_CHECK(bigger.reserve(std::max(used + bytes, buf.cap * 2)));
+    if (used) DGRP_CUDA(cudaMemcpyAsync(bigger.p, buf.p, used, cudaMemcpyDeviceToDevice, c->stream));
+    DGRP_CUDA(cudaStreamSynchronize(c->stream));
+    bigger.reserves = buf.reserves;
+    buf.release();
+    buf = bigger;
+  }
+  ++buf.reserves;
+  DGRP_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(buf.p) + used, d_src, bytes, cudaMemcpyDeviceToDevice, c->stream));
+  return DGRP_OK;
+}
+
 // filename == nullptr: rows are copied to the host (c->fa_rows); else the TSV text is produced on
 // the device and lands in c->tsv_host.
 static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, int64_t nbytes,
@@ -798,6 +815,9 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
   c->fa_rows.clear(); c->fa_hdr_off.clear(); c->fa_hdr_len.clear();
   c->fa_startpos.clear(); c->fa_length.clear();
   c->fa_tsv_off.clear(); c->fa_tsv_len.clear(); c->fa_owner.clear();
+  c->fa_seq_base.clear(); c->fa_row_off.clear();
+  c->mask_nbytes = -1;
+  int64_t dev_rows = 0;             // rows appended to c->fa_tri
   DGRP_REQUIRE(nbytes >= 0, "negative length");
   stamp(c, 0);
   DGRP_CHECK(c->raw.reserve((size_t)nbytes + 16));
@@ -852,6 +872,7 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
       c->fa_hdr_off.push_back(b); c->fa_hdr_len.push_back(e - b);
       c->fa_startpos.push_back(-1); c->fa_length.push_back(hseq[k + 1] - hseq[k]);
       c->fa_tsv_off.push_back(c->tsv_len); c->fa_tsv_len.push_back(0); c->fa_owner.push_back(owner_of[k]);
+      c->fa_seq_base.push_back(hseq[k]); c->fa_row_off.push_back(dev_rows);
       continue;
     }
     const uint8_t *d_seq = c->io_b.as<uint8_t>() + hseq[k];
@@ -868,6 +889,7 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
     c->fa_hdr_off.push_back(b); c->fa_hdr_len.push_back(e - b);
     c->fa_startpos.push_back(startpos); c->fa_length.push_back(length);
     c->fa_tsv_off.push_back(c->tsv_len); c->fa_tsv_len.push_back(0); c->fa_owner.push_back(owner_of[k]);
+    c->fa_seq_base.push_back(hseq[k]); c->fa_row_off.push_back(dev_rows);
     stamp(c, 1);
     if ((rc = core_predict(c, m, c->codes.as<uint8_t>(), length, step, batch_size, compat, use_mss != 0))) break;
     windows += c->timings.windows; bases += length;
@@ -879,6 +901,9 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
       int64_t cnt = 0;
       if ((rc = run_segments(c, c->labels2.as<uint8_t>(), nullptr, length, startpos, false, &d_tri, &cnt))) break;
       total_rows += cnt;
+      // the rows stay on the device as well, for dgrp_mask_fasta_last
+      if (cnt > 0 && (rc = append_dev(c, c->fa_tri, (size_t)dev_rows * 24, d_tri, (size_t)cnt * 24))) break;
+      dev_rows += cnt;
       if (cnt > 0 && filename) {
         // prefix = "<filename>\t<header>\t"
         std::string prefix(filename, fn_len);
@@ -944,6 +969,11 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
   t.kernel_launches = c->launches - launches0;
   *n_rows = total_rows;
   *n_records = (int64_t)c->fa_hdr_off.size();
+  if (rc == DGRP_OK && c->shard_world <= 1) {
+    c->fa_row_off.push_back(dev_rows);
+    c->mask_nbytes = nbytes;
+    c->mask_raw_reserves = c->raw.reserves;
+  }
   return rc;
 }
 
@@ -964,6 +994,100 @@ int dgrp_predict_fasta_tsv(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, int
                                     min_mss_len, xdrop_len, compat, n_rows, n_records);
   if (rc == DGRP_OK) { *tsv = c->tsv_host.as<uint8_t>(); *tsv_len = c->tsv_len; }
   return rc;
+}
+
+/* -------------------------------------- masking ---------------------------------------- */
+
+// Record table of run_mask: rec[2 r] = first sequence rank of kept record r, rec[2 r + 1] = its first row; one
+// more pair for the end (rows in total).  Uploaded to c->mask_rec, followed by `tri` (host triples) if given.
+static int mask_upload(dgrp_ctx *c, const std::vector<int64_t> &base, const std::vector<int64_t> &row_off,
+                       int64_t n_seq, const std::vector<int64_t> &tri, const int64_t **d_rec, const int64_t **d_tri) {
+  const size_t n_rec = base.size();
+  std::vector<int64_t> h(2 * (n_rec + 1) + tri.size());
+  for (size_t r = 0; r <= n_rec; ++r) {
+    h[2 * r] = r < n_rec ? base[r] : n_seq;
+    h[2 * r + 1] = row_off[r];
+  }
+  std::copy(tri.begin(), tri.end(), h.begin() + 2 * (n_rec + 1));
+  DGRP_CHECK(c->mask_rec.reserve(h.size() * 8));
+  DGRP_CUDA(cudaMemcpyAsync(c->mask_rec.p, h.data(), h.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  *d_rec = c->mask_rec.as<int64_t>();
+  *d_tri = c->mask_rec.as<int64_t>() + 2 * (n_rec + 1);
+  return DGRP_OK;
+}
+
+static int mask_finish(dgrp_ctx *c, int64_t nbytes, const FastaScan &f, const int64_t *d_tri, const int64_t *d_rec,
+                       int64_t n_rec, int mode, uint8_t *out) {
+  DGRP_CHECK(c->mask_out.reserve((size_t)nbytes + 16));
+  DGRP_CHECK(run_mask(c, c->raw.as<uint8_t>(), nbytes, f, d_tri, d_rec, n_rec, mode, c->mask_out.as<uint8_t>()));
+  DGRP_CUDA(cudaMemcpyAsync(out, c->mask_out.p, (size_t)nbytes, cudaMemcpyDeviceToHost, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  return DGRP_OK;
+}
+
+int dgrp_mask_fasta(dgrp_ctx *c, const uint8_t *fasta, int64_t nbytes, const dgrp_row_t *rows, int64_t n_rows,
+                    int mode, uint8_t *out) {
+  Use use(c->device);
+  DGRP_REQUIRE(mode == DGRP_MASK_SOFT || mode == DGRP_MASK_HARD, "mask mode must be DGRP_MASK_SOFT or DGRP_MASK_HARD");
+  DGRP_REQUIRE(nbytes >= 0 && n_rows >= 0, "negative length");
+  DGRP_CHECK(c->raw.reserve((size_t)nbytes + 16));
+  if (nbytes > 0) DGRP_CUDA(cudaMemcpyAsync(c->raw.p, fasta, (size_t)nbytes, cudaMemcpyHostToDevice, c->stream));
+  int64_t n_seq = 0, n_hdr = 0;
+  FastaScan f = {};
+  DGRP_CHECK(run_fasta_decode(c, c->raw.as<uint8_t>(), nbytes, &n_seq, &n_hdr, &f));
+  // kept records (non-empty header, __main__.py:36): first rank and untrimmed length
+  auto ws = [](uint8_t b) { return (b >= 9 && b <= 13) || (b >= 28 && b <= 32); };
+  std::vector<int64_t> base, len;
+  const int64_t *t = c->pin_b.as<int64_t>();
+  for (int64_t k = 0; k < n_hdr; ++k) {
+    int64_t b = t[k] + 1, e = b;
+    while (e < nbytes && fasta[e] != '\n' && !(fasta[e] == '\r' && !(e + 1 < nbytes && fasta[e + 1] == '\n'))) ++e;
+    while (e > b && ws(fasta[e - 1])) --e;
+    if (e == b) continue;
+    const int64_t s0 = t[(n_hdr + 1) + k], s1 = k + 1 < n_hdr ? t[(n_hdr + 1) + k + 1] : n_seq;
+    base.push_back(s0); len.push_back(s1 - s0);
+  }
+  const int64_t n_rec = (int64_t)base.size();
+  std::vector<int64_t> row_off(n_rec + 1, n_rows), tri((size_t)n_rows * 3);
+  for (int64_t i = 0; i < n_rows; ++i) {
+    const dgrp_row_t &r = rows[i];
+    DGRP_REQUIRE(r.record >= 0 && r.record < n_rec, "row %lld: record %d out of range (%lld records)", (long long)i,
+                 (int)r.record, (long long)n_rec);
+    DGRP_REQUIRE(r.start >= 0 && r.start < r.end && r.end <= len[r.record],
+                 "row %lld: [%lld, %lld) is not inside record %d of length %lld", (long long)i, (long long)r.start,
+                 (long long)r.end, (int)r.record, (long long)len[r.record]);
+    DGRP_REQUIRE(r.label > 0, "row %lld: label %d is not positive", (long long)i, (int)r.label);
+    if (i > 0) {
+      const dgrp_row_t &p = rows[i - 1];
+      DGRP_REQUIRE(p.record < r.record || (p.record == r.record && p.end <= r.start),
+                   "row %lld: rows must be sorted by (record, start) and disjoint within a record", (long long)i);
+    }
+    if (i == 0 || rows[i - 1].record != r.record)
+      for (int64_t q = i == 0 ? 0 : rows[i - 1].record + 1; q <= r.record; ++q) row_off[q] = i;
+    tri[3 * i] = r.start; tri[3 * i + 1] = r.end; tri[3 * i + 2] = r.label;
+  }
+  for (int64_t q = n_rows > 0 ? rows[n_rows - 1].record + 1 : 0; q <= n_rec; ++q) row_off[q] = n_rows;
+  if (nbytes == 0) return DGRP_OK;
+  const int64_t *d_rec = nullptr, *d_tri = nullptr;
+  DGRP_CHECK(mask_upload(c, base, row_off, n_seq, tri, &d_rec, &d_tri));
+  return mask_finish(c, nbytes, f, d_tri, d_rec, n_rec, mode, out);
+}
+
+int dgrp_mask_fasta_last(dgrp_ctx *c, const uint8_t *fasta, int64_t nbytes, int mode, uint8_t *out) {
+  Use use(c->device);
+  (void)fasta;   // its copy on the device (c->raw) is masked
+  DGRP_REQUIRE(mode == DGRP_MASK_SOFT || mode == DGRP_MASK_HARD, "mask mode must be DGRP_MASK_SOFT or DGRP_MASK_HARD");
+  DGRP_REQUIRE(c->mask_nbytes >= 0 && c->mask_raw_reserves == c->raw.reserves,
+               "no dgrp_predict_fasta result to mask: none ran, it failed or was sharded, or another call has used "
+               "its buffers since");
+  DGRP_REQUIRE(nbytes == c->mask_nbytes, "the last dgrp_predict_fasta had %lld bytes, not %lld",
+               (long long)c->mask_nbytes, (long long)nbytes);
+  if (nbytes == 0) return DGRP_OK;
+  FastaScan f = {};
+  DGRP_CHECK(run_fasta_classify(c, c->raw.as<uint8_t>(), nbytes, &f));
+  const int64_t *d_rec = nullptr, *d_tri = nullptr;
+  DGRP_CHECK(mask_upload(c, c->fa_seq_base, c->fa_row_off, f.n_seq, {}, &d_rec, &d_tri));
+  return mask_finish(c, nbytes, f, c->fa_tri.as<int64_t>(), d_rec, (int64_t)c->fa_seq_base.size(), mode, out);
 }
 
 int dgrp_fasta_rows(dgrp_ctx *c, dgrp_row_t *rows, int64_t cap) {

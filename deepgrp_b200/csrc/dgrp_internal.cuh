@@ -134,6 +134,14 @@ struct dgrp_ctx {
   // buffer has been reserved since)
   int64_t codes_dev_length = -1, codes_dev_rows = 0;
   uint64_t codes_dev_reserves[2] = {};
+  // the last dgrp_predict_fasta[_tsv] for dgrp_mask_fasta_last: every kept record's first sequence rank and first
+  // row (one more row entry: the total), its rows on the device as (start, end, label) triples, its byte count
+  // (-1: it failed, was sharded, or none ran) and the reserve count of c->raw (its text) when it returned
+  std::vector<int64_t> fa_seq_base, fa_row_off;
+  dgrp::DevBuf fa_tri;
+  int64_t mask_nbytes = -1;
+  uint64_t mask_raw_reserves = 0;
+  dgrp::DevBuf mask_rec, mask_bits, mask_out;   // dgrp_mask_fasta*: record table, rank bitmap, masked text
   int shard_rank = 0, shard_world = 1;   // contig sharding of dgrp_predict_fasta* (dgrp_ctx_set_int)
   dgrp::PinBuf tsv_host;     // finished TSV text of the last dgrp_predict_fasta_tsv
   int64_t tsv_len = 0;
@@ -249,7 +257,22 @@ int run_gap_fill(dgrp_ctx *c, const dgrp_seg_t *d_segs, int n_seg, const uint8_t
                  const int64_t *d_label64_in, int n, int nof_labels, uint8_t *d_label_out);
 int launch_labels_to_onehot(dgrp_ctx *c, const uint8_t *d_label, int64_t n, int C, double *d_out);
 // fasta.cu
-int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_seq, int64_t *n_hdr);
+struct FastaScan {              // classification of a FASTA buffer (device arrays in c->scan)
+  int64_t ntiles;
+  uint8_t *tile_state;          // [ntiles] line state in front of every tile
+  unsigned *seq_off, *hdr_off;  // [ntiles] sequence bytes / headers in front of every tile
+  int64_t n_seq, n_hdr;         // totals
+};
+int run_fasta_classify(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, FastaScan *f);
+int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_seq, int64_t *n_hdr,
+                     FastaScan *scan = nullptr);
+// mask.cu
+// Masked copy of the FASTA buffer d_raw[n] (classified in f) into d_out[n]: a sequence byte of rank q is masked
+// when a row of kept record r covers q - rec[2 r] (rec[2 r]: rank of the record's first sequence byte,
+// rec[2 r + 1]: index of its first row in d_tri; rec[2 n_rec + 1] = number of rows).  d_tri: (start, end, label)
+// triples, sorted and disjoint within a record, records in rank order.
+int run_mask(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, const FastaScan &f, const int64_t *d_tri,
+             const int64_t *d_rec, int64_t n_rec, int mode, uint8_t *d_out);
 // tsv.cu
 int run_tsv_measure(dgrp_ctx *c, const int64_t *d_tri, int64_t n, int prefix_len, int64_t *need);
 int run_tsv_write(dgrp_ctx *c, const int64_t *d_tri, int64_t n, const uint8_t *d_prefix,

@@ -14,58 +14,12 @@
 // of sequence bytes in front of every header gives the record boundaries.
 #include "dgrp_internal.cuh"
 #include "fasta_core.cuh"
+#include "fasta_dev.cuh"
 
 namespace dgrp {
 
 using namespace fa;
 
-constexpr int FA_THREADS = 256;
-constexpr int FA_TILE = FA_THREADS * FA_ITEMS;
-
-// Exclusive block scan of per-thread functions; returns the function of everything before this
-// thread in the tile, *total receives the whole tile's function.
-__device__ unsigned block_scan_fn(unsigned f, unsigned *total) {
-  __shared__ unsigned s_w[FA_THREADS / 32];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  unsigned incl = f;
-  for (int off = 1; off < 32; off <<= 1) {
-    const unsigned t = __shfl_up_sync(0xffffffffu, incl, off);
-    if (lane >= off) incl = compose(t, incl);
-  }
-  if (lane == 31) s_w[warp] = incl;
-  __syncthreads();
-  unsigned before = FN_IDENT;
-  for (int w = 0; w < warp; ++w) before = compose(before, s_w[w]);
-  unsigned excl = __shfl_up_sync(0xffffffffu, incl, 1);
-  if (lane == 0) excl = FN_IDENT;
-  unsigned tot = FN_IDENT;
-  for (int w = 0; w < FA_THREADS / 32; ++w) tot = compose(tot, s_w[w]);
-  *total = tot;
-  __syncthreads();
-  return compose(before, excl);
-}
-
-// The FA_ITEMS bytes of one thread plus one look-ahead byte, in registers: one 16-byte load per thread
-// (byte loads for the last, partial vector of the buffer or an unaligned source).  Bytes past the end
-// read as 0, which is neither '\n' nor whitespace.  Every thread of the block must call load_items.
-__device__ __forceinline__ void load_items(const uint8_t *__restrict__ raw, int64_t n, int64_t base, Items &it) {
-  static_assert(FA_ITEMS == 16, "one uint4 per thread");
-  const int64_t left = n - base;
-  it.cnt = left <= 0 ? 0 : (left < FA_ITEMS ? (int)left : FA_ITEMS);
-  if (it.cnt == FA_ITEMS && (reinterpret_cast<uintptr_t>(raw + base) & 15) == 0) {
-    const uint4 v = __ldg(reinterpret_cast<const uint4 *>(raw + base));
-    const unsigned w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-    for (int k = 0; k < FA_ITEMS; ++k) it.b[k] = (w[k >> 2] >> (8 * (k & 3))) & 0xffu;
-  } else {
-#pragma unroll
-    for (int k = 0; k < FA_ITEMS; ++k) it.b[k] = k < it.cnt ? (unsigned)raw[base + k] : 0u;
-  }
-  // look-ahead byte = first byte of the next thread; the last lane of a warp reads it from memory
-  unsigned next = __shfl_down_sync(0xffffffffu, it.b[0], 1);
-  if ((threadIdx.x & 31) == 31) next = left > FA_ITEMS ? (unsigned)raw[base + FA_ITEMS] : 0u;
-  it.b[FA_ITEMS] = next;
-}
 __global__ void fa_tile_fn_kernel(const uint8_t *__restrict__ raw, int64_t n, unsigned *tile_fn) {
   const int64_t base = (int64_t)blockIdx.x * FA_TILE + (int64_t)threadIdx.x * FA_ITEMS;
   Items it;
@@ -193,12 +147,10 @@ __global__ void fa_scatter_kernel(const uint8_t *__restrict__ raw, int64_t n,
 
 __global__ void cp_scan_kernel(unsigned int *a, int64_t m, unsigned long long *total);
 
-// Decode `n` raw bytes on the device.  Outputs (device): compacted sequence bytes in c->io_b,
-// header table in c->rows (hdr_pos | hdr_seq).  Host: *n_seq, *n_hdr, and the header table copied
-// into c->pin_b (hdr_pos[n_hdr], hdr_seq[n_hdr]).
-int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_seq, int64_t *n_hdr) {
-  *n_seq = 0; *n_hdr = 0;
-  if (n <= 0) return DGRP_OK;
+// Classify `n` raw bytes on the device (the part of the decode that the mask kernels share, csrc/mask.cu):
+// the state in front of every tile, and per tile the exclusive scans of the sequence-byte and header counts.
+// Five launches and one synchronisation; a blank line is DGRP_E_FASTA.  The arrays live in c->scan.
+int run_fasta_classify(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, FastaScan *f) {
   DGRP_REQUIRE(n < (int64_t)4000000000LL, "FASTA buffers above 4e9 bytes must be split by record");
   const int64_t ntiles = (n + FA_TILE - 1) / FA_TILE;
   const size_t a = ((size_t)ntiles * 4 + 255) / 256 * 256;
@@ -233,13 +185,32 @@ int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_se
     set_error("string index out of range (blank line in FASTA input)");
     return DGRP_E_FASTA;
   }
+  f->ntiles = ntiles;
+  f->tile_state = tile_state;
+  f->seq_off = seq_cnt;
+  f->hdr_off = hdr_cnt;
+  f->n_seq = total_seq;
+  f->n_hdr = total_hdr;
+  return DGRP_OK;
+}
+
+// Decode `n` raw bytes on the device.  Outputs (device): compacted sequence bytes in c->io_b,
+// header table in c->rows (hdr_pos | hdr_seq).  Host: *n_seq, *n_hdr, and the header table copied
+// into c->pin_b (hdr_pos[n_hdr], hdr_seq[n_hdr]).  *scan (if set) receives the classification, which stays
+// valid until c->scan is reserved again.
+int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_seq, int64_t *n_hdr, FastaScan *scan) {
+  *n_seq = 0; *n_hdr = 0;
+  if (n <= 0) return DGRP_OK;
+  FastaScan f;
+  DGRP_CHECK(run_fasta_classify(c, d_raw, n, &f));
+  const int64_t total_seq = f.n_seq, total_hdr = f.n_hdr;
   DGRP_CHECK(c->io_b.reserve((size_t)total_seq + 64));
   DGRP_CHECK(c->rows.reserve((size_t)(total_hdr + 1) * 16));
   int64_t *hdr_pos = c->rows.as<int64_t>();
   int64_t *hdr_seq = hdr_pos + (total_hdr + 1);
   if (total_seq > 0 || total_hdr > 0) {
-    fa_scatter_kernel<<<(unsigned)ntiles, FA_THREADS, 0, c->stream>>>(
-        d_raw, n, tile_state, seq_cnt, hdr_cnt, 0, c->io_b.as<uint8_t>(), hdr_pos, hdr_seq);
+    fa_scatter_kernel<<<(unsigned)f.ntiles, FA_THREADS, 0, c->stream>>>(
+        d_raw, n, f.tile_state, f.seq_off, f.hdr_off, 0, c->io_b.as<uint8_t>(), hdr_pos, hdr_seq);
     c->launches++;
   }
   DGRP_CHECK(c->pin_b.reserve((size_t)(total_hdr + 1) * 16));
@@ -251,6 +222,7 @@ int run_fasta_decode(dgrp_ctx *c, const uint8_t *d_raw, int64_t n, int64_t *n_se
   DGRP_CUDA(cudaGetLastError());
   *n_seq = total_seq;
   *n_hdr = total_hdr;
+  if (scan) *scan = f;
   return DGRP_OK;
 }
 

@@ -27,6 +27,7 @@ from .model import ModelWeights, Options, create_model, load_model
 from . import preprocessing  # noqa: F401  (Data, as in the reference's import list)
 
 _COMPAT = {"reference": _lib.COMPAT_REFERENCE, "fixed": _lib.COMPAT_FIXED}
+_MASK = {"soft": _lib.MASK_SOFT, "hard": _lib.MASK_HARD}
 
 
 class WindowDataset:
@@ -411,6 +412,70 @@ def predict_fasta_tsv(model: ModelWeights, raw, filename: str, step_size: int, b
     """``predict_fasta_tsv_view`` copied into a ``str``."""
     return bytes(predict_fasta_tsv_view(model, raw, filename, step_size, batch_size, use_mss,
                                         min_mss_len, xdrop_len, compat)).decode("utf-8", "replace")
+
+
+def _mask_mode(mode: str) -> int:
+    if mode not in _MASK:
+        raise ValueError("mask mode must be 'soft' or 'hard', not %r" % (mode,))
+    return _MASK[mode]
+
+
+def mask_fasta(raw, rows: np.ndarray, mode: str = "soft") -> bytes:
+    """The FASTA text ``raw`` with the positions that ``rows`` cover masked, on the GPU: lower-cased (``soft``,
+    ASCII ``A``-``Z`` only) or replaced by ``N`` (``hard``).  ``rows`` is the structured array
+    :func:`predict_fasta` returns (``record`` indexes the records with a non-empty header, untrimmed
+    coordinates); it must be sorted by (record, start) and disjoint within a record.  Every other byte is copied
+    unchanged, so the result has the length of ``raw``.  A blank line raises ``IndexError``."""
+    code = _mask_mode(mode)
+    ctx = _lib.context()
+    n = len(raw)
+    buf = np.frombuffer(raw, dtype=np.uint8) if n else np.zeros(0, np.uint8)
+    rows = np.ascontiguousarray(rows, dtype=_lib.ROW_DTYPE)
+    out = np.empty(max(n, 1), dtype=np.uint8)
+    rc = _lib.lib().dgrp_mask_fasta(ctx.handle, _lib.ptr(buf), n, _lib.ptr(rows), rows.size, code, _lib.ptr(out))
+    if rc == _lib.E_FASTA:
+        raise IndexError("string index out of range")
+    _lib.check(rc)
+    return out[:n].tobytes()
+
+
+def predict_fasta_tsv_masked(model: ModelWeights, raw, filename: str, outstream, maskstream, step_size: int,
+                             batch_size: int, use_mss: bool, min_mss_len: int, xdrop_len: int, mode: str = "soft",
+                             compat: str = "reference") -> dict:
+    """:func:`predict_fasta_tsv_stream` that also writes the masked text of ``raw`` (see :func:`mask_fasta`) to
+    the binary stream ``maskstream``.  The file runs slice by slice (whole records, >= 8 MiB, the streaming
+    driver's cuts with one rank), which bounds device memory: each slice is predicted in one call, its TSV text is
+    written, and its rows, still on the device, mask its bytes.  A slice with a blank line or an all-``N`` record
+    is run again through :func:`predict_fasta_tsv_stream`, so the TSV text holds the rows of the records before the
+    error, as the default route writes them, and the same ``IndexError`` / ``ValueError`` is raised; the masked
+    text then holds the slices before that one.  Returns the totals (rows, records, bases, slices)."""
+    from .sharding import fasta_slices
+    code = _mask_mode(mode)
+    ctx = _lib.context()
+    cuts, _ = fasta_slices(raw, 1)
+    whole = memoryview(raw) if len(raw) else memoryview(b"")
+    totals = {"rows": 0, "records": 0, "bases": 0, "slices": len(cuts) - 1}
+    for k in range(len(cuts) - 1):
+        piece = whole[int(cuts[k]):int(cuts[k + 1])]
+        try:
+            view, n_rows, n_rec = _fasta_tsv_call(model, piece, filename, step_size, batch_size, use_mss,
+                                                  min_mss_len, xdrop_len, compat)
+        except (IndexError, ValueError):
+            predict_fasta_tsv_stream(model, piece, filename, outstream, step_size, batch_size, use_mss,
+                                     min_mss_len, xdrop_len, compat)
+            raise RuntimeError("slice %d failed in the whole-slice call but not in the stream" % k)
+        totals["bases"] += int(ctx.timings()["bases"])
+        totals["rows"] += n_rows
+        totals["records"] += n_rec
+        if len(view):
+            outstream.write(view)
+        n = len(piece)
+        if n:
+            buf = np.frombuffer(piece, dtype=np.uint8)
+            out = np.empty(n, dtype=np.uint8)
+            _lib.check(_lib.lib().dgrp_mask_fasta_last(ctx.handle, _lib.ptr(buf), n, code, _lib.ptr(out)))
+            maskstream.write(out)
+    return totals
 
 
 # ---- evaluation helpers (deepgrp/prediction.py:144-260; used by deepgrp/optimization.py:58-69) -------

@@ -224,6 +224,24 @@ int dgrp_predict_fasta_tsv(dgrp_ctx *ctx, dgrp_model *model, const uint8_t *fast
                            const char *filename, int step, int batch_size, int use_mss,
                            int min_mss_len, int xdrop_len, int compat, const uint8_t **tsv,
                            int64_t *tsv_len, int64_t *n_rows, int64_t *n_records);
+/* Repeat-masked FASTA text: out[nbytes] (host) is the input with every position that a row covers lower-cased
+ * (DGRP_MASK_SOFT: ASCII 'A'-'Z' only, other bytes unchanged) or replaced by 'N' (DGRP_MASK_HARD); every other
+ * byte (headers, terminators, strip() whitespace, text in front of the first '>', records with an empty header,
+ * unmasked positions) is copied unchanged.  A position is a byte of a sequence line inside the line's strip()
+ * span, as _read_multi_fasta counts them (__main__.py:20-43); position p of record r is masked when a row of r has
+ * start <= p < end (untrimmed coordinates).  rows[i].record indexes the kept records in file order, as in
+ * dgrp_fasta_records.  The text is decoded on the GPU by the call.  DGRP_E_ARG for a bad mode, a record index out
+ * of range, start < 0 or end > the record's untrimmed length or start >= end, label <= 0, or rows that are not
+ * sorted by (record, start) or overlap within a record; DGRP_E_FASTA for a blank line. */
+#define DGRP_MASK_SOFT 0
+#define DGRP_MASK_HARD 1
+int dgrp_mask_fasta(dgrp_ctx *ctx, const uint8_t *fasta, int64_t nbytes, const dgrp_row_t *rows, int64_t n_rows,
+                    int mode, uint8_t *out);
+/* The same with the record table and rows that the last dgrp_predict_fasta[_tsv] on this context left on the
+ * device (no row goes to the host); `fasta` and `nbytes` must be that call's text.  DGRP_E_ARG when that call
+ * failed or was sharded (shard_world > 1), when nbytes differs from its, or when another call has overwritten
+ * its text on the device since. */
+int dgrp_mask_fasta_last(dgrp_ctx *ctx, const uint8_t *fasta, int64_t nbytes, int mode, uint8_t *out);
 /* rows[i].record indexes the record table */
 int dgrp_fasta_rows(dgrp_ctx *ctx, dgrp_row_t *rows, int64_t cap);
 /* per record: header text = fasta[hdr_off, hdr_off + hdr_len); startpos = leading 'N' count;
