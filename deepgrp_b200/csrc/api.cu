@@ -147,15 +147,13 @@ static int core_labels(dgrp_ctx *c, const float *d_pred, const uint8_t *d_lab_in
     DGRP_CHECK(run_mss_segments(c, nullptr, sc, (int)L, min_sc, xdrop, &d_segs, &n_seg));
     DGRP_CHECK(run_gap_fill(c, d_segs, n_seg, lab, nullptr, (int)L, C, c->labels2.as<uint8_t>()));
   } else {
-    // softmax (prediction.py:62-65) then argmax (__main__.py:83)
-    if (d_pred) {
-      DGRP_CHECK(c->io_a.reserve((size_t)L * C * 4));
-      DGRP_CHECK(launch_softmax_global(c, d_pred, L, C, c->io_a.as<float>()));
-      DGRP_CHECK(launch_score(c, c->io_a.as<float>(), L, C, c->labels2.as<uint8_t>(), nullptr,
-                              nullptr, nullptr));
-    } else {
-      DGRP_CUDA(cudaMemcpyAsync(c->labels2.p, d_lab_in, (size_t)L, cudaMemcpyDeviceToDevice, c->stream));
-    }
+    // softmax (prediction.py:62-65) then argmax (__main__.py:83); ready labels are the raw vote's argmax, which
+    // is not this (finish_requires_mss)
+    DGRP_REQUIRE(d_pred, "labels without MSS need the predictions");
+    DGRP_CHECK(c->io_a.reserve((size_t)L * C * 4));
+    DGRP_CHECK(launch_softmax_global(c, d_pred, L, C, c->io_a.as<float>()));
+    DGRP_CHECK(launch_score(c, c->io_a.as<float>(), L, C, c->labels2.as<uint8_t>(), nullptr,
+                            nullptr, nullptr));
     stamp(c, 3);
   }
   return DGRP_OK;
@@ -1406,6 +1404,17 @@ static int core_predict_range(dgrp_ctx *c, dgrp_model *m, const uint8_t *d_codes
   return launch_score(c, c->pred.as<float>(), rows, m->C, d_labels, d_scores, nullptr, nullptr);
 }
 
+// The gathered labels of a chunk-sharded record are each range's argmax of the raw vote.  Without MSS the
+// reference takes the argmax after a softmax with the record's global maximum (prediction.py:62-65), which rounds
+// the top two probabilities into a tie (first index wins) where they are a few ulp apart; no range sees that
+// maximum, so the finish would return other labels than the whole record at such positions.  Refused instead.
+static int finish_requires_mss(int use_mss) {
+  if (use_mss) return DGRP_OK;
+  set_error("finishing a chunk-sharded record needs use_mss: without MSS the labels are the argmax after a softmax "
+            "over the whole record's maximum, which the ranges' labels do not carry; predict the record whole");
+  return DGRP_E_UNSUPPORTED;
+}
+
 extern "C" {
 
 int dgrp_predict_range(dgrp_ctx *c, dgrp_model *m, const uint8_t *codes, int64_t codes_base,
@@ -1447,6 +1456,7 @@ int dgrp_finish_record(dgrp_ctx *c, const uint8_t *labels, const float *scores, 
                        uint8_t *labels_out, dgrp_row_t *rows, int64_t cap, int64_t *n_rows) {
   Use use(c->device);
   *n_rows = 0;
+  DGRP_CHECK(finish_requires_mss(use_mss));
   if (length <= 0) return DGRP_OK;
   DGRP_CHECK(c->labels.reserve((size_t)length));
   DGRP_CHECK(c->scores32.reserve((size_t)length * 4));
@@ -1467,6 +1477,7 @@ int dgrp_finish_record_dev(dgrp_ctx *c, const uint8_t *d_labels, const float *d_
   Use use(c->device);
   const int64_t launches0 = c->launches;
   *n_rows = 0;
+  DGRP_CHECK(finish_requires_mss(use_mss));
   stamp(c, 0); stamp(c, 1); stamp(c, 2);
   DGRP_CHECK(core_labels(c, nullptr, d_labels, d_scores, length, n_classes, use_mss, min_mss_len, xdrop_len));
   stamp(c, 4);

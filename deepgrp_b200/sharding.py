@@ -88,7 +88,12 @@ def predict_range(model, codes: np.ndarray, length: int, p0: int, p1: int, step_
 def finish_record(labels: np.ndarray, scores: np.ndarray, n_classes: int, use_mss: bool,
                   min_mss_len: int, xdrop_len: int, startpos: int):
     """MSS gap fill + segment rows from gathered (label, score) of a whole record
-    (``dgrp_finish_record``): returns (labels uint8[L], rows)."""
+    (``dgrp_finish_record``): returns (labels uint8[L], rows).  ``use_mss`` must be true: without MSS the
+    reference's labels are the argmax after a softmax over the whole record's maximum, which can round two close
+    probabilities into a tie that the ranges' labels (argmax of the raw vote) do not reproduce."""
+    if not use_mss:
+        raise ValueError("finish_record needs use_mss: without MSS the labels depend on the whole record's "
+                         "softmax, which the ranges' labels do not carry; predict the record whole")
     from . import _lib
     ctx = _lib.context()
     labels = np.ascontiguousarray(labels, dtype=np.uint8)

@@ -192,7 +192,10 @@ int dgrp_predict_sequence(dgrp_ctx *ctx, dgrp_model *model, const uint8_t *seq, 
 int dgrp_predict_range(dgrp_ctx *ctx, dgrp_model *model, const uint8_t *codes, int64_t codes_base,
                        int64_t codes_len, int64_t length, int64_t pos0, int64_t pos1, int step,
                        int batch_size, int compat, uint8_t *labels, float *scores);
-/* MSS gap fill + segment rows from gathered (label, score) of a whole record. */
+/* MSS gap fill + segment rows from gathered (label, score) of a whole record.  use_mss = 0 is refused
+ * (DGRP_E_UNSUPPORTED), here and in _finish_record_dev: without MSS the reference's labels are the argmax
+ * after a softmax over the record's global maximum, which can round two close probabilities into a tie
+ * that the ranges' raw-vote labels do not reproduce.  Predict such a record whole. */
 int dgrp_finish_record(dgrp_ctx *ctx, const uint8_t *labels, const float *scores, int64_t length,
                        int n_classes, int use_mss, int min_mss_len, int xdrop_len,
                        int64_t startpos, uint8_t *labels_out, dgrp_row_t *rows, int64_t cap,

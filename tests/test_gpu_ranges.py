@@ -497,12 +497,13 @@ def test_range_vote_forms_agree_bit_for_bit(dg, name, step, mode):
 # ------------------------------------------------------------------ 4. the owner's finish
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["a", "d"])
-def test_finish_record_of_gathered_ranges_equals_oracle(dg, oracle, name):
+def test_finish_record_of_gathered_ranges_equals_oracle_and_refuses_no_mss(dg, oracle, name):
     """dgrp_finish_record on the gathered labels and scores of 8 ranges: its labels are the oracle's MSS relabelling
-    (or the labels themselves without MSS) and its rows the oracle's segments with label 0 removed, bit for bit, at
-    several MSS settings and start positions.  dgrp_finish_record_dev is checked by its row count alone: it leaves
-    its labels and rows on the device, and the C ABI has no call that returns them (dgrp_predict_codes_dev_results
-    refuses them), so its labels are those of the host form, which runs the same code."""
+    and its rows the oracle's segments with label 0 removed, bit for bit, at several MSS settings and start
+    positions.  Both forms refuse to finish without MSS, whose labels the ranges' raw-vote labels do not give.
+    dgrp_finish_record_dev is checked by its row count alone: it leaves its labels and rows on the device, and the
+    C ABI has no call that returns them (dgrp_predict_codes_dev_results refuses them), so its labels are those of
+    the host form, which runs the same code."""
     import torch
     from deepgrp_b200 import _lib, sharding
     s, w, codes = make_case(dg, name)
@@ -511,8 +512,18 @@ def test_finish_record_of_gathered_ranges_equals_oracle(dg, oracle, name):
     lab, sc = R.gathered(parts8 := [a for a, _ in split_positions(L, 8)] + [L])
     assert len(parts8) == 9
     d_lab, d_sc = torch.from_numpy(lab).cuda(), torch.from_numpy(sc).cuda()
-    for use_mss, mn, xd in ((1, 50, 50), (1, 1, 0), (1, 20, 5), (0, 50, 50)):
-        exp = oracle.find_mss_relabel(sc.astype(np.float64), lab, 5, mn, xd) if use_mss else lab
+    # without MSS the finish is refused: the whole record's softmax decides those labels (tests/test_gpu_options.py)
+    with pytest.raises(ValueError, match="use_mss"):
+        sharding.finish_record(lab, sc, 5, False, 50, 50, 0)
+    n_rows = ctypes.c_int64(0)
+    for fn, args in ((_lib.lib().dgrp_finish_record, (_lib.ptr(lab), _lib.ptr(sc), L, 5, 0, 50, 50, 0,
+                                                      _lib.ptr(np.zeros(L, np.uint8)), None, 0)),
+                     (_lib.lib().dgrp_finish_record_dev, (ctypes.c_void_p(d_lab.data_ptr()),
+                                                          ctypes.c_void_p(d_sc.data_ptr()), L, 5, 0, 50, 50))):
+        assert fn(dg.ctx.handle, *args, ctypes.byref(n_rows)) == _lib.E_UNSUPPORTED
+        assert "use_mss" in _lib.last_error()
+    for use_mss, mn, xd in ((1, 50, 50), (1, 1, 0), (1, 20, 5)):
+        exp = oracle.find_mss_relabel(sc.astype(np.float64), lab, 5, mn, xd)
         for startpos in (0, 17):
             out, rows = sharding.finish_record(lab, sc, 5, bool(use_mss), mn, xd, startpos)
             assert np.array_equal(out, exp), (use_mss, mn, xd)
