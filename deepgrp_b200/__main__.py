@@ -3,7 +3,8 @@
 (reference ``deepgrp/__main__.py``).  Same options (``-b -s -x -l -t --xla -v``, ``predict
 --output --no_use_mss``); ``-t`` and ``--xla`` are accepted and ignored (there is no TensorFlow).
 The README form ``deepgrp <modelfile> <fastafile>...`` (reference ``README.rst:92-98``) is accepted
-as well as the ``predict`` sub-command.  ``train`` trains a GRU model on the GPU (``deepgrp_b200.training``).
+as well as the ``predict`` sub-command.  ``train`` trains a GRU model on the GPU (``deepgrp_b200.training``);
+``evaluate`` scores a model's predictions against a repeat annotation.
 """
 from __future__ import annotations
 
@@ -126,7 +127,9 @@ class CommandLineParser:
         sub = {name: commands.add_parser(name=name, description=text,
                                          formatter_class=argparse.ArgumentDefaultsHelpFormatter)
                for name, text in (("predict", "predict using a deepgrp model"),
-                                  ("train", "Train a deepgrp model"))}
+                                  ("train", "Train a deepgrp model"),
+                                  ("evaluate", "score the predictions of a deepgrp model against a repeat "
+                                               "annotation (per-base confusion matrices and metrics, JSON)"))}
         sub["predict"].add_argument("model", type=str, help="Keras model in HDF5 format (or .npz weights)")
         sub["predict"].add_argument("FASTA", nargs="+", type=str, help="Fasta input files")
         sub["predict"].add_argument("--output", type=str, default="-", help="Output filename")
@@ -145,6 +148,16 @@ class CommandLineParser:
                            ("validfile", "one-hot .npz of the validation chromosome"),
                            ("bedfile", "repeat annotations: chromosome, begin, end, repeat number")):
             sub["train"].add_argument(name, type=str, help=text)
+        sub["evaluate"].add_argument("model", type=str, help="Keras model in HDF5 format (or .npz weights)")
+        sub["evaluate"].add_argument("annotation", type=str,
+                                     help="repeat annotations: chromosome, begin, end, repeat number (0-based, "
+                                          "half-open, whitespace-separated, further columns ignored)")
+        sub["evaluate"].add_argument("FASTA", nargs="+", type=str, help="Fasta input files")
+        sub["evaluate"].add_argument("--output", type=str, default="-", help="Output filename (JSON)")
+        sub["evaluate"].add_argument("--no_use_mss", "-m", action="store_true",
+                                     help="Disable maximum scoring segment algorithm")
+        sub["evaluate"].add_argument("--repeats", type=int, nargs="+", default=None, metavar="N",
+                                     help="repeat numbers to score (default: 1 .. classes-1 of the model)")
         sub["train"].add_argument("--logdir", type=str, default=".", help="Directory for best.hdf5 and history.tsv")
         sub["train"].add_argument("--modelfile", type=str, default="model.hdf5", help="Keras HDF5 file to write")
 
@@ -152,7 +165,8 @@ class CommandLineParser:
         """Parse command line arguments."""
         argv = list(sys.argv[1:] if argv is None else argv)
         # README form: `deepgrp [options] <modelfile> <fasta...>` without the sub-command
-        if not any(a in ("predict", "train") for a in argv) and not any(a in ("-h", "--help") for a in argv):
+        commands = ("predict", "train", "evaluate")
+        if not any(a in commands for a in argv) and not any(a in ("-h", "--help") for a in argv):
             with_value = {"-b", "--batch_size", "-s", "--step_size", "-x", "--xdrop_length", "-l",
                           "--min_mss_length", "-t", "--threads"}
             i = 0
@@ -253,6 +267,39 @@ class CommandLineParser:
                     options.batch_size, use_mss, options.min_mss_len, options.xdrop_len)
                 _LOG.info("%s: %d records, %d bases, %d rows", filename, stats["records"], stats["bases"],
                           stats["rows"])
+
+    def evaluate(self, args: argparse.Namespace, options: dgmodel.Options):
+        """Predict every FASTA file as ``predict`` does with the same options and score the rows against the annotation:
+        one JSON document with each kept record's confusion matrix and metrics (rows: true class) and their total.
+        Nothing is written when a file fails."""
+        import json
+        from . import preprocessing as dgprep
+        model = dgmodel.load_model(args.model)
+        C = model.n_classes
+        try:
+            repeats = dgpred.searched_repeats(args.repeats, C)
+        except ValueError as err:
+            self.parser.error("evaluate: --repeats: %s" % err)
+        annotation = dgprep.read_annotation(args.annotation, repeats)
+        use_mss = not args.no_use_mss
+        records, total = [], np.zeros((C, C), np.int64)
+        for filename in args.FASTA:
+            result = dgpred.evaluate_fasta(model, _read_raw(filename), annotation, args.step_size,
+                                           options.batch_size, use_mss, options.min_mss_len, options.xdrop_len, repeats)
+            records += [{"file": filename, **rec} for rec in result["records"]]
+            total += result["total"]["confusion"]
+            _LOG.info("%s: %d records, %d bases, TotalACC %.6f, MCC %.6f", filename, len(result["records"]),
+                      int(result["total"]["confusion"].sum()), result["total"]["metrics"]["TotalACC"],
+                      result["total"]["metrics"]["MCC"])
+        document = {"classes": C, "repeats": repeats, "step_size": args.step_size, "batch_size": options.batch_size,
+                    "use_mss": use_mss, "min_mss_length": options.min_mss_len, "xdrop_length": options.xdrop_len,
+                    "records": records, "total": {"confusion": total, "metrics": dgpred.confusion_metrics(total)}}
+        text = json.dumps(dgpred.jsonable(document), indent=1) + "\n"
+        if args.output == "-":
+            sys.stdout.write(text)
+        else:
+            with open(args.output, "w") as fh:
+                fh.write(text)
 
     @staticmethod
     def train(args: argparse.Namespace, options: dgmodel.Options):

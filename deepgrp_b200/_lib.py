@@ -94,6 +94,7 @@ SIGNATURES = {
                                     ctypes.POINTER(_P), _PL, _PL, _PL]),
     "dgrp_mask_fasta": (_I, [_P, _P, _L, _P, _L, _I, _P]),
     "dgrp_mask_fasta_last": (_I, [_P, _P, _L, _I, _P]),
+    "dgrp_evaluate_last": (_I, [_P, _I, _P, _P, _L, _P]),
     "dgrp_fasta_rows": (_I, [_P, _P, _L]),
     "dgrp_fasta_records": (_I, [_P, _P, _P, _P, _P, _L]),
     "dgrp_fasta_record_tsv": (_I, [_P, _P, _P, _P, _L]),

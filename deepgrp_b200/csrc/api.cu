@@ -16,6 +16,7 @@
 #include <cmath>
 
 #include "dgrp_internal.cuh"
+#include "eval_core.cuh"
 
 namespace dgrp {
 
@@ -277,6 +278,7 @@ int dgrp_ctx_destroy(dgrp_ctx *c) {
   c->pin_small.release(); c->pin_a.release(); c->pin_b.release(); c->tsv_host.release();
   c->tsv_dev.release(); c->tsv_prefix.release();
   c->fa_tri.release(); c->mask_rec.release(); c->mask_bits.release(); c->mask_out.release();
+  c->eval_tab.release(); c->eval_counts.release();
   for (int i = 0; i < 2; ++i) { c->st_raw[i].release(); c->st_text[i].release(); c->st_stage[i].release(); }
   for (int i = 0; i < 4; ++i) c->st_slot[i].release();
   for (auto &e : c->ev) cudaEventDestroy(e);
@@ -332,6 +334,7 @@ int dgrp_ctx_get_int(dgrp_ctx *c, const char *key, int64_t *value) {
   else if (!strcmp(key, "forward_slab_mb")) *value = c->forward_slab_bytes >> 20;
   else if (!strcmp(key, "forward_used_tc")) *value = c->forward_used_tc;
   else if (!strcmp(key, "sm_count")) *value = c->sm_count;
+  else if (!strcmp(key, "eval_kernel_ns")) *value = c->eval_kernel_ns;
   else { set_error("unknown option %s", key); return DGRP_E_ARG; }
   return DGRP_OK;
 }
@@ -971,6 +974,7 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
     c->fa_row_off.push_back(dev_rows);
     c->mask_nbytes = nbytes;
     c->mask_raw_reserves = c->raw.reserves;
+    c->fa_classes = m->C;
   }
   return rc;
 }
@@ -1071,13 +1075,20 @@ int dgrp_mask_fasta(dgrp_ctx *c, const uint8_t *fasta, int64_t nbytes, const dgr
   return mask_finish(c, nbytes, f, d_tri, d_rec, n_rec, mode, out);
 }
 
+// The record table and device rows of the last dgrp_predict_fasta[_tsv] are still there: that call succeeded
+// unsharded, and no call has reserved c->raw since (every call that overwrites them reserves it first).
+static int require_last_fasta(dgrp_ctx *c, const char *what) {
+  DGRP_REQUIRE(c->mask_nbytes >= 0 && c->mask_raw_reserves == c->raw.reserves,
+               "no dgrp_predict_fasta result to %s: none ran, it failed or was sharded, or another call has used "
+               "its buffers since", what);
+  return DGRP_OK;
+}
+
 int dgrp_mask_fasta_last(dgrp_ctx *c, const uint8_t *fasta, int64_t nbytes, int mode, uint8_t *out) {
   Use use(c->device);
   (void)fasta;   // its copy on the device (c->raw) is masked
   DGRP_REQUIRE(mode == DGRP_MASK_SOFT || mode == DGRP_MASK_HARD, "mask mode must be DGRP_MASK_SOFT or DGRP_MASK_HARD");
-  DGRP_REQUIRE(c->mask_nbytes >= 0 && c->mask_raw_reserves == c->raw.reserves,
-               "no dgrp_predict_fasta result to mask: none ran, it failed or was sharded, or another call has used "
-               "its buffers since");
+  DGRP_CHECK(require_last_fasta(c, "mask"));
   DGRP_REQUIRE(nbytes == c->mask_nbytes, "the last dgrp_predict_fasta had %lld bytes, not %lld",
                (long long)c->mask_nbytes, (long long)nbytes);
   if (nbytes == 0) return DGRP_OK;
@@ -1086,6 +1097,46 @@ int dgrp_mask_fasta_last(dgrp_ctx *c, const uint8_t *fasta, int64_t nbytes, int 
   const int64_t *d_rec = nullptr, *d_tri = nullptr;
   DGRP_CHECK(mask_upload(c, c->fa_seq_base, c->fa_row_off, f.n_seq, {}, &d_rec, &d_tri));
   return mask_finish(c, nbytes, f, c->fa_tri.as<int64_t>(), d_rec, (int64_t)c->fa_seq_base.size(), mode, out);
+}
+
+/* ------------------------------------- evaluation -------------------------------------- */
+
+int dgrp_evaluate_last(dgrp_ctx *c, int n_classes, const int64_t *ann, const int64_t *ann_off, int64_t n_records,
+                       int64_t *counts) {
+  Use use(c->device);
+  DGRP_REQUIRE(ann != nullptr && ann_off != nullptr && counts != nullptr, "ann, ann_off and counts must not be NULL");
+  DGRP_CHECK(require_last_fasta(c, "evaluate"));
+  const int64_t n_rec = (int64_t)c->fa_startpos.size();
+  DGRP_REQUIRE(n_records == n_rec, "the last dgrp_predict_fasta kept %lld records, not %lld", (long long)n_rec,
+               (long long)n_records);
+  const int C = n_classes;
+  DGRP_REQUIRE(C == c->fa_classes, "the last dgrp_predict_fasta ran a model of %d classes, not %d", c->fa_classes, C);
+  DGRP_REQUIRE(ann_off[0] >= 0, "ann_off[0] is negative");
+  for (int64_t r = 0; r < n_rec; ++r)
+    DGRP_REQUIRE(ann_off[r] <= ann_off[r + 1], "ann_off decreases at record %lld", (long long)r);
+  for (int64_t i = ann_off[0]; i < ann_off[n_rec]; ++i) {
+    DGRP_REQUIRE(ann[3 * i] >= 0 && ann[3 * i + 1] >= 0, "annotation %lld: negative coordinate [%lld, %lld)",
+                 (long long)i, (long long)ann[3 * i], (long long)ann[3 * i + 1]);
+    DGRP_REQUIRE(ann[3 * i + 2] >= 1 && ann[3 * i + 2] < C, "annotation %lld: class %lld is not in [1, %d)",
+                 (long long)i, (long long)ann[3 * i + 2], C);
+  }
+  eval::Table t;
+  eval::build_table(C, ann, ann_off, n_rec, c->fa_startpos.data(), c->fa_length.data(), c->fa_row_off.data(), t);
+  DGRP_CHECK(c->eval_tab.reserve(t.h.size() * 8));
+  DGRP_CHECK(c->eval_counts.reserve((size_t)(n_rec > 0 ? n_rec : 1) * C * C * 8));
+  DGRP_CUDA(cudaMemcpyAsync(c->eval_tab.p, t.h.data(), t.h.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  DGRP_CUDA(cudaMemsetAsync(c->eval_counts.p, 0, (size_t)n_rec * C * C * 8, c->stream));
+  DGRP_CUDA(cudaEventRecord(c->ev[6], c->stream));
+  DGRP_CHECK(run_eval_confusion(c, C, t, c->eval_tab.as<int64_t>(), c->fa_tri.as<int64_t>(),
+                                c->eval_counts.as<int64_t>()));
+  DGRP_CUDA(cudaEventRecord(c->ev[7], c->stream));
+  if (n_rec > 0)
+    DGRP_CUDA(cudaMemcpyAsync(counts, c->eval_counts.p, (size_t)n_rec * C * C * 8, cudaMemcpyDeviceToHost, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  float ms = 0.f;
+  DGRP_CUDA(cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]));
+  c->eval_kernel_ns = (int64_t)(ms * 1e6f);
+  return DGRP_OK;
 }
 
 int dgrp_fasta_rows(dgrp_ctx *c, dgrp_row_t *rows, int64_t cap) {

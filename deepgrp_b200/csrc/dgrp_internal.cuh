@@ -134,13 +134,17 @@ struct dgrp_ctx {
   // buffer has been reserved since)
   int64_t codes_dev_length = -1, codes_dev_rows = 0;
   uint64_t codes_dev_reserves[2] = {};
-  // the last dgrp_predict_fasta[_tsv] for dgrp_mask_fasta_last: every kept record's first sequence rank and first
-  // row (one more row entry: the total), its rows on the device as (start, end, label) triples, its byte count
-  // (-1: it failed, was sharded, or none ran) and the reserve count of c->raw (its text) when it returned
+  // the last dgrp_predict_fasta[_tsv] for dgrp_mask_fasta_last and dgrp_evaluate_last: every kept record's first
+  // sequence rank and first row (one more row entry: the total), its rows on the device as (start, end, label)
+  // triples, its byte count (-1: it failed, was sharded, or none ran) and the reserve count of c->raw (its text)
+  // when it returned
   std::vector<int64_t> fa_seq_base, fa_row_off;
   dgrp::DevBuf fa_tri;
   int64_t mask_nbytes = -1;
   uint64_t mask_raw_reserves = 0;
+  int fa_classes = 0;                  // the model classes of that call (dgrp_evaluate_last)
+  dgrp::DevBuf eval_tab, eval_counts;  // dgrp_evaluate_last: record / run table, per-record counts
+  int64_t eval_kernel_ns = 0;          // device time of the last evaluation kernel (CUDA events)
   dgrp::DevBuf mask_rec, mask_bits, mask_out;   // dgrp_mask_fasta*: record table, rank bitmap, masked text
   int shard_rank = 0, shard_world = 1;   // contig sharding of dgrp_predict_fasta* (dgrp_ctx_set_int)
   dgrp::PinBuf tsv_host;     // finished TSV text of the last dgrp_predict_fasta_tsv
@@ -281,6 +285,11 @@ int run_tsv_write(dgrp_ctx *c, const int64_t *d_tri, int64_t n, const uint8_t *d
 int launch_filter_segments(dgrp_ctx *c, const uint8_t *d_in, uint8_t *d_out, int64_t n, int64_t min_len);
 int launch_confusion(dgrp_ctx *c, const uint8_t *d_truth, const uint8_t *d_pred, int64_t n,
                      unsigned long long *d_cnf, int *d_bad);
+namespace eval { struct Table; }
+// K10: adds the confusion counts of every record of the table t (uploaded to d_tab) against the rows d_tri of
+// dgrp_predict_fasta to d_counts[r][t][p] (int64, zeroed by the caller); one launch
+int run_eval_confusion(dgrp_ctx *c, int C, const eval::Table &t, const int64_t *d_tab, const int64_t *d_tri,
+                       int64_t *d_counts);
 // segments.cu
 // open_tail != nullptr: the labels are a prefix of a record whose continuation is not known yet.  The
 // reference's special case of the record's last element does not apply, and a run that reaches the end of

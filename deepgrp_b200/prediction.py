@@ -222,6 +222,17 @@ def predict_fasta(model: ModelWeights, raw: bytes, step_size: int, batch_size: i
     pipeline.  ``rows``: structured array (start, end, label, record); ``records``: list of
     ``(header, startpos, length)``.  A blank line raises ``IndexError`` and an all-'N' record
     ``ValueError``, as the reference does."""
+    n_rows, records = _predict_fasta_call(model, raw, step_size, batch_size, use_mss, min_mss_len, xdrop_len,
+                                          compat)
+    rows = np.zeros(n_rows, dtype=_lib.ROW_DTYPE)
+    if n_rows:
+        _lib.check(_lib.lib().dgrp_fasta_rows(_lib.context().handle, _lib.ptr(rows), n_rows))
+    return rows, records
+
+
+def _predict_fasta_call(model: ModelWeights, raw, step_size: int, batch_size: int, use_mss: bool,
+                        min_mss_len: int, xdrop_len: int, compat: str):
+    """``dgrp_predict_fasta`` -> (number of rows, records); the rows stay in the context."""
     ctx = _lib.context()
     n = len(raw)
     buf = np.frombuffer(raw, dtype=np.uint8) if n else np.zeros(0, np.uint8)
@@ -235,9 +246,6 @@ def predict_fasta(model: ModelWeights, raw: bytes, step_size: int, batch_size: i
     if rc == _lib.E_ALLN:
         raise ValueError("negative dimensions are not allowed")
     _lib.check(rc)
-    rows = np.zeros(n_rows.value, dtype=_lib.ROW_DTYPE)
-    if n_rows.value:
-        _lib.check(_lib.lib().dgrp_fasta_rows(ctx.handle, _lib.ptr(rows), n_rows.value))
     k = n_rec.value
     off, ln = np.zeros(k, np.int64), np.zeros(k, np.int64)
     sp, le = np.zeros(k, np.int64), np.zeros(k, np.int64)
@@ -246,7 +254,7 @@ def predict_fasta(model: ModelWeights, raw: bytes, step_size: int, batch_size: i
                                                  _lib.ptr(sp), _lib.ptr(le), k))
     records = [(bytes(raw[off[i]:off[i] + ln[i]]).decode("utf-8", "replace"), int(sp[i]), int(le[i]))
                for i in range(k)]
-    return rows, records
+    return int(n_rows.value), records
 
 
 def _fasta_tsv_call(model: ModelWeights, raw, filename: str, step_size: int, batch_size: int,
@@ -512,6 +520,86 @@ def _calculate_metrics(cnf_matrix: np.ndarray) -> dict:
     metrics["F1"] = 2 * metrics["TPR"] * metrics["PPV"] / (metrics["TPR"] + metrics["PPV"])
     metrics["MCC"] = calculate_multiclass_matthews_cc(cnf_matrix)
     return metrics
+
+
+def confusion_metrics(cnf_matrix: np.ndarray) -> dict:
+    """The metrics :func:`calculate_metrics` reports for a confusion matrix (``_calculate_metrics`` + ``TotalACC``);
+    a 0/0 rate is NaN, as numpy computes it, without a warning."""
+    cnf_matrix = np.asarray(cnf_matrix)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        metrics = _calculate_metrics(cnf_matrix)
+        metrics["TotalACC"] = np.trace(cnf_matrix) / cnf_matrix.sum()
+    return metrics
+
+
+def jsonable(value):
+    """``value`` with numpy arrays and scalars as JSON types; NaN becomes ``None`` (JSON ``null``)."""
+    if isinstance(value, dict):
+        return {k: jsonable(v) for k, v in value.items()}
+    if isinstance(value, (list, tuple, np.ndarray)):
+        return [jsonable(v) for v in value]
+    if isinstance(value, (bool, np.bool_)):
+        return bool(value)
+    if isinstance(value, (int, np.integer)):
+        return int(value)
+    if isinstance(value, (float, np.floating)):
+        return None if np.isnan(value) else float(value)
+    return value
+
+
+def searched_repeats(repeats, n_classes: int) -> list:
+    """The repeat numbers evaluation searches for, sorted and without duplicates: ``repeats``, or ``1 .. C-1`` when it
+    is None.  ``ValueError`` for a number outside ``[1, n_classes)``."""
+    out = list(range(1, n_classes)) if repeats is None else sorted({int(r) for r in repeats})
+    bad = [r for r in out if not 1 <= r < n_classes]
+    if bad or not out:
+        raise ValueError("repeat numbers must lie in [1, %d) for a %d-class model, got %s"
+                         % (n_classes, n_classes, bad or "none"))
+    return out
+
+
+def evaluate_fasta(model: ModelWeights, raw, annotation: dict, step_size: int, batch_size: int, use_mss: bool,
+                   min_mss_len: int, xdrop_len: int, repeats=None, compat: str = "reference") -> dict:
+    """Score the prediction of one FASTA file (the rows ``deepgrp predict`` writes with these options) against a repeat
+    annotation, on the GPU.  ``annotation``: :func:`deepgrp_b200.preprocessing.read_annotation`'s
+    ``{chromosome: int64[n, 3]}``; a record's chromosome is the first word of its header.  A record's evaluated span is
+    ``[startpos, startpos + length)``; a position's true class is the lowest searched repeat number among the
+    annotations that cover it (``preprocess_y(...).argmax(0)``), 0 where none does; its predicted class is the label of
+    the row that covers it, 0 where none does.  The file runs slice by slice (whole records, >= 8 MiB), which bounds
+    device memory; no per-base array is built.  Returns ``{classes, repeats, records: [{header, chromosome, startpos,
+    length, confusion, metrics}], total: {confusion, metrics}}`` with ``C x C`` int64 matrices (rows: true class).
+    A blank line raises ``IndexError`` and an all-``N`` record ``ValueError``, as in ``predict``."""
+    from .sharding import fasta_slices
+    C = model.n_classes
+    repeats = searched_repeats(repeats, C)
+    wanted = np.asarray(repeats, dtype=np.int64)
+    ctx = _lib.context()
+    cuts, _ = fasta_slices(raw, 1)
+    whole = memoryview(raw) if len(raw) else memoryview(b"")
+    records = []
+    none = np.zeros((0, 3), np.int64)
+    for k in range(len(cuts) - 1):
+        piece = whole[int(cuts[k]):int(cuts[k + 1])]
+        _, recs = _predict_fasta_call(model, piece, step_size, batch_size, use_mss, min_mss_len, xdrop_len, compat)
+        chroms = [header.split()[0] for header, _, _ in recs]
+        lists = []
+        for chrom in chroms:
+            a = np.asarray(annotation.get(chrom, none), dtype=np.int64).reshape(-1, 3)
+            lists.append(a[np.isin(a[:, 2], wanted)])
+        ann = np.ascontiguousarray(np.concatenate(lists) if lists else none)
+        ann_off = np.zeros(len(recs) + 1, np.int64)
+        ann_off[1:] = np.cumsum([len(a) for a in lists])
+        counts = np.zeros((max(len(recs), 1), C, C), np.int64)
+        _lib.check(_lib.lib().dgrp_evaluate_last(ctx.handle, C, _lib.ptr(ann), _lib.ptr(ann_off), len(recs),
+                                                 _lib.ptr(counts)))
+        for (header, startpos, length), chrom, cnf in zip(recs, chroms, counts):
+            records.append({"header": header, "chromosome": chrom, "startpos": startpos, "length": length,
+                            "confusion": cnf, "metrics": confusion_metrics(cnf)})
+    total = np.zeros((C, C), np.int64)
+    for rec in records:
+        total += rec["confusion"]
+    return {"classes": C, "repeats": repeats, "records": records,
+            "total": {"confusion": total, "metrics": confusion_metrics(total)}}
 
 
 def _labels_u8(name: str, a) -> np.ndarray:

@@ -11,7 +11,7 @@ import gzip
 import hashlib
 import os
 import sys
-from typing import BinaryIO, List, NamedTuple, Tuple
+from typing import BinaryIO, Dict, List, NamedTuple, Tuple
 
 import numpy as np
 
@@ -19,17 +19,49 @@ import numpy as np
 Data = NamedTuple("Data", [("fwd", np.ndarray), ("truelbl", np.ndarray)])
 
 
-def preprocess_y(filename, chromosom: str, length: int, repeats_to_search: List[int]) -> np.ndarray:
-    """Reference ``deepgrp/preprocessing.py:9-46``: the whitespace-separated table ``parse_rm`` writes
-    (chromosome, begin, end, repeat number, ...) -> one-hot annotations int8[len(repeats) + 1, length];
-    row ``r`` is set on [begin, end) of every line of ``chromosom`` whose repeat number ``r`` is searched
-    for (the number itself is the row index, as in the reference), row 0 wherever no other row is."""
+def read_annotation(filename, repeats_to_search: List[int]) -> Dict[str, np.ndarray]:
+    """The whitespace-separated table ``parse_rm`` writes (chromosome, begin, end, repeat number; further columns are
+    ignored, no header) -> ``{chromosome: int64[n, 3]}`` of (begin, end, number), in file order, for the lines whose
+    repeat number is searched for.  Coordinates are 0-based and half-open as ``preprocess_y`` indexes them.  A
+    non-integer begin, end or number, or a negative coordinate, on any line is a ``ValueError``."""
     import pandas as pd
-    table = pd.read_csv(filename, sep=r"\s+", header=None, index_col=False, usecols=[0, 1, 2, 3],
-                        names=["chromosom", "begin", "end", "repeatnumber"])
-    table = table[(table.chromosom == chromosom) & table.repeatnumber.isin(list(repeats_to_search))]
+    try:
+        table = pd.read_csv(filename, sep=r"\s+", header=None, index_col=False, usecols=[0, 1, 2, 3],
+                            names=["chromosom", "begin", "end", "repeatnumber"], dtype=str)
+    except pd.errors.EmptyDataError:
+        return {}
+    cols = ("begin", "end", "repeatnumber")
+    for col in cols:
+        ok = table[col].str.fullmatch(r"[+-]?[0-9]+").fillna(False).to_numpy(bool)
+        if not ok.all():
+            line = int(np.argmin(ok))
+            raise ValueError("annotation row %d: %s %r is not an integer" % (line + 1, col, table[col].iloc[line]))
+    values = table[list(cols)].to_numpy().astype(np.int64)
+    negative = (values[:, :2] < 0).any(axis=1)
+    if negative.any():
+        line = int(np.argmax(negative))
+        raise ValueError("annotation row %d: negative coordinate %d %d" % (line + 1, values[line, 0], values[line, 1]))
+    keep = np.isin(values[:, 2], np.asarray(list(repeats_to_search), dtype=np.int64))
+    chrom = table["chromosom"].to_numpy()[keep]
+    values = values[keep]
+    out = {}
+    if len(chrom):
+        names, first, inverse = np.unique(chrom, return_index=True, return_inverse=True)
+        order = np.argsort(inverse, kind="stable")
+        bounds = np.searchsorted(inverse[order], np.arange(len(names) + 1))
+        for k in np.argsort(first):
+            out[str(names[k])] = np.ascontiguousarray(values[order[bounds[k]:bounds[k + 1]]])
+    return out
+
+
+def preprocess_y(filename, chromosom: str, length: int, repeats_to_search: List[int]) -> np.ndarray:
+    """Reference ``deepgrp/preprocessing.py:9-46``: the annotation table (:func:`read_annotation`) -> one-hot
+    annotations int8[len(repeats) + 1, length]; row ``r`` is set on [begin, end) of every line of ``chromosom`` whose
+    repeat number ``r`` is searched for (the number itself is the row index, as in the reference), row 0 wherever no
+    other row is."""
+    lines = read_annotation(filename, repeats_to_search).get(chromosom, np.zeros((0, 3), np.int64))
     yarray = np.zeros((len(repeats_to_search) + 1, length), dtype=np.int8)
-    for begin, end, number in zip(table.begin.to_numpy(), table.end.to_numpy(), table.repeatnumber.to_numpy()):
+    for begin, end, number in lines:
         yarray[number, begin:end] = 1
     yarray[0, ~yarray[1:].any(axis=0)] = 1
     return yarray

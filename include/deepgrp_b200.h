@@ -86,7 +86,8 @@ int64_t dgrp_ctx_launch_count(dgrp_ctx *ctx);
  * window-probability buffer), "forward_fuse_score" (fuse vote + score transform for whole-record calls),
  * "stream_slot_mb" (host piece size of dgrp_fasta_stream), "stream_early_rows" / "stream_early_slabs" /
  * "stream_early_ratio" / "stream_early_unit" (position slabs of a long record in dgrp_fasta_stream; get-only
- * "stream_early_parts": parts of the last record's text that left before its last slab). */
+ * "stream_early_parts": parts of the last record's text that left before its last slab); get-only "eval_kernel_ns"
+ * (device time of the last dgrp_evaluate_last kernel, nanoseconds). */
 int dgrp_ctx_set_int(dgrp_ctx *ctx, const char *key, int64_t value);
 int dgrp_ctx_get_int(dgrp_ctx *ctx, const char *key, int64_t *value);
 
@@ -245,6 +246,20 @@ int dgrp_mask_fasta(dgrp_ctx *ctx, const uint8_t *fasta, int64_t nbytes, const d
  * failed or was sharded (shard_world > 1), when nbytes differs from its, or when another call has overwritten
  * its text on the device since. */
 int dgrp_mask_fasta_last(dgrp_ctx *ctx, const uint8_t *fasta, int64_t nbytes, int mode, uint8_t *out);
+/* Evaluation against a repeat annotation (the per-base multi-class confusion matrix that deepgrp/optimization.py:58-69
+ * scores models with): counts[r][t][p] (int64[n_records][C][C], host) = positions of kept record r's span
+ * [startpos, startpos + length) (dgrp_fasta_records) whose true class is t and whose predicted class is p, for the rows
+ * the last dgrp_predict_fasta[_tsv] left on the device.  The predicted class of a position is the label of the row
+ * that covers it, 0 where none does.  ann holds (begin, end, class) triples, 0-based half-open in untrimmed record
+ * coordinates, record r's at [ann_off[r], ann_off[r + 1]) in any order, overlapping or not; they are clipped to the
+ * span, and begin >= end contributes nothing.  The true class of a position is the lowest class among the triples that
+ * cover it, 0 where none does (preprocess_y(...).argmax(axis=0), deepgrp/preprocessing.py:9-46).  No per-base array is
+ * built: the rows and the sorted, merged runs of every (record, class) are compared as interval lists.  DGRP_E_ARG
+ * when there is no such prediction (as in dgrp_mask_fasta_last), when n_records or n_classes differ from that call's
+ * kept records and model classes, for a class outside [1, n_classes), a negative coordinate, a decreasing ann_off, or
+ * a NULL pointer.  The device time of the kernel is read with dgrp_ctx_get_int(ctx, "eval_kernel_ns", ...). */
+int dgrp_evaluate_last(dgrp_ctx *ctx, int n_classes, const int64_t *ann, const int64_t *ann_off, int64_t n_records,
+                       int64_t *counts);
 /* rows[i].record indexes the record table */
 int dgrp_fasta_rows(dgrp_ctx *ctx, dgrp_row_t *rows, int64_t cap);
 /* per record: header text = fasta[hdr_off, hdr_off + hdr_len); startpos = leading 'N' count;
