@@ -143,6 +143,11 @@ class CommandLineParser:
                                          "('-' = stdout, when --output is a file); every input file in order")
         sub["predict"].add_argument("--mask_mode", choices=("soft", "hard"), default="soft",
                                     help="soft: lower-case the masked bases; hard: replace them by N")
+        sub["predict"].add_argument("--track", type=str, default=None, metavar="PREFIX",
+                                    help="Also write the binned max-vote probability of every repeat class c to "
+                                         "PREFIX.<c>.bedGraph; every input file in order")
+        sub["predict"].add_argument("--track_bin", type=int, default=10, metavar="N",
+                                    help="Bases per bin of --track (1 .. %d)" % dgpred.TRACK_BIN_MAX)
         for name, text in (("parameter", "TOML file of hyper-parameters (Options)"),
                            ("trainfile", "one-hot .npz of the training chromosome (preprocess_sequence)"),
                            ("validfile", "one-hot .npz of the validation chromosome"),
@@ -184,6 +189,13 @@ class CommandLineParser:
                 self.parser.error("--mask is not available with --stepwise")
             if args.mask == "-" and args.output == "-":
                 self.parser.error("--mask - needs --output to name a file")
+        if getattr(args, "track", None) is not None:
+            if args.stepwise:
+                self.parser.error("--track is not available with --stepwise")
+            if args.track == "-":
+                self.parser.error("--track names files (PREFIX.<class>.bedGraph), not '-'")
+        if args.command == "predict" and not 1 <= args.track_bin <= dgpred.TRACK_BIN_MAX:
+            self.parser.error("--track_bin must lie in [1, %d], not %d" % (dgpred.TRACK_BIN_MAX, args.track_bin))
         self.threads = args.threads
         self.verbose = args.verbose
         self.xla = args.xla
@@ -219,18 +231,25 @@ class CommandLineParser:
         use_mss = not args.no_use_mss
         mask = getattr(args, "mask", None)
         maskstream = None
-        if mask is not None:
-            maskstream = _ByteSink(sys.stdout) if mask == "-" else open(mask, "wb")
+        trackstreams = {}
         try:
-            CommandLineParser._predict_files(args, options, model, outstream, use_mss, maskstream)
+            if mask is not None:
+                maskstream = _ByteSink(sys.stdout) if mask == "-" else open(mask, "wb")
+            track = getattr(args, "track", None)
+            if track is not None:
+                for c in range(1, model.n_classes):
+                    trackstreams[c] = open("%s.%d.bedGraph" % (track, c), "wb")
+            CommandLineParser._predict_files(args, options, model, outstream, use_mss, maskstream, trackstreams)
         finally:
             if maskstream is not None and mask != "-":
                 maskstream.close()
+            for stream in trackstreams.values():
+                stream.close()
         if args.output != "-":
             outstream.close()
 
     @staticmethod
-    def _predict_files(args, options, model, outstream, use_mss, maskstream):
+    def _predict_files(args, options, model, outstream, use_mss, maskstream, trackstreams=None):
         for filename in args.FASTA:
             _LOG.info("Processing %s", filename)
             if getattr(args, "stepwise", False):
@@ -252,13 +271,15 @@ class CommandLineParser:
                 finally:
                     if filename != "-":
                         filestream.close()
-            elif maskstream is not None:
-                # slice by slice: each slice's rows, then its masked text
-                stats = dgpred.predict_fasta_tsv_masked(
-                    model, _read_raw(filename), filename, _ByteSink(outstream), maskstream, args.step_size,
-                    options.batch_size, use_mss, options.min_mss_len, options.xdrop_len, args.mask_mode)
-                _LOG.info("%s: %d records, %d bases, %d rows, masked", filename, stats["records"], stats["bases"],
-                          stats["rows"])
+            elif maskstream is not None or trackstreams:
+                # slice by slice: each slice's rows, then its masked text and its track lines
+                stats = dgpred.predict_fasta_sliced(
+                    model, _read_raw(filename), filename, _ByteSink(outstream), args.step_size, options.batch_size,
+                    use_mss, options.min_mss_len, options.xdrop_len, maskstream=maskstream,
+                    mask_mode=args.mask_mode, trackstreams=trackstreams, track_bin=args.track_bin)
+                _LOG.info("%s: %d records, %d bases, %d rows%s%s", filename, stats["records"], stats["bases"],
+                          stats["rows"], ", masked" if maskstream is not None else "",
+                          ", tracks" if trackstreams else "")
             else:
                 # records stream through the GPU pipeline; a record's rows are written as soon as it is done,
                 # so an error in a later record leaves the earlier rows in the output, as in the reference

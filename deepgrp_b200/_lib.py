@@ -95,6 +95,7 @@ SIGNATURES = {
     "dgrp_mask_fasta": (_I, [_P, _P, _L, _P, _L, _I, _P]),
     "dgrp_mask_fasta_last": (_I, [_P, _P, _L, _I, _P]),
     "dgrp_evaluate_last": (_I, [_P, _I, _P, _P, _L, _P]),
+    "dgrp_track_last": (_I, [_P, _I, _I, ctypes.POINTER(_P), _PL]),
     "dgrp_fasta_rows": (_I, [_P, _P, _L]),
     "dgrp_fasta_records": (_I, [_P, _P, _P, _P, _P, _L]),
     "dgrp_fasta_record_tsv": (_I, [_P, _P, _P, _P, _L]),

@@ -17,6 +17,7 @@
 
 #include "dgrp_internal.cuh"
 #include "eval_core.cuh"
+#include "track_core.cuh"
 
 namespace dgrp {
 
@@ -261,6 +262,7 @@ int dgrp_ctx_create(int device, dgrp_ctx **out) {
     return DGRP_E_CUDA;
   }
   for (auto &e : c->ev) cudaEventCreate(&e);
+  for (auto &e : c->tev) cudaEventCreate(&e);
   for (int i = 0; i < 6; ++i) cudaEventRecord(c->ev[i], c->stream);
   *out = c;
   return DGRP_OK;
@@ -279,9 +281,12 @@ int dgrp_ctx_destroy(dgrp_ctx *c) {
   c->tsv_dev.release(); c->tsv_prefix.release();
   c->fa_tri.release(); c->mask_rec.release(); c->mask_bits.release(); c->mask_out.release();
   c->eval_tab.release(); c->eval_counts.release();
+  c->fa_pred.release(); c->track_tab.release(); c->track_work.release(); c->track_text.release();
+  c->track_host.release();
   for (int i = 0; i < 2; ++i) { c->st_raw[i].release(); c->st_text[i].release(); c->st_stage[i].release(); }
   for (int i = 0; i < 4; ++i) c->st_slot[i].release();
   for (auto &e : c->ev) cudaEventDestroy(e);
+  for (auto &e : c->tev) cudaEventDestroy(e);
   cudaStreamDestroy(c->stream);
   delete c;
   return DGRP_OK;
@@ -312,6 +317,7 @@ int dgrp_ctx_set_int(dgrp_ctx *c, const char *key, int64_t value) {
   else if (!strcmp(key, "forward_slab_mb")) c->forward_slab_bytes = (int64_t)value << 20;
   else if (!strcmp(key, "shard_rank")) c->shard_rank = (int)value;
   else if (!strcmp(key, "shard_world")) c->shard_world = (int)value;
+  else if (!strcmp(key, "keep_votes")) c->keep_votes = value != 0;
   else { set_error("unknown option %s", key); return DGRP_E_ARG; }
   return DGRP_OK;
 }
@@ -335,6 +341,9 @@ int dgrp_ctx_get_int(dgrp_ctx *c, const char *key, int64_t *value) {
   else if (!strcmp(key, "forward_used_tc")) *value = c->forward_used_tc;
   else if (!strcmp(key, "sm_count")) *value = c->sm_count;
   else if (!strcmp(key, "eval_kernel_ns")) *value = c->eval_kernel_ns;
+  else if (!strcmp(key, "keep_votes")) *value = c->keep_votes;
+  else if (!strcmp(key, "votes_append_ns")) *value = c->votes_append_ns;
+  else if (!strcmp(key, "track_kernel_ns")) *value = c->track_kernel_ns;
   else { set_error("unknown option %s", key); return DGRP_E_ARG; }
   return DGRP_OK;
 }
@@ -785,17 +794,23 @@ int dgrp_predict_sequence(dgrp_ctx *c, dgrp_model *m, const uint8_t *seq, int64_
   return rc;
 }
 
-// buf[used, used + bytes) = d_src[0, bytes) (device to device), growing buf and keeping buf[0, used)
-static int append_dev(dgrp_ctx *c, DevBuf &buf, size_t used, const void *d_src, size_t bytes) {
-  if (used + bytes > buf.cap) {
+// grow buf to hold at least `need` bytes, keeping buf[0, used)
+static int grow_dev(dgrp_ctx *c, DevBuf &buf, size_t used, size_t need) {
+  if (need > buf.cap) {
     DevBuf bigger;
-    DGRP_CHECK(bigger.reserve(std::max(used + bytes, buf.cap * 2)));
+    DGRP_CHECK(bigger.reserve(std::max(need, buf.cap * 2)));
     if (used) DGRP_CUDA(cudaMemcpyAsync(bigger.p, buf.p, used, cudaMemcpyDeviceToDevice, c->stream));
     DGRP_CUDA(cudaStreamSynchronize(c->stream));
     bigger.reserves = buf.reserves;
     buf.release();
     buf = bigger;
   }
+  return DGRP_OK;
+}
+
+// buf[used, used + bytes) = d_src[0, bytes) (device to device), growing buf and keeping buf[0, used)
+static int append_dev(dgrp_ctx *c, DevBuf &buf, size_t used, const void *d_src, size_t bytes) {
+  DGRP_CHECK(grow_dev(c, buf, used, used + bytes));
   ++buf.reserves;
   DGRP_CUDA(cudaMemcpyAsync(static_cast<uint8_t *>(buf.p) + used, d_src, bytes, cudaMemcpyDeviceToDevice, c->stream));
   return DGRP_OK;
@@ -819,6 +834,13 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
   c->fa_seq_base.clear(); c->fa_row_off.clear();
   c->mask_nbytes = -1;
   int64_t dev_rows = 0;             // rows appended to c->fa_tri
+  // keep_votes: every kept record's vote rows are appended to c->fa_pred (dgrp_track_last)
+  const bool keep = c->keep_votes && c->shard_world <= 1;
+  c->fa_votes = false;
+  if (!keep) c->fa_pred.release();   // the votes of an earlier call are not needed any more: free their memory
+  c->fa_pred_off.clear(); c->fa_chrom_off.clear(); c->fa_chrom.clear();
+  c->votes_append_ns = 0;
+  int64_t pred_rows = 0;            // rows appended to c->fa_pred
   DGRP_REQUIRE(nbytes >= 0, "negative length");
   stamp(c, 0);
   DGRP_CHECK(c->raw.reserve((size_t)nbytes + 16));
@@ -891,8 +913,19 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
     c->fa_startpos.push_back(startpos); c->fa_length.push_back(length);
     c->fa_tsv_off.push_back(c->tsv_len); c->fa_tsv_len.push_back(0); c->fa_owner.push_back(owner_of[k]);
     c->fa_seq_base.push_back(hseq[k]); c->fa_row_off.push_back(dev_rows);
+    if (keep) {
+      // the chromosome: the header's first word
+      int64_t w0 = b, w1;
+      while (w0 < e && ws(fasta[w0])) ++w0;
+      for (w1 = w0; w1 < e && !ws(fasta[w1]);) ++w1;
+      c->fa_pred_off.push_back(pred_rows);
+      c->fa_chrom_off.push_back((int64_t)c->fa_chrom.size());
+      c->fa_chrom.append(reinterpret_cast<const char *>(fasta + w0), (size_t)(w1 - w0));
+    }
     stamp(c, 1);
-    if ((rc = core_predict(c, m, c->codes.as<uint8_t>(), length, step, batch_size, compat, use_mss != 0))) break;
+    // with keep_votes the votes are always materialised: the fused vote + score route never writes them
+    if ((rc = core_predict(c, m, c->codes.as<uint8_t>(), length, step, batch_size, compat, use_mss != 0 && !keep)))
+      break;
     windows += c->timings.windows; bases += length;
     stamp(c, 2);
     if ((rc = core_labels_after_predict(c, length, m->C, use_mss, min_mss_len, xdrop_len))) break;
@@ -953,6 +986,17 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
       }
     }
     stamp(c, 5);
+    // the votes are still in c->pred (the label, MSS and segment stages do not write it); appended outside the
+    // stamped stages, so timings.forward_ms stays the forward alone
+    const bool appended = keep && length > 0;
+    if (appended) {
+      const size_t used = (size_t)pred_rows * m->C * 4, bytes = (size_t)length * m->C * 4;
+      if ((rc = grow_dev(c, c->fa_pred, used, used + bytes))) break;   // allocation outside the timed copy
+      cudaEventRecord(c->tev[0], c->stream);
+      if ((rc = append_dev(c, c->fa_pred, used, c->pred.p, bytes))) break;
+      cudaEventRecord(c->tev[1], c->stream);
+      pred_rows += length;
+    }
     cudaStreamSynchronize(c->stream);
     float ms;
     cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]); enc_ms += ms;
@@ -960,6 +1004,8 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
     cudaEventElapsedTime(&ms, c->ev[2], c->ev[3]); score_ms += ms;
     cudaEventElapsedTime(&ms, c->ev[3], c->ev[4]); mss_ms += ms;
     cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]); seg_ms += ms;
+    if (appended && cudaEventElapsedTime(&ms, c->tev[0], c->tev[1]) == cudaSuccess)
+      c->votes_append_ns += (int64_t)(ms * 1e6f);
   }
   cudaEventRecord(e_end, c->stream);
   cudaStreamSynchronize(c->stream);
@@ -975,6 +1021,11 @@ static int predict_fasta_impl(dgrp_ctx *c, dgrp_model *m, const uint8_t *fasta, 
     c->mask_nbytes = nbytes;
     c->mask_raw_reserves = c->raw.reserves;
     c->fa_classes = m->C;
+    if (keep) {
+      c->fa_pred_off.push_back(pred_rows);
+      c->fa_chrom_off.push_back((int64_t)c->fa_chrom.size());
+      c->fa_votes = true;
+    }
   }
   return rc;
 }
@@ -1136,6 +1187,51 @@ int dgrp_evaluate_last(dgrp_ctx *c, int n_classes, const int64_t *ann, const int
   float ms = 0.f;
   DGRP_CUDA(cudaEventElapsedTime(&ms, c->ev[6], c->ev[7]));
   c->eval_kernel_ns = (int64_t)(ms * 1e6f);
+  return DGRP_OK;
+}
+
+/* ------------------------------------ probability tracks ------------------------------------ */
+
+int dgrp_track_last(dgrp_ctx *c, int cls, int bin, const uint8_t **text, int64_t *len) {
+  Use use(c->device);
+  DGRP_REQUIRE(text != nullptr && len != nullptr, "text and len must not be NULL");
+  *text = nullptr; *len = 0;
+  DGRP_CHECK(require_last_fasta(c, "track"));
+  DGRP_REQUIRE(c->fa_votes, "the last dgrp_predict_fasta did not keep its votes (set the keep_votes option first)");
+  DGRP_REQUIRE(cls >= 1 && cls < c->fa_classes, "class %d is not in [1, %d)", cls, c->fa_classes);
+  DGRP_REQUIRE(bin >= 1 && bin <= track::BIN_MAX, "bin size %d is not in [1, %lld]", bin, (long long)track::BIN_MAX);
+  const int64_t n_rec = (int64_t)c->fa_startpos.size();
+  // prefix text: "chrom\t" per record
+  std::vector<int64_t> pfx_off(n_rec + 1, 0);
+  std::string pfx;
+  for (int64_t r = 0; r < n_rec; ++r) {
+    pfx_off[r] = (int64_t)pfx.size();
+    pfx.append(c->fa_chrom, (size_t)c->fa_chrom_off[r], (size_t)(c->fa_chrom_off[r + 1] - c->fa_chrom_off[r]));
+    pfx.push_back('\t');
+  }
+  pfx_off[n_rec] = (int64_t)pfx.size();
+  track::Table t;
+  track::build_table(n_rec, c->fa_startpos.data(), c->fa_length.data(), c->fa_pred_off.data(), pfx_off.data(), bin, t);
+  const size_t tab_bytes = t.h.size() * 8;
+  DGRP_CHECK(c->track_tab.reserve(tab_bytes + pfx.size() + 16));
+  DGRP_CUDA(cudaMemcpyAsync(c->track_tab.p, t.h.data(), tab_bytes, cudaMemcpyHostToDevice, c->stream));
+  if (!pfx.empty())
+    DGRP_CUDA(cudaMemcpyAsync(c->track_tab.as<uint8_t>() + tab_bytes, pfx.data(), pfx.size(), cudaMemcpyHostToDevice,
+                              c->stream));
+  DGRP_CUDA(cudaEventRecord(c->tev[0], c->stream));
+  int64_t n = 0;
+  DGRP_CHECK(run_track(c, t, c->track_tab.as<int64_t>(), c->track_tab.as<uint8_t>() + tab_bytes, c->fa_pred.as<float>(),
+                       c->fa_classes, cls, c->track_work, c->track_text, &n));
+  DGRP_CUDA(cudaEventRecord(c->tev[1], c->stream));
+  DGRP_CHECK(c->track_host.reserve((size_t)n + 16));
+  if (n > 0)
+    DGRP_CUDA(cudaMemcpyAsync(c->track_host.p, c->track_text.p, (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+  DGRP_CUDA(cudaStreamSynchronize(c->stream));
+  float ms = 0.f;
+  DGRP_CUDA(cudaEventElapsedTime(&ms, c->tev[0], c->tev[1]));
+  c->track_kernel_ns = (int64_t)(ms * 1e6f);
+  *text = c->track_host.as<uint8_t>();
+  *len = n;
   return DGRP_OK;
 }
 

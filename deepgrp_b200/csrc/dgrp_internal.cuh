@@ -145,6 +145,21 @@ struct dgrp_ctx {
   int fa_classes = 0;                  // the model classes of that call (dgrp_evaluate_last)
   dgrp::DevBuf eval_tab, eval_counts;  // dgrp_evaluate_last: record / run table, per-record counts
   int64_t eval_kernel_ns = 0;          // device time of the last evaluation kernel (CUDA events)
+  // dgrp_track_last: with keep_votes set, dgrp_predict_fasta[_tsv] also keeps every kept record's max-vote rows
+  // (f32[length][C], record r's from row fa_pred_off[r]) and its chromosome (first word of the header, fa_chrom at
+  // fa_chrom_off[r]); fa_votes: the last call did so and succeeded.  fa_pred holds the votes of the largest call
+  // (grow-only while keep_votes is set) and is freed by the next call without keep_votes.  track_* hold the table, the
+  // bin words, the line starts, the text on the device and in pinned host memory (the view dgrp_track_last returns)
+  int keep_votes = 0;
+  bool fa_votes = false;
+  dgrp::DevBuf fa_pred;
+  std::vector<int64_t> fa_pred_off, fa_chrom_off;
+  std::string fa_chrom;
+  dgrp::DevBuf track_tab, track_work, track_text;
+  dgrp::PinBuf track_host;
+  int64_t votes_append_ns = 0;         // device time of the vote appends of the last dgrp_predict_fasta[_tsv]
+  int64_t track_kernel_ns = 0;         // device time of the kernels of the last dgrp_track_last (CUDA events)
+  cudaEvent_t tev[2] = {};
   dgrp::DevBuf mask_rec, mask_bits, mask_out;   // dgrp_mask_fasta*: record table, rank bitmap, masked text
   int shard_rank = 0, shard_world = 1;   // contig sharding of dgrp_predict_fasta* (dgrp_ctx_set_int)
   dgrp::PinBuf tsv_host;     // finished TSV text of the last dgrp_predict_fasta_tsv
@@ -290,6 +305,13 @@ namespace eval { struct Table; }
 // dgrp_predict_fasta to d_counts[r][t][p] (int64, zeroed by the caller); one launch
 int run_eval_confusion(dgrp_ctx *c, int C, const eval::Table &t, const int64_t *d_tab, const int64_t *d_tri,
                        int64_t *d_counts);
+// track.cu
+namespace track { struct Table; }
+// K11: the bedGraph text of class cls for every record of the table t (uploaded to d_tab, prefix text at d_text)
+// from the vote rows d_pred into text (device, reserved here); *n_bytes = its length.  Bin words and line starts go
+// to work; synchronises twice (line count, byte count)
+int run_track(dgrp_ctx *c, const track::Table &t, const int64_t *d_tab, const uint8_t *d_text, const float *d_pred,
+              int C, int cls, DevBuf &work, DevBuf &text, int64_t *n_bytes);
 // segments.cu
 // open_tail != nullptr: the labels are a prefix of a record whose continuation is not known yet.  The
 // reference's special case of the record's last element does not apply, and a run that reaches the end of

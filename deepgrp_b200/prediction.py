@@ -15,6 +15,7 @@ Differences that callers can see:
 from __future__ import annotations
 
 import ctypes
+import io
 import os
 from typing import Iterator, Optional, Tuple
 
@@ -28,6 +29,7 @@ from . import preprocessing  # noqa: F401  (Data, as in the reference's import l
 
 _COMPAT = {"reference": _lib.COMPAT_REFERENCE, "fixed": _lib.COMPAT_FIXED}
 _MASK = {"soft": _lib.MASK_SOFT, "hard": _lib.MASK_HARD}
+TRACK_BIN_MAX = 1_000_000
 
 
 class WindowDataset:
@@ -451,39 +453,110 @@ def predict_fasta_tsv_masked(model: ModelWeights, raw, filename: str, outstream,
                              batch_size: int, use_mss: bool, min_mss_len: int, xdrop_len: int, mode: str = "soft",
                              compat: str = "reference") -> dict:
     """:func:`predict_fasta_tsv_stream` that also writes the masked text of ``raw`` (see :func:`mask_fasta`) to
-    the binary stream ``maskstream``.  The file runs slice by slice (whole records, >= 8 MiB, the streaming
-    driver's cuts with one rank), which bounds device memory: each slice is predicted in one call, its TSV text is
-    written, and its rows, still on the device, mask its bytes.  A slice with a blank line or an all-``N`` record
-    is run again through :func:`predict_fasta_tsv_stream`, so the TSV text holds the rows of the records before the
-    error, as the default route writes them, and the same ``IndexError`` / ``ValueError`` is raised; the masked
-    text then holds the slices before that one.  Returns the totals (rows, records, bases, slices)."""
+    the binary stream ``maskstream``: :func:`predict_fasta_sliced` with a mask stream."""
+    return predict_fasta_sliced(model, raw, filename, outstream, step_size, batch_size, use_mss, min_mss_len,
+                                xdrop_len, compat, maskstream=maskstream, mask_mode=mode)
+
+
+def _track_bin(bin: int) -> int:
+    if int(bin) != bin or not 1 <= bin <= TRACK_BIN_MAX:
+        raise ValueError("track bin size must be an integer in [1, %d], not %r" % (TRACK_BIN_MAX, bin))
+    return int(bin)
+
+
+def track_last(cls: int, bin: int) -> memoryview:
+    """``dgrp_track_last``: the bedGraph text of class ``cls`` of the last :func:`predict_fasta` call, which ran with
+    the context option ``keep_votes`` set.  A read-only view of pinned host memory owned by the context, valid until
+    the next call: write it out (or copy it) first."""
+    ctx = _lib.context()
+    text, n = ctypes.c_void_p(), ctypes.c_int64(0)
+    _lib.check(_lib.lib().dgrp_track_last(ctx.handle, int(cls), int(bin), ctypes.byref(text), ctypes.byref(n)))
+    if n.value == 0:
+        return memoryview(b"")
+    return memoryview((ctypes.c_ubyte * n.value).from_address(text.value)).cast("B").toreadonly()
+
+
+def predict_fasta_sliced(model: ModelWeights, raw, filename: str, outstream, step_size: int, batch_size: int,
+                         use_mss: bool, min_mss_len: int, xdrop_len: int, compat: str = "reference", maskstream=None,
+                         mask_mode: str = "soft", trackstreams: Optional[dict] = None, track_bin: int = 10) -> dict:
+    """Predict one FASTA file slice by slice (whole records, >= 8 MiB, the streaming driver's cuts with one rank),
+    which bounds device memory.  One prediction per slice serves every output:
+
+    * ``outstream`` (binary, or None): the TSV text, as :func:`predict_fasta_tsv_stream` writes it;
+    * ``maskstream`` (binary, or None): the masked text of the slice (see :func:`mask_fasta`, ``mask_mode``), made
+      from its rows while they are still on the device;
+    * ``trackstreams`` (``{class: binary stream}``, or None): the bedGraph lines of each class with bins of
+      ``track_bin`` bases (see :func:`predict_fasta_tracks`), from the slice's max-vote rows kept on the device.
+
+    A slice with a blank line or an all-``N`` record is run again through :func:`predict_fasta_tsv_stream` (when there
+    is an ``outstream``), so the TSV text holds the rows of the records before the error, as the default route writes
+    them, and the same ``IndexError`` / ``ValueError`` is raised; the masked text and the tracks then hold the slices
+    before that one.  Returns the totals (rows, records, bases, slices)."""
     from .sharding import fasta_slices
-    code = _mask_mode(mode)
+    code = _mask_mode(mask_mode) if maskstream is not None else None
+    if trackstreams:
+        track_bin = _track_bin(track_bin)
+        bad = [c for c in trackstreams if not 1 <= int(c) < model.n_classes]
+        if bad:
+            raise ValueError("track classes must lie in [1, %d), got %s" % (model.n_classes, bad))
     ctx = _lib.context()
     cuts, _ = fasta_slices(raw, 1)
     whole = memoryview(raw) if len(raw) else memoryview(b"")
     totals = {"rows": 0, "records": 0, "bases": 0, "slices": len(cuts) - 1}
     for k in range(len(cuts) - 1):
         piece = whole[int(cuts[k]):int(cuts[k + 1])]
+        keep = ctx.get_int("keep_votes")          # the caller's setting, restored after the call
+        if trackstreams:
+            ctx.set_int("keep_votes", 1)
         try:
-            view, n_rows, n_rec = _fasta_tsv_call(model, piece, filename, step_size, batch_size, use_mss,
-                                                  min_mss_len, xdrop_len, compat)
+            if outstream is not None:
+                view, n_rows, n_rec = _fasta_tsv_call(model, piece, filename, step_size, batch_size, use_mss,
+                                                      min_mss_len, xdrop_len, compat)
+            else:
+                n_rows, recs = _predict_fasta_call(model, piece, step_size, batch_size, use_mss, min_mss_len,
+                                                   xdrop_len, compat)
+                view, n_rec = memoryview(b""), len(recs)
         except (IndexError, ValueError):
+            if outstream is None:
+                raise
             predict_fasta_tsv_stream(model, piece, filename, outstream, step_size, batch_size, use_mss,
                                      min_mss_len, xdrop_len, compat)
             raise RuntimeError("slice %d failed in the whole-slice call but not in the stream" % k)
+        finally:
+            ctx.set_int("keep_votes", keep)
         totals["bases"] += int(ctx.timings()["bases"])
         totals["rows"] += n_rows
         totals["records"] += n_rec
         if len(view):
             outstream.write(view)
         n = len(piece)
-        if n:
+        if maskstream is not None and n:
             buf = np.frombuffer(piece, dtype=np.uint8)
             out = np.empty(n, dtype=np.uint8)
             _lib.check(_lib.lib().dgrp_mask_fasta_last(ctx.handle, _lib.ptr(buf), n, code, _lib.ptr(out)))
             maskstream.write(out)
+        for cls, stream in (trackstreams or {}).items():
+            text = track_last(cls, track_bin)
+            if len(text):
+                stream.write(text)
     return totals
+
+
+def predict_fasta_tracks(model: ModelWeights, raw, step_size: int, batch_size: int, bin: int = 10,
+                         compat: str = "reference") -> dict:
+    """Per-base repeat probability tracks of one FASTA file: ``{class: bedGraph bytes}`` for every repeat class
+    ``1 .. C-1``, computed and formatted on the GPU.  The value of a position is its max-vote probability
+    (:func:`predict`, before MSS or softmax) in untrimmed record coordinates; positions outside a record's span
+    ``[startpos, startpos + length)`` (its edge ``N`` s) have none.  Bins ``[k bin, (k + 1) bin)`` are aligned to 0 and
+    clipped to the span; a bin's value is ``rint(mean * 1000) / 1000`` (float64 sum in position order, round half to
+    even), written as ``%d.%03d``.  Consecutive bins of one record with the same value make one line
+    ``chrom\tstart\tend\tvalue``; ``chrom`` is the header's first word.  The file runs in slices (whole records,
+    >= 8 MiB).  A blank line raises ``IndexError`` and an all-``N`` record ``ValueError``, as in ``predict``."""
+    bin = _track_bin(bin)
+    streams = {c: io.BytesIO() for c in range(1, model.n_classes)}
+    predict_fasta_sliced(model, raw, "", None, step_size, batch_size, False, 50, 50, compat,
+                         trackstreams=streams, track_bin=bin)
+    return {c: s.getvalue() for c, s in streams.items()}
 
 
 # ---- evaluation helpers (deepgrp/prediction.py:144-260; used by deepgrp/optimization.py:58-69) -------

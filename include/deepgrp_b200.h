@@ -87,7 +87,11 @@ int64_t dgrp_ctx_launch_count(dgrp_ctx *ctx);
  * "stream_slot_mb" (host piece size of dgrp_fasta_stream), "stream_early_rows" / "stream_early_slabs" /
  * "stream_early_ratio" / "stream_early_unit" (position slabs of a long record in dgrp_fasta_stream; get-only
  * "stream_early_parts": parts of the last record's text that left before its last slab); get-only "eval_kernel_ns"
- * (device time of the last dgrp_evaluate_last kernel, nanoseconds). */
+ * (device time of the last dgrp_evaluate_last kernel, nanoseconds); "keep_votes" (0 / 1, default 0: whether
+ * dgrp_predict_fasta[_tsv] keeps every record's max-vote rows on the device for dgrp_track_last -- 4 C bytes per base
+ * of the call, held until the next dgrp_predict_fasta[_tsv] without it or the context's destruction); get-only
+ * "votes_append_ns" (device time of those copies in the last call) and "track_kernel_ns" (device time of the last
+ * dgrp_track_last from its first kernel to its last, nanoseconds). */
 int dgrp_ctx_set_int(dgrp_ctx *ctx, const char *key, int64_t value);
 int dgrp_ctx_get_int(dgrp_ctx *ctx, const char *key, int64_t *value);
 
@@ -260,6 +264,17 @@ int dgrp_mask_fasta_last(dgrp_ctx *ctx, const uint8_t *fasta, int64_t nbytes, in
  * a NULL pointer.  The device time of the kernel is read with dgrp_ctx_get_int(ctx, "eval_kernel_ns", ...). */
 int dgrp_evaluate_last(dgrp_ctx *ctx, int n_classes, const int64_t *ann, const int64_t *ann_off, int64_t n_records,
                        int64_t *counts);
+/* Probability track (bedGraph) of class cls for every kept record of the last dgrp_predict_fasta[_tsv], which must
+ * have run with the option "keep_votes" set.  The value of a position is its max-vote pred[p][cls] before MSS or
+ * softmax (the predictions of deepgrp/prediction.py:89-111).  Bins [k bin, (k + 1) bin) in untrimmed record
+ * coordinates, clipped to the record's span [startpos, startpos + length); a bin's value is the float64 mean of its
+ * positions' votes summed in ascending order, rounded half-to-even to thousandths (rint(mean * 1000.0)) and written
+ * as "%d.%03d".  Consecutive bins of one record with the same value form one line "chrom\tstart\tend\tvalue\n";
+ * chrom is the first word of the header; no track line, records in file order.  *text is pinned host memory owned by
+ * the context, valid until the next call of this function or the context's destruction.  DGRP_E_ARG when there is no
+ * such prediction (as in dgrp_mask_fasta_last), when it did not keep its votes, for cls outside [1, C), a bin outside
+ * [1, 1000000] or a NULL pointer. */
+int dgrp_track_last(dgrp_ctx *ctx, int cls, int bin, const uint8_t **text, int64_t *len);
 /* rows[i].record indexes the record table */
 int dgrp_fasta_rows(dgrp_ctx *ctx, dgrp_row_t *rows, int64_t cap);
 /* per record: header text = fasta[hdr_off, hdr_off + hdr_len); startpos = leading 'N' count;
